@@ -2,6 +2,7 @@
 
     python bench.py --gpus N --steps K --warmup W            # this repo's CUDA path
     python bench.py --impl reference ...                      # the reference's CPU path (oracle port)
+    python bench.py ... --dump-outputs DIR                    # also write the last timed step's results as .npy
 
 One "step" = the hot path of reference trainer.py:105-120 over one batch of 64 synthetic
 MIND-shaped impressions per GPU (title <= 32, abstract <= 128, history 50, K = 4, 300-d words,
@@ -58,7 +59,16 @@ def parse():
     ap.add_argument('--no-graph', action='store_true', help='launch every kernel of a step from the host instead of replaying a CUDA graph')
     ap.add_argument('--no-extras', action='store_true', help='skip the extra measurements (scoring, full-length regime)')
     ap.add_argument('--scoring-news', type=int, default=100000, help='news in the synthetic corpus of the scoring extra')
-    return ap.parse_args()
+    ap.add_argument('--dump-outputs', metavar='DIR',
+                    help='after the timed steps, write what the last one computed (loss, gradient norm before clipping, every '
+                         'parameter after the update and its gradient before clipping) to DIR/<name>.npy, to compare two builds '
+                         'output for output')
+    a = ap.parse_args()
+    if a.steps < 1:
+        ap.error('--steps must be at least 1')
+    if a.dump_outputs and a.impl == 'reference':
+        ap.error('--dump-outputs writes the results of the CUDA path; --impl reference has none')
+    return a
 
 
 def workload_name(a):
@@ -293,6 +303,33 @@ def extra_full_lengths(a, ts, dev, peaks):
 
 
 # -------------------------------------------------------------------------------------------------
+# --dump-outputs: the results of the last timed step, for comparing two builds output for output
+# -------------------------------------------------------------------------------------------------
+DUMP_MAX_ELEMENTS = 1 << 18      # per tensor; keeps the directory under 40 MB (the word table is the only tensor --vocab resizes)
+
+
+def dump_outputs(directory, ts, loss):
+    """What a caller of TrainStep.step has after the last timed step: the returned loss, the total gradient norm before
+    clipping (ts.grad_norm, what clip_grad_norm_ returns) and, for every trainable parameter, its value after the Adam update
+    (param.<name>) and its gradient before clipping (grad.<name>; with N > 1 the sum over ranks, which the optimizer kernel
+    scales by 1/N), flattened, float32.  A tensor of more than DUMP_MAX_ELEMENTS elements is written as its
+    elements at DUMP_MAX_ELEMENTS sorted flat positions drawn by a generator seeded with 0: the same positions on every run
+    and every build."""
+    import numpy as np
+    os.makedirs(directory, exist_ok=True)
+    torch.cuda.synchronize()
+    out = {'loss': loss.detach(), 'grad_norm': ts.grad_norm}
+    for name, p in ts.model.named_parameters():
+        if p.requires_grad:
+            out['param.' + name] = p.detach()
+            out['grad.' + name] = p.grad
+    for name, t in out.items():
+        a = t.float().reshape(-1).cpu().numpy()
+        if a.size > DUMP_MAX_ELEMENTS:
+            a = a[np.sort(np.random.default_rng(0).choice(a.size, DUMP_MAX_ELEMENTS, replace=False))]
+        np.save(os.path.join(directory, name + '.npy'), a)
+
+
 def main():
     a = parse()
     if a.impl == 'reference':
@@ -382,6 +419,8 @@ def main():
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
     ms = t.item()
     value = a.batch * world * a.steps / (ms / 1e3)
+    if a.dump_outputs and rank == 0:                          # before the passes below move the parameters on
+        dump_outputs(a.dump_outputs, ts, loss)
 
     # ---- end to end: pinned host batch -> device every step, loss read back every step ----------
     for i in range(2):                                        # untimed warm-up of this path (allocator, copy engine)

@@ -35,16 +35,21 @@ def test_oracle_matches_golden_gradients(name):
     cfg.dropout_rate = 0.0
     p = O.formula_params(cfg)
     logits, loss, grads = O.forward_backward(p, cfg, batch, sort_fn=O.stable_sort)
+    _, _, grads64 = O.forward_backward(p, cfg, batch, dtype=torch.float64, sort_fn=O.stable_sort)
     np.testing.assert_allclose(logits.numpy(), z['train_logits'], atol=2e-5)
     assert abs(float(loss) - float(z['train_loss'])) < 1e-5
     gscale = max(float(z['grad_' + k][2]) for k in grads)            # largest gradient entry overall
     for k, g in grads.items():
         ref = z['grad_' + k]
         mine = grad_digest(g)
-        tol = 1e-4 * max(ref[2], 1e-4 * gscale)
+        # fp32 rounding of the oracle where the test runs (its fp32 digest against its fp64 one): gradients that are sums with heavy
+        # cancellation (the self-attention biases, ~1e-7 against a largest entry of ~0.07) move by that much with the CPU's
+        # summation order (thread count, vector width), here and in the golden run alike -- as in test_model_gpu's tolerance
+        noise = np.abs(mine - grad_digest(grads64[k]))
+        tol = 1e-4 * max(ref[2], 1e-4 * gscale) + 8 * max(noise[2], noise[3:].max())
         assert abs(mine[2] - ref[2]) <= tol, k
         assert np.all(np.abs(mine[3:] - ref[3:]) <= tol), k
-        assert abs(mine[0] - ref[0]) <= 1e-4 * max(ref[1], 1e-12) + 1e-9, k
+        assert abs(mine[0] - ref[0]) <= 1e-4 * max(ref[1], 1e-12) + 1e-9 + 8 * noise[0], k
 
 
 def test_loop_lstm_equals_aten_lstm():
@@ -65,7 +70,8 @@ def test_oracle_fp64_consistency():
     assert (l32.double() - l64).abs().max().item() < 1e-5
 
 
-@pytest.mark.skipif(not R.available(), reason='reference checkout not present (GPU box)')
+@pytest.mark.skipif(not R.available(), reason='needs a checkout of the original NNR project at NNR_REFERENCE_ROOT; '
+                    'test_oracle_matches_golden_logits checks against its stored outputs')
 def test_oracle_matches_live_reference():
     cfg, batch, _ = load_golden('tiny')
     p = O.formula_params(cfg, salt=3)                                 # different weights than the golden run

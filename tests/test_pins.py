@@ -1,5 +1,5 @@
 """CPU tests that PIN the restated test infrastructure against the reference itself, executed (skipped where
-/root/reference does not exist, i.e. on the GPU box):
+no checkout of the original NNR project is found at NNR_REFERENCE_ROOT):
 
   * oracle/graph.py           against the literal source lines MIND_corpus.py:178-213 run under stub variables
                               (MIND_corpus.py cannot be imported: it needs nltk / torchtext at module level)
@@ -26,7 +26,8 @@ from oracle import nnr_oracle as O
 from oracle import reference_import as R
 from tests.util import GOLDEN_DIR
 
-needs_reference = pytest.mark.skipif(not R.available(), reason='reference checkout not present (GPU box)')
+needs_reference = pytest.mark.skipif(not R.available(), reason='needs a checkout of the original NNR project at NNR_REFERENCE_ROOT; '
+                                     'the *_committed_reference_vectors tests check against its stored outputs')
 
 FLAG_SETS = [dict(no_self_connection=False, no_adjacent_normalization=False, gcn_normalization_type='symmetric'),
              dict(no_self_connection=False, no_adjacent_normalization=False, gcn_normalization_type='asymmetric'),
