@@ -166,7 +166,10 @@ int nnr_segment_colsum(const float* X, int64_t ldx, const int32_t* off, int N, i
                        int64_t ldo, void* stream);
 
 /* ---- bidirectional LSTM recurrence: nn.LSTM at newsEncoders.py:66-67,122-127 ----------------
- * Persistent thread-block-cluster kernel; W_hh stays in shared memory for all time steps.
+ * Persistent thread-block-cluster kernel; W_hh stays on chip for all time steps.
+ * Hidden sizes: 0 < H <= 200 with H % 4 == 0 (tensor-core kernels, clusters of max(2, ceil(H / 40)) CTAs); the exact-fp32
+ * FFMA kernels (NNR_LSTM_ALGO=ffma) and the shared-memory W variants (NNR_LSTM_FWD_TM=0 / NNR_LSTM_BWD_TM=0) take H = 200
+ * only.  Any other H returns NNR_ERR_UNSUPPORTED before a CUDA call, with the rule in nnr_last_error().
  *   gx      [tokens, 2, 4H]  in: x_t W_ih^T + b_ih + b_hh (gate order i,f,g,o per direction)
  *                            out: the activated gates (stash for the backward pass)
  *   w_hh    [2, 4H, H]       forward / reverse recurrent weights

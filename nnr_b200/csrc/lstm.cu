@@ -505,12 +505,13 @@ static int launch_cluster(K kernel, size_t smem, int ntiles, cudaStream_t st, vo
 }
 
 // tensor-core variant (lstm_mma.cu); NNR_LSTM_ALGO=ffma selects the exact-fp32 FFMA kernels of this file
-int nnr_lstm_fwd_mma(float* gx, const float* w_hh, const int32_t* len, const int32_t* off, const int32_t* order, int N,
+int nnr_lstm_fwd_mma(float* gx, const float* w_hh, const int32_t* len, const int32_t* off, const int32_t* order, int N, int H,
                      float* h_out, float* c_stash, float* c_n, int32_t* tile_counters, cudaStream_t st, void* h_planes,
                      size_t plane_stride, int two_planes, int cap);
 int nnr_lstm_fwd_planes_ok(void);
+int nnr_lstm_bwd_tm_ok(void);
 int nnr_lstm_bwd_mma(float* gates, const float* c_stash, const float* w_hh, const int32_t* len, const int32_t* off,
-                     const int32_t* order, int N, const float* dh, const float* dcn, int32_t* tile_counters, cudaStream_t st,
+                     const int32_t* order, int N, int H, const float* dh, const float* dcn, int32_t* tile_counters, cudaStream_t st,
                      void* dz_planes, size_t plane_stride, int two_planes, float* db_partial, float* db, int cap);
 static bool lstm_use_mma() {
   static int v = -1;
@@ -521,15 +522,28 @@ static bool lstm_use_mma() {
   return v == 1;
 }
 
+// The hidden sizes a recurrence entry point accepts, checked before any CUDA call.  The tensor-core kernels with the W slice in
+// tensor memory (the default) take 0 < H <= 200, H % 4 == 0 (clusters of 2..5 CTAs of 40 units, 16 B chunks of 4 units); the
+// exact-fp32 FFMA kernels and the shared-memory W variants are instantiated for hidden_dim 200 only.
+static int lstm_check_hidden(const char* fn, int H, bool tm) {
+  NNR_REQUIRE(H > 0 && H <= 200 && H % 4 == 0, NNR_ERR_UNSUPPORTED,
+              "%s: hidden_dim %d: the tensor-core recurrence takes H %% 4 == 0 and H <= 200", fn, H);
+  NNR_REQUIRE(H == 200 || lstm_use_mma(), NNR_ERR_UNSUPPORTED,
+              "%s: hidden_dim %d: the exact-fp32 FFMA recurrence (NNR_LSTM_ALGO=ffma) takes hidden_dim 200 only", fn, H);
+  NNR_REQUIRE(H == 200 || tm, NNR_ERR_UNSUPPORTED, "%s: hidden_dim %d: the shared-memory W variant (%s=0) takes hidden_dim 200 only", fn, H,
+              !strcmp(fn, "nnr_lstm_fwd") ? "NNR_LSTM_FWD_TM" : "NNR_LSTM_BWD_TM");
+  return 0;
+}
+
 extern "C" int nnr_lstm_fwd(float* gx, const float* w_hh, const int32_t* len, const int32_t* off, const int32_t* order,
                             int N, int L, int H, float* h_out, float* c_stash, float* c_n, int32_t* tile_counters,
                             void* stream) {
   NNR_REQUIRE(gx && w_hh && len && off && order && h_out && c_stash && c_n && tile_counters && N > 0 && L > 0, NNR_ERR_ARG,
               "nnr_lstm_fwd: bad arguments");
-  NNR_REQUIRE(H == 200, NNR_ERR_UNSUPPORTED, "nnr_lstm_fwd: hidden_dim %d not instantiated (200 only)", H);
+  if (int rc = lstm_check_hidden("nnr_lstm_fwd", H, nnr_lstm_fwd_planes_ok())) return rc;
   NNR_REQUIRE(nnr_aligned16(gx) && nnr_aligned16(h_out) && nnr_aligned16(c_stash) && nnr_aligned16(c_n), NNR_ERR_ALIGN,
               "nnr_lstm_fwd: buffers must be 16B aligned");
-  if (lstm_use_mma()) return nnr_lstm_fwd_mma(gx, w_hh, len, off, order, N, h_out, c_stash, c_n, tile_counters, (cudaStream_t)stream, NULL, 0, 0, 0);
+  if (lstm_use_mma()) return nnr_lstm_fwd_mma(gx, w_hh, len, off, order, N, H, h_out, c_stash, c_n, tile_counters, (cudaStream_t)stream, NULL, 0, 0, 0);
   typedef FwdCfg200 C;
   int ntiles = (N + C::MT - 1) / C::MT;
   NNR_CUDA(cudaMemsetAsync(tile_counters, 0, 2 * sizeof(int32_t), (cudaStream_t)stream));
@@ -542,11 +556,11 @@ extern "C" int nnr_lstm_bwd(float* gates, const float* c_stash, const float* w_h
                             int32_t* tile_counters, void* stream) {
   NNR_REQUIRE(gates && c_stash && w_hh && len && off && order && dh && dcn && tile_counters && N > 0 && L > 0, NNR_ERR_ARG,
               "nnr_lstm_bwd: bad arguments");
-  NNR_REQUIRE(H == 200, NNR_ERR_UNSUPPORTED, "nnr_lstm_bwd: hidden_dim %d not instantiated (200 only)", H);
+  if (int rc = lstm_check_hidden("nnr_lstm_bwd", H, nnr_lstm_bwd_tm_ok())) return rc;
   NNR_REQUIRE(nnr_aligned16(gates) && nnr_aligned16(c_stash) && nnr_aligned16(dh) && nnr_aligned16(dcn), NNR_ERR_ALIGN,
               "nnr_lstm_bwd: buffers must be 16B aligned");
   if (lstm_use_mma())
-    return nnr_lstm_bwd_mma(gates, c_stash, w_hh, len, off, order, N, dh, dcn, tile_counters, (cudaStream_t)stream, NULL, 0, 0, NULL, NULL, 0);
+    return nnr_lstm_bwd_mma(gates, c_stash, w_hh, len, off, order, N, H, dh, dcn, tile_counters, (cudaStream_t)stream, NULL, 0, 0, NULL, NULL, 0);
   typedef BwdCfg200 C;
   int ntiles = (N + C::MT - 1) / C::MT;
   NNR_CUDA(cudaMemsetAsync(tile_counters, 0, 2 * sizeof(int32_t), (cudaStream_t)stream));
@@ -574,7 +588,7 @@ extern "C" int nnr_lstm_fwd_planes(float* gx, const float* w_hh, const int32_t* 
   const int two = algo == NNR_GEMM_TC_BF16X3;
   const size_t plane = (size_t)cap * 2 * H;
   NNR_REQUIRE(planes_bytes >= plane * 2 * (two ? 2 : 1), NNR_ERR_WORKSPACE, "nnr_lstm_fwd_planes: planes buffer too small");
-  return nnr_lstm_fwd_mma(gx, w_hh, len, off, order, N, h_out, c_stash, c_n, tile_counters, (cudaStream_t)stream, planes, plane, two, cap);
+  return nnr_lstm_fwd_mma(gx, w_hh, len, off, order, N, H, h_out, c_stash, c_n, tile_counters, (cudaStream_t)stream, planes, plane, two, cap);
 }
 
 // BPTT with dL/dgx emitted as GEMM operand planes + its column sums (the bias gradient): dL/dgx is only ever read by the
@@ -600,6 +614,6 @@ extern "C" int nnr_lstm_bwd_planes(const float* gates, const float* c_stash, con
               NNR_ERR_ALIGN, "nnr_lstm_bwd_planes: buffers must be 16B aligned");
   NNR_REQUIRE(planes_bytes >= nnr_tc_split_bytes(cap, 8 * H, algo), NNR_ERR_WORKSPACE, "nnr_lstm_bwd_planes: planes buffer too small");
   NNR_REQUIRE(workspace_bytes >= nnr_lstm_bwd_planes_workspace_bytes(N, H), NNR_ERR_WORKSPACE, "nnr_lstm_bwd_planes: workspace too small");
-  return nnr_lstm_bwd_mma(const_cast<float*>(gates), c_stash, w_hh, len, off, order, N, dh, dcn, tile_counters, (cudaStream_t)stream,
+  return nnr_lstm_bwd_mma(const_cast<float*>(gates), c_stash, w_hh, len, off, order, N, H, dh, dcn, tile_counters, (cudaStream_t)stream,
                           dz_planes, (size_t)cap * 8 * H, algo == NNR_GEMM_TC_BF16X3 ? 1 : 0, (float*)workspace, db, cap);
 }

@@ -1,4 +1,5 @@
-// Tensor-core variant of the persistent bidirectional LSTM kernels (forward and BPTT) for H = 200.
+// Tensor-core variant of the persistent bidirectional LSTM kernels (forward and BPTT) for 0 < H <= 200, H % 4 == 0 (clusters of
+// CL = max(2, ceil(H / 40)) CTAs, see G; the shared-memory W variants for H = 200 only).  The description below is for H = 200.
 // Same interface, data layout and stash protocol as lstm.cu; replaces cuDNN's RNN behind nn.LSTM at
 // newsEncoders.py:66-67,119-127.
 //
@@ -39,10 +40,17 @@ __device__ unsigned long long g_lstm_prof[16];
 
 namespace {
 
+// The cluster size CL sets the padded hidden size HP = 40 CL the kernels are laid out for (CL = max(2, ceil(H / 40))).  Units
+// [H, HP) are ghost units: never read from or written to global memory, zero inside the kernel (zero W rows and K slots, h = c =
+// dz = dc = 0).  Global strides use the runtime H; shared / tensor memory layouts use HP.  CL = 1 is not instantiated: the
+// exchange and its transaction counts assume peers.
+template <int CL_>
 struct G {
-  static constexpr int HID = 200, CL = 5, MT = 32, UPC = 40, COLS = 160, CT = 128, NT = 256, UPW = 10, NTW = 5;   // CT compute + 128 copy threads
-  // forward: A = h [32][K=208 (200 + zero pad)], B = W slice [160 cols][208]; pitch 432 B -> ldmatrix conflict free
-  static constexpr int FK = 208, FKS = 13, FPITCH = 432;
+  static constexpr int CL = CL_, HP = 40 * CL, MT = 32, UPC = 40, COLS = 160, CT = 128, NT = 256, UPW = 10, NTW = 5;   // CT compute + 128 copy threads
+  // forward: A = h [32][K=FK (HP + zero pad to a multiple of 16)], B = W slice [160 cols][FK]; pitch 432 B -> ldmatrix conflict free
+  // (the shared-memory W variant exists for CL = 5 only).  HALF: HP % 16 == 8, the last k-step is half padding (HP = 120, 200).
+  static constexpr bool HALF = HP % 16 == 8;
+  static constexpr int FK = (HP + 15) / 16 * 16, FKS = FK / 16, FPITCH = 432;
   // h tile = [source CTA j][plane hi/lo][32 rows][40 slots = 80 B]: the slice a CTA produces is ONE contiguous 5120 B
   // block (a single cp.async.bulk per peer); row pitch 80 B keeps ldmatrix conflict free.  A 16 B zero chunk pads K.
   static constexpr int F_W_PLANE = COLS * FPITCH, F_HROW = 80, F_HPLANE = MT * F_HROW, F_HBLK = 2 * F_HPLANE, F_HBUF = CL * F_HBLK;
@@ -56,33 +64,70 @@ struct G {
   // ([source CTA][32 rows][40 units] fp32 = 5120 B blocks: one bulk copy each) and the staging tile of the same shape
   // the partials are copied from.  The W slice is XOR-swizzled (16 B chunk ^= (row >> 1) & 3) instead of padded.
   static constexpr int BK = 160, BKS = 10, BPITCH = 336, BWPITCH = 320, RPITCH = UPC * 4;
-  static constexpr int B_W_PLANE = HID * BWPITCH, B_Z_PLANE = MT * BPITCH, B_RBLK = MT * RPITCH, B_RECV = CL * B_RBLK;
+  static constexpr int B_W_PLANE = HP * BWPITCH, B_Z_PLANE = MT * BPITCH, B_RBLK = MT * RPITCH, B_RECV = CL * B_RBLK;
   static constexpr int B_NARR = 5;                       // i, f, g, o (stash in, dz out), dh
   static constexpr size_t BWD_SMEM = 2 * (size_t)B_W_PLANE + 2 * (size_t)B_Z_PLANE + 2 * (size_t)B_RECV + B_NARR * (size_t)SARR + 3 * MT * sizeof(int);
   static constexpr uint32_t B_TX = CL * B_RBLK;
+  // backward phase 2: the 5 CL n8 tiles of output units over the 4 compute warps, the first EXTRA warps take one more
+  // (CL = 5: 7, 6, 6, 6; CL = 4: 5 each; CL = 3: 4, 4, 4, 3; CL = 2: 3, 3, 2, 2)
+  static constexpr int NTILE = 5 * CL, BASE = NTILE / 4, EXTRA = NTILE % 4, NTWB = BASE + (EXTRA > 0);
 };
 
 
 // forward variant with the W slice in TENSOR MEMORY (lstm_fwd_tm_kernel): 4 compute + 2 copy warps, no W planes in shared memory
+template <int CL_>
 struct G2 {
-  static constexpr int HID = G::HID, CL = G::CL, MT = G::MT, UPC = G::UPC, COLS = G::COLS, UPW = G::UPW, NTW = G::NTW;
+  using G1 = G<CL_>;
+  static constexpr int HP = G1::HP, CL = G1::CL, MT = G1::MT, UPC = G1::UPC, COLS = G1::COLS, UPW = G1::UPW, NTW = G1::NTW;
   static constexpr int CT = 128, NT = 192;
-  static constexpr int FK = G::FK, FKS = G::FKS;
-  static constexpr int F_HROW = G::F_HROW, F_HPLANE = G::F_HPLANE, F_HBLK = G::F_HBLK, F_HBUF = G::F_HBUF;
-  static constexpr int SROW = G::SROW, SARR = G::SARR, F_NARR = G::F_NARR;
-  static constexpr uint32_t F_TX = G::F_TX;
-  static constexpr int TM_COLS = 256;                      // 12 k-steps x 20 + 10 = 250 columns used
-  static constexpr size_t FWD_SMEM = 2 * (size_t)F_HBUF + 16 + F_NARR * (size_t)SARR + 3 * MT * sizeof(int);
+  static constexpr bool HALF = G1::HALF;
+  static constexpr int FK = G1::FK, FKS = G1::FKS;
+  static constexpr int F_HROW = G1::F_HROW, F_HPLANE = G1::F_HPLANE, F_HBLK = G1::F_HBLK, F_HBUF = G1::F_HBUF;
+  static constexpr int SROW = G1::SROW, SARR = G1::SARR, F_NARR = G1::F_NARR;
+  static constexpr uint32_t F_TX = G1::F_TX;
+  static constexpr int F_ZERO = HALF ? 16 : 0;             // the K pad chunk the half k-step reads
+  // 20 columns per full k-step, 10 for the half one: 100 / 150 / 200 / 250 for CL = 2 .. 5
+  static constexpr int TM_USED = 20 * (FKS - HALF) + 10 * HALF, TM_COLS = TM_USED <= 128 ? 128 : 256;
+  static_assert(TM_USED <= 256, "forward W slice exceeds the tensor memory of one CTA");
+  static constexpr size_t FWD_SMEM = 2 * (size_t)F_HBUF + F_ZERO + F_NARR * (size_t)SARR + 3 * MT * sizeof(int);
 };
 
-// backward variant with the W slice in TENSOR MEMORY (lstm_bwd_mma_kernel<SINGLE, true>): 4 compute + 2 copy warps; six of a
-// warp's n8 tiles live in tensor memory as ready-made mma.sync B fragments, warp 0's seventh tile (8 units) stays in shared memory
+// backward variant with the W slice in TENSOR MEMORY (lstm_bwd_mma_kernel<SINGLE, true, CL>): 4 compute + 2 copy warps; up to six
+// of a warp's n8 tiles live in tensor memory as ready-made mma.sync B fragments, the remainder (CL = 5: warp 0's seventh tile,
+// 8 units) stays in shared memory
+template <int CL_>
 struct G3 {
-  static constexpr int NT = 192, TM_COLS = 256;            // 10 k-steps x 6 n-tiles x 4 registers = 240 columns used
-  static constexpr int W7_PLANE = 8 * G::BWPITCH;          // [8 units][160 k] bf16, same XOR swizzle as the full slice
-  static constexpr size_t BWD_SMEM = 2 * (size_t)W7_PLANE + 2 * (size_t)G::B_Z_PLANE + 2 * (size_t)G::B_RECV + G::B_NARR * (size_t)G::SARR +
-                                     3 * G::MT * sizeof(int);
+  using G1 = G<CL_>;
+  static constexpr int NT = 192;
+  static constexpr int NTM = G1::NTWB < 6 ? G1::NTWB : 6, NSM = G1::NTWB - NTM;   // n8 tiles per warp in tensor / shared memory
+  static_assert(NSM == 0 || (NSM == 1 && G1::EXTRA == 1), "the shared-memory tile is warp 0's only");
+  static constexpr int TM_USED = G1::BKS * NTM * 4, TM_COLS = TM_USED <= 128 ? 128 : 256;   // 10 k-steps x NTM tiles x 4 registers
+  static constexpr int W7_PLANE = NSM * 8 * G1::BWPITCH;   // [8 units][160 k] bf16, same XOR swizzle as the full slice
+  static constexpr size_t BWD_SMEM = 2 * (size_t)W7_PLANE + 2 * (size_t)G1::B_Z_PLANE + 2 * (size_t)G1::B_RECV + G1::B_NARR * (size_t)G1::SARR +
+                                     3 * G1::MT * sizeof(int);
 };
+
+// tensor memory -> registers, N consecutive columns of the warp's lane quarter (x16 / x8 / x4 pieces)
+template <int N>
+__device__ __forceinline__ void tm_ld(uint32_t* r, uint32_t addr) {
+  if constexpr (N >= 16) {
+    asm volatile("tcgen05.ld.sync.aligned.32x32b.x16.b32 {%0, %1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15}, [%16];"
+                 : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]), "=r"(r[7]), "=r"(r[8]), "=r"(r[9]),
+                   "=r"(r[10]), "=r"(r[11]), "=r"(r[12]), "=r"(r[13]), "=r"(r[14]), "=r"(r[15])
+                 : "r"(addr));
+    tm_ld<N - 16>(r + 16, addr + 16);
+  } else if constexpr (N >= 8) {
+    asm volatile("tcgen05.ld.sync.aligned.32x32b.x8.b32 {%0, %1, %2, %3, %4, %5, %6, %7}, [%8];"
+                 : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]), "=r"(r[7])
+                 : "r"(addr));
+    tm_ld<N - 8>(r + 8, addr + 8);
+  } else if constexpr (N >= 4) {
+    asm volatile("tcgen05.ld.sync.aligned.32x32b.x4.b32 {%0, %1, %2, %3}, [%4];" : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]) : "r"(addr));
+    tm_ld<N - 4>(r + 4, addr + 4);
+  } else {
+    static_assert(N == 0, "column count must be a multiple of 4");
+  }
+}
 
 __device__ __forceinline__ void ldsm_x4(uint32_t addr, uint32_t& r0, uint32_t& r1, uint32_t& r2, uint32_t& r3) {
   asm volatile("ldmatrix.sync.aligned.m8n8.x4.shared.b16 {%0, %1, %2, %3}, [%4];" : "=r"(r0), "=r"(r1), "=r"(r2), "=r"(r3) : "r"(addr));
@@ -184,12 +229,14 @@ __device__ __forceinline__ int fwd_slot_unit(int kk) {
 // ------------------------------------------------------------------------------------------------
 // forward
 // ------------------------------------------------------------------------------------------------
+// W slice in shared memory: hidden_dim 200 (CL = 5) only
 template <bool SINGLE>   // SINGLE: one 16-bit product (hi x hi) instead of the three split products -- the bf16 variant
-__global__ void __launch_bounds__(G::NT, 1)
+__global__ void __launch_bounds__(G<5>::NT, 1)
 lstm_fwd_mma_kernel(float* __restrict__ gx, const float* __restrict__ w_hh, const int32_t* __restrict__ len,
                     const int32_t* __restrict__ off, const int32_t* __restrict__ order, int N, int ntiles,
                     float* __restrict__ h_out, float* __restrict__ c_stash, float* __restrict__ c_n, int* __restrict__ tile_counter) {
-  constexpr int HID = G::HID, CL = G::CL, MT = G::MT, UPC = G::UPC, COLS = G::COLS, NTW = G::NTW, UPW = G::UPW;
+  using G = ::G<5>;
+  constexpr int HID = G::HP, CL = G::CL, MT = G::MT, UPC = G::UPC, COLS = G::COLS, NTW = G::NTW, UPW = G::UPW;
   constexpr int PITCH = G::FPITCH;
   extern __shared__ __align__(16) unsigned char smem_raw[];
   unsigned char* Wsm = smem_raw;                                   // [2 planes][COLS][PITCH]
@@ -500,19 +547,23 @@ lstm_fwd_mma_kernel(float* __restrict__ gx, const float* __restrict__ w_hh, cons
 // ------------------------------------------------------------------------------------------------
 // forward, W slice in tensor memory, two CTAs per SM (see the comment at the W fill)
 // ------------------------------------------------------------------------------------------------
-template <bool SINGLE>   // SINGLE: one 16-bit product (hi x hi) instead of the three split products -- the bf16 variant
-__global__ void __launch_bounds__(G2::NT, 2)
+// HC: the hidden size as a compile-time constant (200: no ghost units, the arithmetic and addressing of a fixed-size kernel), or 0
+// (taken from H_arg at run time)
+template <bool SINGLE, int CL, int HC>   // SINGLE: one 16-bit product (hi x hi) instead of the three split products -- the bf16 variant
+__global__ void __launch_bounds__(G2<CL>::NT, 2)
 lstm_fwd_tm_kernel(float* __restrict__ gx, const float* __restrict__ w_hh, const int32_t* __restrict__ len,
-                    const int32_t* __restrict__ off, const int32_t* __restrict__ order, int N, int ntiles,
+                    const int32_t* __restrict__ off, const int32_t* __restrict__ order, int N, int H_arg, int ntiles,
                     float* __restrict__ h_out, float* __restrict__ c_stash, float* __restrict__ c_n, int* __restrict__ tile_counter,
                     __nv_bfloat16* __restrict__ hp, size_t hp_stride, int hp_lo) {
   // hp != NULL: h also leaves as the bf16 operand planes of the tensor-core GEMMs that consume it ([hi|lo][cap][2H], plane
   // stride hp_stride elements, lo plane only if hp_lo) -- the split pass over h is skipped (same rounding as tc_split_store4)
-  constexpr int HID = G2::HID, CL = G2::CL, MT = G2::MT, UPC = G2::UPC, COLS = G2::COLS, NTW = G2::NTW, UPW = G2::UPW;
+  using G2 = ::G2<CL>;
+  constexpr int MT = G2::MT, UPC = G2::UPC, NTW = G2::NTW, UPW = G2::UPW;
+  const int H = HC ? HC : H_arg;
   extern __shared__ __align__(16) unsigned char smem_raw[];
   unsigned char* Hsm = smem_raw;                                   // [2 buffers][CL blocks][2 planes][MT][80 B]
-  unsigned char* Zero16 = Hsm + 2 * G2::F_HBUF;                     // the K pad chunk
-  unsigned char* Stg = Zero16 + 16;                                // [F_NARR][MT][SROW] staging tile
+  unsigned char* Zero16 = Hsm + 2 * G2::F_HBUF;                     // the K pad chunk (HALF only)
+  unsigned char* Stg = Zero16 + G2::F_ZERO;                        // [F_NARR][MT][SROW] staging tile
   int* s_row = reinterpret_cast<int*>(Stg + G2::F_NARR * G2::SARR);
   int* s_len = s_row + MT;
   int* s_off = s_len + MT;
@@ -530,8 +581,8 @@ lstm_fwd_tm_kernel(float* __restrict__ gx, const float* __restrict__ w_hh, const
   // can only reach the lane quarter of its own index) keeps, for every k-step ks and n8 tile nt of the warp's 40 gate
   // columns, the registers b0 = W[n][16 ks + 2 (l % 4) + {0, 1}], b1 = the same 8 further along k, n = 40 w + 8 nt + l / 4
   // (rows in (warp, n-tile, gate, unit) order, k permuted by fwd_slot_unit like the h operand), as fp16 hi and lo:
-  // columns ks * 20 + {0..9: hi (nt, b0/b1), 10..19: lo}; the last k-step (k = 192..207, upper half = zero pad) only
-  // stores b0: columns 240 + {0..4: hi, 5..9: lo}.  250 of the 256 allocated columns.  This frees the 2 x 69 KB the W
+  // columns ks * 20 + {0..9: hi (nt, b0/b1), 10..19: lo}; with HALF the last k-step (upper 8 k = zero pad) only stores b0:
+  // columns 20 ks + {0..4: hi, 5..9: lo}.  250 of the 256 allocated columns at CL = 5.  This frees the 2 x 69 KB the W
   // planes took in shared memory: two CTAs (of two different clusters) now share an SM, and the tensor pipe is busy with
   // one CTA's products while the other CTA is in its exchange wait / cell / store phases.
   __shared__ uint32_t tmem_slot;
@@ -544,22 +595,24 @@ lstm_fwd_tm_kernel(float* __restrict__ gx, const float* __restrict__ w_hh, const
   asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
   const uint32_t tm_w = tmem_slot + ((uint32_t)((w & 3) * 32) << 16);       // this warp's lane quarter
   if (w < 4) {
-    const float* W = w_hh + (size_t)dir * 4 * HID * HID;
+    const float* W = w_hh + (size_t)dir * 4 * H * H;
     const int c = lane >> 2, g = c >> 1, u = c & 1;
 #pragma unroll 1
     for (int ks = 0; ks < G2::FKS; ++ks) {
 #pragma unroll
       for (int nt = 0; nt < NTW; ++nt) {
-        const float* wrow = W + (size_t)(g * HID + rank * UPC + w * UPW + 2 * nt + u) * HID;
+        const int unit = rank * UPC + w * UPW + 2 * nt + u;       // gate row; ghost rows are zero
+        const float* wrow = W + (size_t)(g * H + unit) * H;
         uint32_t hi[2], lo[2];
 #pragma unroll
         for (int j = 0; j < 2; ++j) {
           const int kk = 16 * ks + 8 * j + 2 * (lane & 3);
-          const float v0 = (kk < HID) ? wrow[fwd_slot_unit(kk)] : 0.f;
-          const float v1 = (kk + 1 < HID) ? wrow[fwd_slot_unit(kk + 1)] : 0.f;
+          const int k0 = fwd_slot_unit(kk), k1 = fwd_slot_unit(kk + 1);   // K slots of ghost units (and of the pad) are zero
+          const float v0 = (unit < H && k0 < H) ? wrow[k0] : 0.f;
+          const float v1 = (unit < H && k1 < H) ? wrow[k1] : 0.f;
           split2<true>(v0, v1, hi[j], lo[j]);
         }
-        if (ks < G2::FKS - 1) {
+        if (!G2::HALF || ks < G2::FKS - 1) {
           asm volatile("tcgen05.st.sync.aligned.32x32b.x2.b32 [%0], {%1, %2};" ::"r"(tm_w + (uint32_t)(ks * 20 + nt * 2)), "r"(hi[0]), "r"(hi[1]) : "memory");
           asm volatile("tcgen05.st.sync.aligned.32x32b.x2.b32 [%0], {%1, %2};" ::"r"(tm_w + (uint32_t)(ks * 20 + 10 + nt * 2)), "r"(lo[0]), "r"(lo[1]) : "memory");
         } else {
@@ -570,7 +623,9 @@ lstm_fwd_tm_kernel(float* __restrict__ gx, const float* __restrict__ w_hh, const
     }
     asm volatile("tcgen05.wait::st.sync.aligned;" ::: "memory");
   }
-  for (int idx = tid; idx < (2 * G2::F_HBUF + 16) / 16; idx += G2::NT) reinterpret_cast<uint4*>(Hsm)[idx] = make_uint4(0u, 0u, 0u, 0u);
+  // h buffers, the pad chunk and the staging tile start zero (the staging bytes of ghost units are never loaded)
+  for (int idx = tid; idx < (2 * G2::F_HBUF + G2::F_ZERO + G2::F_NARR * G2::SARR) / 16; idx += G2::NT)
+    reinterpret_cast<uint4*>(Hsm)[idx] = make_uint4(0u, 0u, 0u, 0u);
   __shared__ __align__(8) uint64_t hfull[2];        // "all of h for the next step has landed in buffer b"
   __shared__ int s_tile;
   const uint32_t h_local = smem_addr_u32(Hsm), bar_local = smem_addr_u32(&hfull[0]);
@@ -584,7 +639,7 @@ lstm_fwd_tm_kernel(float* __restrict__ gx, const float* __restrict__ w_hh, const
   cluster_arrive();
   cluster_wait();
   uint32_t hph[2] = {0u, 0u};
-  const size_t GS = (size_t)2 * 4 * HID;
+  const size_t GS = (size_t)2 * 4 * H;
   PROF_DECL
 
   // per-lane fragment offsets (bytes)
@@ -593,6 +648,7 @@ lstm_fwd_tm_kernel(float* __restrict__ gx, const float* __restrict__ w_hh, const
   const uint32_t zero_local = smem_addr_u32(Zero16), stg_local = smem_addr_u32(Stg);
   const bool copy_role = w >= 4;                                 // warps 4-7 move the staging tile to / from global memory
   const int c_ch = tid & 15, c_rs = (tid - G2::CT) >> 4;          // cooperative copy: chunk and row slot of a copy thread
+  const bool ch_ok = c_ch < 10 && rank * UPC + c_ch * 4 < H;     // the chunk's 4 units are all real or all ghost (H % 4 == 0)
   const uint32_t c_so = (uint32_t)(c_rs * G2::SROW + c_ch * 16);  // its offset inside an array of the staging tile
   const bool pf_lane = (c_ch == 0 || c_ch == 4 || c_ch == 8 || c_ch == 9);   // copy threads that issue the L2 prefetches
   // where this lane's h values go inside this CTA's block of an h tile (plane 0; plane 1 is F_HPLANE further)
@@ -630,14 +686,14 @@ lstm_fwd_tm_kernel(float* __restrict__ gx, const float* __restrict__ w_hh, const
       int c_len[8], c_off[8];
 #pragma unroll
       for (int rr = 0; rr < 8; ++rr) { c_len[rr] = s_len[c_rs + 4 * rr]; c_off[rr] = s_off[c_rs + 4 * rr]; }
-      if (c_ch < 10) {                    // gx of step 0
+      if (ch_ok) {                        // gx of step 0
 #pragma unroll
         for (int rr = 0; rr < 8; ++rr) {
           if (0 < c_len[rr]) {
             const int t = dir ? (c_len[rr] - 1) : 0;
-            const float* g1 = gx + ((size_t)c_off[rr] + t) * GS + (size_t)dir * 4 * HID + rank * UPC + c_ch * 4;
+            const float* g1 = gx + ((size_t)c_off[rr] + t) * GS + (size_t)dir * 4 * H + rank * UPC + c_ch * 4;
 #pragma unroll
-            for (int a = 0; a < 4; ++a) cp_async16(stg_local + c_so + rr * 4 * G2::SROW + a * G2::SARR, g1 + a * HID);
+            for (int a = 0; a < 4; ++a) cp_async16(stg_local + c_so + rr * 4 * G2::SROW + a * G2::SARR, g1 + a * H);
           }
         }
       }
@@ -646,7 +702,7 @@ lstm_fwd_tm_kernel(float* __restrict__ gx, const float* __restrict__ w_hh, const
       bar_arrive(3, G2::NT);
       for (int s = 0; s < maxlen; ++s) {
         bar_sync(2, G2::NT);              // the staging tile holds the stash of step s
-        if (c_ch < 10) {
+        if (ch_ok) {
 #pragma unroll
           for (int rr = 0; rr < 8; ++rr) {
             const int rl = c_len[rr];
@@ -654,13 +710,13 @@ lstm_fwd_tm_kernel(float* __restrict__ gx, const float* __restrict__ w_hh, const
               const int t = dir ? (rl - 1 - s) : s;
               const size_t p = (size_t)c_off[rr] + t;
               const unsigned char* sp = Stg + c_so + rr * 4 * G2::SROW;
-              float* g0 = gx + p * GS + (size_t)dir * 4 * HID + rank * UPC + c_ch * 4;
+              float* g0 = gx + p * GS + (size_t)dir * 4 * H + rank * UPC + c_ch * 4;
 #pragma unroll
-              for (int a = 0; a < 4; ++a) *reinterpret_cast<float4*>(g0 + a * HID) = *reinterpret_cast<const float4*>(sp + a * G2::SARR);
+              for (int a = 0; a < 4; ++a) *reinterpret_cast<float4*>(g0 + a * H) = *reinterpret_cast<const float4*>(sp + a * G2::SARR);
               const float4 cv = *reinterpret_cast<const float4*>(sp + 4 * G2::SARR);
-              *reinterpret_cast<float4*>(c_stash + (p * 2 + dir) * HID + rank * UPC + c_ch * 4) = cv;
+              *reinterpret_cast<float4*>(c_stash + (p * 2 + dir) * H + rank * UPC + c_ch * 4) = cv;
               const float4 hv = *reinterpret_cast<const float4*>(sp + 5 * G2::SARR);
-              const size_t ho = p * 2 * HID + (size_t)dir * HID + rank * UPC + c_ch * 4;
+              const size_t ho = p * 2 * H + (size_t)dir * H + rank * UPC + c_ch * 4;
               *reinterpret_cast<float4*>(h_out + ho) = hv;
               if (hp) {
                 const __nv_bfloat162 h01 = __floats2bfloat162_rn(hv.x, hv.y), h23 = __floats2bfloat162_rn(hv.z, hv.w);
@@ -676,16 +732,16 @@ lstm_fwd_tm_kernel(float* __restrict__ gx, const float* __restrict__ w_hh, const
                 }
               }
               if (s == rl - 1)
-                *reinterpret_cast<float4*>(c_n + (size_t)s_row[c_rs + 4 * rr] * 2 * HID + (size_t)dir * HID + rank * UPC + c_ch * 4) = cv;
+                *reinterpret_cast<float4*>(c_n + (size_t)s_row[c_rs + 4 * rr] * 2 * H + (size_t)dir * H + rank * UPC + c_ch * 4) = cv;
               if (s + 1 < rl) {            // the row's next token is the adjacent one
                 const float* g1 = dir ? g0 - GS : g0 + GS;
 #pragma unroll
-                for (int a = 0; a < 4; ++a) cp_async16(stg_local + c_so + rr * 4 * G2::SROW + a * G2::SARR, g1 + a * HID);
+                for (int a = 0; a < 4; ++a) cp_async16(stg_local + c_so + rr * 4 * G2::SROW + a * G2::SARR, g1 + a * H);
               }
               if (NNR_LSTM_PFD > 0 && pf_lane && s + NNR_LSTM_PFD < rl) {   // 160 B segment: chunks 0, 4, 8, 9 touch every line of it
                 const float* g3 = dir ? g0 - (size_t)NNR_LSTM_PFD * GS : g0 + (size_t)NNR_LSTM_PFD * GS;
 #pragma unroll
-                for (int a = 0; a < 4; ++a) prefetch_l2(g3 + a * HID);
+                for (int a = 0; a < 4; ++a) prefetch_l2(g3 + a * H);
               }
             }
           }
@@ -730,7 +786,7 @@ lstm_fwd_tm_kernel(float* __restrict__ gx, const float* __restrict__ w_hh, const
 #pragma unroll
         for (int mt = 0; mt < 2; ++mt) {
           uint32_t ad_h, ad_l;
-          if (c1 < 25) {
+          if (c1 < 5 * CL) {
             ad_h = hA + mt * 16 * G2::F_HROW + (a_hi ? o1 : o0);
             ad_l = ad_h + G2::F_HPLANE;
           } else {                      // K pad: the upper chunk reads zeros
@@ -741,7 +797,7 @@ lstm_fwd_tm_kernel(float* __restrict__ gx, const float* __restrict__ w_hh, const
           if (!SINGLE) ldsm_x4(ad_l, f.al[mt][0], f.al[mt][1], f.al[mt][2], f.al[mt][3]);
         }
         // B fragments of this k-step from tensor memory (asynchronous: tm_wait() before their first use)
-        if (ks < G2::FKS - 1) {
+        if (!G2::HALF || ks < G2::FKS - 1) {
           uint32_t r[20];
           if (!SINGLE) {
             asm volatile("tcgen05.ld.sync.aligned.32x32b.x16.b32 {%0, %1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15}, [%16];"
@@ -761,7 +817,7 @@ lstm_fwd_tm_kernel(float* __restrict__ gx, const float* __restrict__ w_hh, const
             f.bh[nt][0] = r[2 * nt]; f.bh[nt][1] = r[2 * nt + 1];
             if (!SINGLE) { f.bl[nt][0] = r[10 + 2 * nt]; f.bl[nt][1] = r[10 + 2 * nt + 1]; }
           }
-        } else {                         // k = 192..207: the upper 8 are padding, b1 = 0
+        } else {                         // half k-step: the upper 8 k are padding, b1 = 0
           uint32_t r[10];
           asm volatile("tcgen05.ld.sync.aligned.32x32b.x8.b32 {%0, %1, %2, %3, %4, %5, %6, %7}, [%8];"
                        : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]), "=r"(r[7])
@@ -826,6 +882,7 @@ lstm_fwd_tm_kernel(float* __restrict__ gx, const float* __restrict__ w_hh, const
         unsigned char* sp = Stg + R * G2::SROW + w * (UPW * 4);
 #pragma unroll
         for (int nt = 0; nt < NTW; ++nt) {
+          const bool live = unit0 + 2 * nt < H;   // units 2 nt, 2 nt + 1 are both real or both ghost (H even)
           float2* gi = reinterpret_cast<float2*>(sp + 0 * G2::SARR + nt * 8);
           float2* gf = reinterpret_cast<float2*>(sp + 1 * G2::SARR + nt * 8);
           float2* gg_ = reinterpret_cast<float2*>(sp + 2 * G2::SARR + nt * 8);
@@ -842,8 +899,10 @@ lstm_fwd_tm_kernel(float* __restrict__ gx, const float* __restrict__ w_hh, const
             fg[u] = fast_sigmoid(zf[u]);
             gg[u] = fast_tanh(zg[u]);
             og[u] = fast_sigmoid(zo[u]);
-            cst[2 * nt + u] = fg[u] * cst[2 * nt + u] + ig[u] * gg[u];
-            hst[2 * nt + u] = og[u] * fast_tanh(cst[2 * nt + u]);
+            const float cnew = fg[u] * cst[2 * nt + u] + ig[u] * gg[u];
+            const float hnew = og[u] * fast_tanh(cnew);
+            cst[2 * nt + u] = live ? cnew : 0.f;   // ghost units stay exactly zero
+            hst[2 * nt + u] = live ? hnew : 0.f;
           }
           *gi = make_float2(ig[0], ig[1]);
           *gf = make_float2(fg[0], fg[1]);
@@ -896,24 +955,29 @@ lstm_fwd_tm_kernel(float* __restrict__ gx, const float* __restrict__ w_hh, const
 // two different clusters) share an SM -- one CTA's products keep the tensor pipe busy while the other is in its exchange wait /
 // point-wise / store phases.  Same protocol, same arithmetic as the shared-memory variant (the per-tile bias-gradient partials group the
 // rows by 4 copy-thread slots instead of 8: deterministic, last-bit different).
-template <bool SINGLE, bool TM>   // SINGLE: one 16-bit product (hi x hi) instead of the three split products -- the bf16 variant
-__global__ void __launch_bounds__(TM ? G3::NT : G::NT, TM ? 2 : 1)
+template <bool SINGLE, bool TM, int CL, int HC>   // SINGLE: one 16-bit product (hi x hi) instead of the three split products -- the bf16 variant
+__global__ void __launch_bounds__(TM ? G3<CL>::NT : G<CL>::NT, TM ? 2 : 1)
 lstm_bwd_mma_kernel(float* __restrict__ gates, const float* __restrict__ c_stash, const float* __restrict__ w_hh,
                     const int32_t* __restrict__ len, const int32_t* __restrict__ off, const int32_t* __restrict__ order,
-                    int N, int ntiles, const float* __restrict__ dh, const float* __restrict__ dcn, int* __restrict__ tile_counter,
+                    int N, int H_arg, int ntiles, const float* __restrict__ dh, const float* __restrict__ dcn, int* __restrict__ tile_counter,
                     __nv_bfloat16* __restrict__ dzp, size_t dzp_stride, int dzp_lo, float* __restrict__ db_partial) {
   // dzp != NULL: dL/dgx leaves as the bf16 operand planes of the tensor-core GEMMs ([hi|lo][cap][8H], plane stride
   // dzp_stride elements, lo plane only if dzp_lo) instead of fp32 into `gates`, and the column sums of every tile (the
   // bias gradient) go to db_partial[tile][8H] -- fixed summation order, so the result does not depend on which cluster
   // ran the tile.
-  constexpr int HID = G::HID, CL = G::CL, MT = G::MT, UPC = G::UPC, UPW = G::UPW, NTW = G::NTW;
+  static_assert(TM || (CL == 5 && HC == 200), "the shared-memory W variant exists for hidden_dim 200 only");
+  using G = ::G<CL>;
+  using G3 = ::G3<CL>;
+  constexpr int HP = G::HP, MT = G::MT, UPC = G::UPC, UPW = G::UPW, NTW = G::NTW;
+  const int H = HC ? HC : H_arg;                                   // HC: see lstm_fwd_tm_kernel
   constexpr int PITCH = G::BPITCH, WP = G::BWPITCH, RP = G::RPITCH;
   constexpr int NTH = TM ? G3::NT : G::NT;                         // threads of the CTA
   constexpr int NCOPY = NTH - G::CT;                               // copy threads: 16 chunk lanes x RSLOT row slots
   constexpr int RSLOT = NCOPY / 16, RPT = MT / RSLOT;              // row slots, rows per copy thread (8 x 4, or 4 x 8 with TM)
   constexpr int W_PLANE = TM ? G3::W7_PLANE : G::B_W_PLANE;
+  constexpr int NTWB = G::NTWB;                                    // n8 tiles of the warp with the most
   extern __shared__ __align__(16) unsigned char smem_raw[];
-  unsigned char* Wsm = smem_raw;                                   // [2 planes][HID units][WP] swizzled  (B operand); TM: units 48..55 only
+  unsigned char* Wsm = smem_raw;                                   // [2 planes][HP units][WP] swizzled  (B operand); TM: the NSM tile only
   unsigned char* Zsm = Wsm + 2 * W_PLANE;                          // [2 planes][MT][PITCH]          (A operand: dz)
   unsigned char* Rsm = Zsm + 2 * G::B_Z_PLANE;                     // [CL sources][MT][40] fp32 partial dh from each CTA
   unsigned char* Ssm = Rsm + G::B_RECV;                            // [CL owners][MT][40]  fp32 partials staged for the bulk copies
@@ -931,19 +995,23 @@ lstm_bwd_mma_kernel(float* __restrict__ gates, const float* __restrict__ c_stash
   const int R = r8 + 8 * q;
   const int unit0 = rank * UPC + w * UPW;
 
-  // phase 2 tiling: 25 n8 tiles of output units over 4 warps: 7, 6, 6, 6
-  const int nt0 = w * 6 + (w > 0 ? 1 : 0);
-  const bool seven = (w == 0);
+  // phase 2 tiling: 5 CL n8 tiles of output units over 4 warps (G::NTILE); tile nt of warp w exists iff active(nt)
+  const int nt0 = w * G::BASE + min(w, G::EXTRA);
+  auto active = [&](int nt) { return nt < G::BASE || w < G::EXTRA; };
   // W slice (bf16 hi / lo): row n = hidden unit k of the OUTPUT dh, column kk = own gate column in
-  // (warp, gate, unit) order -- the order phase 1 writes dz in
+  // (warp, gate, unit) order -- the order phase 1 writes dz in.  Ghost gate columns and ghost output units are zero.
+  const float* W = w_hh + (size_t)dir * 4 * H * H;
+  auto wval = [&](int kk, int n) -> float {
+    const int ww = kk / 40, rem = kk - ww * 40, g = rem / UPW, i = rem - g * UPW;
+    const int unit = rank * UPC + ww * UPW + i;
+    return (unit < H && n < H) ? W[(size_t)(g * H + unit) * H + n] : 0.f;
+  };
   __shared__ uint32_t tmem_slot;
   uint32_t tm_w = 0;
   if (!TM) {
-    const float* W = w_hh + (size_t)dir * 4 * HID * HID;
-    for (int idx = tid; idx < G::BK * HID; idx += NTH) {
-      const int kk = idx / HID, n = idx - kk * HID;
-      const int ww = kk / 40, rem = kk - ww * 40, g = rem / UPW, i = rem - g * UPW;
-      const float v = W[(size_t)(g * HID + rank * UPC + ww * UPW + i) * HID + n];
+    for (int idx = tid; idx < G::BK * HP; idx += NTH) {
+      const int kk = idx / HP, n = idx - kk * HP;
+      const float v = wval(kk, n);
       uint16_t hi, lo;
       split1<false>(v, hi, lo);
       const size_t o = (size_t)n * WP + (((kk >> 3) ^ ((n >> 1) & 3)) << 4) + (kk & 7) * 2;
@@ -952,9 +1020,10 @@ lstm_bwd_mma_kernel(float* __restrict__ gates, const float* __restrict__ c_stash
     }
   } else {
     // -> TENSOR MEMORY, already in mma.sync B-fragment form.  Lane l of compute warp w (TMEM lanes 32 w + l) keeps, for every
-    // k-step ks and each of the warp's first six n8 tiles nt, the registers b0 = W^T[16 ks + 2 (l % 4) + {0, 1}][n], b1 = the
-    // same 8 further along k, n = 8 (nt0 + nt) + l / 4, as bf16 hi and lo: columns (ks * 6 + nt) * 4 + {0: hi b0, 1: hi b1,
-    // 2: lo b0, 3: lo b1}.  Warp 0's seventh tile (units 48..55) stays in shared memory in the layout of the full slice.
+    // k-step ks and each of the warp's first NTM n8 tiles nt, the registers b0 = W^T[16 ks + 2 (l % 4) + {0, 1}][n], b1 = the
+    // same 8 further along k, n = 8 (nt0 + nt) + l / 4, as bf16 hi and lo: columns (ks * NTM + nt) * 4 + {0: hi b0, 1: hi b1,
+    // 2: lo b0, 3: lo b1}.  With CL = 5 warp 0's seventh tile (units 48..55) stays in shared memory in the layout of the
+    // full slice.
     if (w == 0) {
       asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_addr_u32(&tmem_slot)), "n"(G3::TM_COLS) : "memory");
       asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
@@ -963,32 +1032,27 @@ lstm_bwd_mma_kernel(float* __restrict__ gates, const float* __restrict__ c_stash
     __syncthreads();
     asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
     tm_w = tmem_slot + ((uint32_t)((w & 3) * 32) << 16);           // this warp's lane quarter
-    const float* W = w_hh + (size_t)dir * 4 * HID * HID;
-    auto wval = [&](int kk, int n) -> float {
-      const int ww = kk / 40, rem = kk - ww * 40, g = rem / UPW, i = rem - g * UPW;
-      return W[(size_t)(g * HID + rank * UPC + ww * UPW + i) * HID + n];
-    };
     if (w < 4) {
 #pragma unroll 1
       for (int ks = 0; ks < G::BKS; ++ks) {
 #pragma unroll 1
-        for (int nt = 0; nt < 6; ++nt) {
+        for (int nt = 0; nt < G3::NTM; ++nt) {
           const int n = 8 * (nt0 + nt) + (lane >> 2);
           const int k0 = 16 * ks + 2 * (lane & 3);
           uint32_t h0, l0, h1, l1;
           split2<false>(wval(k0, n), wval(k0 + 1, n), h0, l0);
           split2<false>(wval(k0 + 8, n), wval(k0 + 9, n), h1, l1);
-          asm volatile("tcgen05.st.sync.aligned.32x32b.x4.b32 [%0], {%1, %2, %3, %4};" ::"r"(tm_w + (uint32_t)((ks * 6 + nt) * 4)), "r"(h0),
+          asm volatile("tcgen05.st.sync.aligned.32x32b.x4.b32 [%0], {%1, %2, %3, %4};" ::"r"(tm_w + (uint32_t)((ks * G3::NTM + nt) * 4)), "r"(h0),
                        "r"(h1), "r"(l0), "r"(l1)
                        : "memory");
         }
       }
       asm volatile("tcgen05.wait::st.sync.aligned;" ::: "memory");
     }
-    for (int idx = tid; idx < G::BK * 8; idx += NTH) {             // units 48..55 (warp 0's seventh n-tile)
+    for (int idx = tid; idx < G3::NSM * G::BK * 8; idx += NTH) {   // units 8 NTM .. 8 NTM + 7 (warp 0's seventh n-tile)
       const int kk = idx >> 3, r = idx & 7;
       uint16_t hi, lo;
-      split1<false>(wval(kk, 48 + r), hi, lo);
+      split1<false>(wval(kk, 8 * G3::NTM + r), hi, lo);
       const size_t o = (size_t)r * WP + (((kk >> 3) ^ ((r >> 1) & 3)) << 4) + (kk & 7) * 2;
       *reinterpret_cast<uint16_t*>(Wsm + o) = hi;
       *reinterpret_cast<uint16_t*>(Wsm + G3::W7_PLANE + o) = lo;
@@ -1009,7 +1073,7 @@ lstm_bwd_mma_kernel(float* __restrict__ gates, const float* __restrict__ c_stash
   cluster_arrive();      // all CTAs of the cluster are running before the first remote shared-memory store (see the forward kernel)
   cluster_wait();
   uint32_t ph_full = 0u, ph_free = 0u;
-  const size_t GS = (size_t)2 * 4 * HID;
+  const size_t GS = (size_t)2 * 4 * H;
   PROF_DECL
 
   const uint32_t a_off = (uint32_t)((lane & 15) * PITCH + (lane >> 4) * 16);
@@ -1020,8 +1084,9 @@ lstm_bwd_mma_kernel(float* __restrict__ gates, const float* __restrict__ c_stash
   const bool copy_role = w >= 4;                                 // warps 4-7 move the staging tile to / from global memory
   const int c_ch = tid & 15, c_rs = (tid - G::CT) >> 4;
   const uint32_t c_so = (uint32_t)(c_rs * G::SROW + c_ch * 16);
+  const bool ch_ok = c_ch < 10 && rank * UPC + c_ch * 4 < H;     // the chunk's 4 units are all real or all ghost (H % 4 == 0)
   const bool pf_lane = (c_ch == 0 || c_ch == 4 || c_ch == 8 || c_ch == 9);   // copy threads that issue the L2 prefetches
-  const bool leader = (tid == 96);                               // barrier / copy-engine duties (a warp with six n-tiles)
+  const bool leader = (tid == 96);                               // barrier / copy-engine duties (a warp with the fewest n-tiles)
 
   for (;;) {
     if (rank == 0 && tid == 0) {
@@ -1052,25 +1117,25 @@ lstm_bwd_mma_kernel(float* __restrict__ gates, const float* __restrict__ c_stash
 #pragma unroll
       for (int rr = 0; rr < RPT; ++rr) { c_len[rr] = s_len[c_rs + RSLOT * rr]; c_off[rr] = s_off[c_rs + RSLOT * rr]; }
       auto prefetch_stash = [&](int s1) {
-        if (c_ch < 10) {
+        if (ch_ok) {
 #pragma unroll
           for (int rr = 0; rr < RPT; ++rr) {
             if (s1 < c_len[rr]) {
               const int t = dir ? (c_len[rr] - 1 - s1) : s1;
               const size_t p = (size_t)c_off[rr] + t;
-              const float* g1 = gates + p * GS + (size_t)dir * 4 * HID + rank * UPC + c_ch * 4;
+              const float* g1 = gates + p * GS + (size_t)dir * 4 * H + rank * UPC + c_ch * 4;
 #pragma unroll
-              for (int a = 0; a < 4; ++a) cp_async16(stg_local + c_so + rr * RSLOT * G::SROW + a * G::SARR, g1 + a * HID);
-              cp_async16(stg_local + c_so + rr * RSLOT * G::SROW + 4 * G::SARR, dh + p * 2 * HID + (size_t)dir * HID + rank * UPC + c_ch * 4);
+              for (int a = 0; a < 4; ++a) cp_async16(stg_local + c_so + rr * RSLOT * G::SROW + a * G::SARR, g1 + a * H);
+              cp_async16(stg_local + c_so + rr * RSLOT * G::SROW + 4 * G::SARR, dh + p * 2 * H + (size_t)dir * H + rank * UPC + c_ch * 4);
             }
             const int s3 = s1 - NNR_LSTM_PFD;                  // the iteration NNR_LSTM_PFD steps ahead: pull its lines into L2
             if (NNR_LSTM_PFD > 0 && pf_lane && s3 >= 0 && s3 < c_len[rr]) {
               const int t3 = dir ? (c_len[rr] - 1 - s3) : s3;
               const size_t p3 = (size_t)c_off[rr] + t3;
-              const float* g3 = gates + p3 * GS + (size_t)dir * 4 * HID + rank * UPC + c_ch * 4;
+              const float* g3 = gates + p3 * GS + (size_t)dir * 4 * H + rank * UPC + c_ch * 4;
 #pragma unroll
-              for (int a = 0; a < 4; ++a) prefetch_l2(g3 + a * HID);
-              prefetch_l2(dh + p3 * 2 * HID + (size_t)dir * HID + rank * UPC + c_ch * 4);
+              for (int a = 0; a < 4; ++a) prefetch_l2(g3 + a * H);
+              prefetch_l2(dh + p3 * 2 * H + (size_t)dir * H + rank * UPC + c_ch * 4);
             }
           }
         }
@@ -1086,14 +1151,14 @@ lstm_bwd_mma_kernel(float* __restrict__ gates, const float* __restrict__ c_stash
         for (int j = 0; j < 4; ++j) csum[a][j] = 0.f;
       for (int s = maxlen - 1; s >= 0; --s) {
         bar_sync(2, NTH);              // the staging tile holds dL/dgx of iteration s
-        if (c_ch < 10) {
+        if (ch_ok) {
 #pragma unroll
           for (int rr = 0; rr < RPT; ++rr) {
             if (s < c_len[rr]) {
               const int t = dir ? (c_len[rr] - 1 - s) : s;
               const size_t p = (size_t)c_off[rr] + t;
               const unsigned char* spc = Stg + c_so + rr * RSLOT * G::SROW;
-              const size_t go = p * GS + (size_t)dir * 4 * HID + rank * UPC + c_ch * 4;
+              const size_t go = p * GS + (size_t)dir * 4 * H + rank * UPC + c_ch * 4;
               if (dzp) {
 #pragma unroll
                 for (int a = 0; a < 4; ++a) {
@@ -1101,7 +1166,7 @@ lstm_bwd_mma_kernel(float* __restrict__ gates, const float* __restrict__ c_stash
                   csum[a][0] += v.x; csum[a][1] += v.y; csum[a][2] += v.z; csum[a][3] += v.w;
                   // same rounding as tc_split_store4 (gemm_tc.cu): hi = rn(x), lo = rn(x - hi)
                   const __nv_bfloat162 h01 = __floats2bfloat162_rn(v.x, v.y), h23 = __floats2bfloat162_rn(v.z, v.w);
-                  __nv_bfloat16* o = dzp + go + a * HID;
+                  __nv_bfloat16* o = dzp + go + a * H;
                   uint2 hv;
                   hv.x = *reinterpret_cast<const uint32_t*>(&h01); hv.y = *reinterpret_cast<const uint32_t*>(&h23);
                   *reinterpret_cast<uint2*>(o) = hv;
@@ -1116,7 +1181,7 @@ lstm_bwd_mma_kernel(float* __restrict__ gates, const float* __restrict__ c_stash
               } else {
                 float* g0 = gates + go;
 #pragma unroll
-                for (int a = 0; a < 4; ++a) *reinterpret_cast<float4*>(g0 + a * HID) = *reinterpret_cast<const float4*>(spc + a * G::SARR);
+                for (int a = 0; a < 4; ++a) *reinterpret_cast<float4*>(g0 + a * H) = *reinterpret_cast<const float4*>(spc + a * G::SARR);
               }
             }
           }
@@ -1139,7 +1204,7 @@ lstm_bwd_mma_kernel(float* __restrict__ gates, const float* __restrict__ c_stash
 #pragma unroll
           for (int rs = 0; rs < RSLOT; ++rs) sum += scr[rs * G::COLS + col];
           const int a = col / UPC, u = col - a * UPC;
-          db_partial[(size_t)tile * GS + (size_t)dir * 4 * HID + a * HID + rank * UPC + u] = sum;
+          if (rank * UPC + u < H) db_partial[(size_t)tile * GS + (size_t)dir * 4 * H + a * H + rank * UPC + u] = sum;
         }
       }
       continue;
@@ -1163,14 +1228,16 @@ lstm_bwd_mma_kernel(float* __restrict__ gates, const float* __restrict__ c_stash
         const int t = dir ? (rlen - 1 - s) : s;
         const size_t p = (size_t)roff + t;
         if (s > 0) {
-          const float* cpp = c_stash + ((dir ? p + 1 : p - 1) * 2 + dir) * HID + unit0;
+          const float* cpp = c_stash + ((dir ? p + 1 : p - 1) * 2 + dir) * H + unit0;
 #pragma unroll
-          for (int nt = 0; nt < NTW; ++nt) p_cp[nt] = *reinterpret_cast<const float2*>(cpp + 2 * nt);
+          for (int nt = 0; nt < NTW; ++nt)
+            if (unit0 + 2 * nt < H) p_cp[nt] = *reinterpret_cast<const float2*>(cpp + 2 * nt);
         }
         if (s == rlen - 1) {          // first iteration of the row: its c_t has not been seen as a c_{t-1} yet
-          const float* cp = c_stash + (p * 2 + dir) * HID + unit0;
+          const float* cp = c_stash + (p * 2 + dir) * H + unit0;
 #pragma unroll
-          for (int nt = 0; nt < NTW; ++nt) ccur[nt] = *reinterpret_cast<const float2*>(cp + 2 * nt);
+          for (int nt = 0; nt < NTW; ++nt)
+            if (unit0 + 2 * nt < H) ccur[nt] = *reinterpret_cast<const float2*>(cp + 2 * nt);
         }
       }
       PROF_MARK(0)
@@ -1189,10 +1256,10 @@ lstm_bwd_mma_kernel(float* __restrict__ gates, const float* __restrict__ c_stash
             dht[2 * nt] = v.x; dht[2 * nt + 1] = v.y;
           }
           if (s == rlen - 1) {       // the row's last step: start of its backward recursion
-            const float* d0 = dcn + (size_t)rrow * 2 * HID + (size_t)dir * HID + unit0;
+            const float* d0 = dcn + (size_t)rrow * 2 * H + (size_t)dir * H + unit0;
 #pragma unroll
             for (int nt = 0; nt < NTW; ++nt) {
-              const float2 v = *reinterpret_cast<const float2*>(d0 + 2 * nt);
+              const float2 v = unit0 + 2 * nt < H ? *reinterpret_cast<const float2*>(d0 + 2 * nt) : make_float2(0.f, 0.f);
               dcc[2 * nt] = v.x; dcc[2 * nt + 1] = v.y;
             }
           } else {                   // recurrent part: the CL partials summed in fixed order
@@ -1220,16 +1287,17 @@ lstm_bwd_mma_kernel(float* __restrict__ gates, const float* __restrict__ c_stash
             const float2 og = *reinterpret_cast<const float2*>(sp + 3 * G::SARR + nt * 8);
             const float iv[2] = {ig.x, ig.y}, fv[2] = {fg.x, fg.y}, gv[2] = {gg.x, gg.y}, ov[2] = {og.x, og.y};
             const float cv[2] = {ccur[nt].x, ccur[nt].y}, cpv[2] = {p_cp[nt].x, p_cp[nt].y};
+            const bool live = unit0 + 2 * nt < H;   // ghost units: dz = dc = 0 exactly
 #pragma unroll
             for (int u = 0; u < 2; ++u) {
               const int i = 2 * nt + u;
               const float tc = fast_tanh(cv[u]);
               const float dc = dcc[i] + dht[i] * ov[u] * (1.f - tc * tc);
-              dz[3][i] = dht[i] * tc * ov[u] * (1.f - ov[u]);
-              dz[0][i] = dc * gv[u] * iv[u] * (1.f - iv[u]);
-              dz[2][i] = dc * iv[u] * (1.f - gv[u] * gv[u]);
-              dz[1][i] = dc * cpv[u] * fv[u] * (1.f - fv[u]);
-              dcc[i] = dc * fv[u];
+              dz[3][i] = live ? dht[i] * tc * ov[u] * (1.f - ov[u]) : 0.f;
+              dz[0][i] = live ? dc * gv[u] * iv[u] * (1.f - iv[u]) : 0.f;
+              dz[2][i] = live ? dc * iv[u] * (1.f - gv[u] * gv[u]) : 0.f;
+              dz[1][i] = live ? dc * cpv[u] * fv[u] * (1.f - fv[u]) : 0.f;
+              dcc[i] = live ? dc * fv[u] : 0.f;
             }
             ccur[nt] = p_cp[nt];
           }
@@ -1271,15 +1339,16 @@ lstm_bwd_mma_kernel(float* __restrict__ gates, const float* __restrict__ c_stash
       if (s == 0) break;
       PROF_MARK(3)
       // ---- phase 2: partial dh_{t-1}[32 x units of this warp's n-tiles] = dz[32 x 160] x W_slice --------------
-      float acc[2][7][4];
+      float acc[2][NTWB][4];
 #pragma unroll
       for (int mt = 0; mt < 2; ++mt)
 #pragma unroll
-        for (int nt = 0; nt < 7; ++nt)
+        for (int nt = 0; nt < NTWB; ++nt)
 #pragma unroll
           for (int e = 0; e < 4; ++e) acc[mt][nt][e] = 0.f;
-      struct Frag { uint32_t ah[2][4], al[2][4], bh[7][2], bl[7][2]; };
-      auto load_frags = [&](Frag& f, int ks) {
+      struct Frag { uint32_t ah[2][4], al[2][4], bh[NTWB][2], bl[NTWB][2]; };
+      auto load_frags = [&](Frag& f, int ks) {   // shared-memory W slice (CL = 5 only)
+        if constexpr (!TM) {
 #pragma unroll
         for (int mt = 0; mt < 2; ++mt) {
           ldsm_x4(z_local + a_off + mt * 16 * PITCH + ks * 32, f.ah[mt][0], f.ah[mt][1], f.ah[mt][2], f.ah[mt][3]);
@@ -1293,9 +1362,10 @@ lstm_bwd_mma_kernel(float* __restrict__ gates, const float* __restrict__ c_stash
             ldsm_x4(w_local + G::B_W_PLANE + b_row + pr * 16 * WP + bc, f.bl[2 * pr][0], f.bl[2 * pr][1], f.bl[2 * pr + 1][0],
                     f.bl[2 * pr + 1][1]);
         }
-        if (seven) {
+        if (active(6)) {
           ldsm_x2(w_local + b_row6 + bc, f.bh[6][0], f.bh[6][1]);
           if (!SINGLE) ldsm_x2(w_local + G::B_W_PLANE + b_row6 + bc, f.bl[6][0], f.bl[6][1]);
+        }
         }
       };
       auto mma_all = [&](const Frag& f) {
@@ -1303,21 +1373,21 @@ lstm_bwd_mma_kernel(float* __restrict__ gates, const float* __restrict__ c_stash
 #pragma unroll
           for (int mt = 0; mt < 2; ++mt)
 #pragma unroll
-            for (int nt = 0; nt < 7; ++nt)
-              if (nt < 6 || seven) mma16816<false>(acc[mt][nt], f.al[mt], f.bh[nt][0], f.bh[nt][1]);
+            for (int nt = 0; nt < NTWB; ++nt)
+              if (active(nt)) mma16816<false>(acc[mt][nt], f.al[mt], f.bh[nt][0], f.bh[nt][1]);
 #pragma unroll
           for (int mt = 0; mt < 2; ++mt)
 #pragma unroll
-            for (int nt = 0; nt < 7; ++nt)
-              if (nt < 6 || seven) mma16816<false>(acc[mt][nt], f.ah[mt], f.bl[nt][0], f.bl[nt][1]);
+            for (int nt = 0; nt < NTWB; ++nt)
+              if (active(nt)) mma16816<false>(acc[mt][nt], f.ah[mt], f.bl[nt][0], f.bl[nt][1]);
         }
 #pragma unroll
         for (int mt = 0; mt < 2; ++mt)
 #pragma unroll
-          for (int nt = 0; nt < 7; ++nt)
-            if (nt < 6 || seven) mma16816<false>(acc[mt][nt], f.ah[mt], f.bh[nt][0], f.bh[nt][1]);
+          for (int nt = 0; nt < NTWB; ++nt)
+            if (active(nt)) mma16816<false>(acc[mt][nt], f.ah[mt], f.bh[nt][0], f.bh[nt][1]);
       };
-      if (!TM) {
+      if constexpr (!TM) {
         Frag f0, f1;
         load_frags(f0, 0);
 #pragma unroll
@@ -1329,7 +1399,7 @@ lstm_bwd_mma_kernel(float* __restrict__ gates, const float* __restrict__ c_stash
         }
       } else {
         // A fragments (dz, shared memory) double-buffered in registers; B fragments of one k-step from tensor memory
-        // (24 registers: six tiles x {hi b0, hi b1, lo b0, lo b1}), the seventh tile of warp 0 from shared memory
+        // (4 NTM registers: NTM tiles x {hi b0, hi b1, lo b0, lo b1}), the seventh tile of warp 0 (CL = 5) from shared memory
         struct FragA { uint32_t ah[2][4], al[2][4]; };
         auto load_a = [&](FragA& f, int ks) {
 #pragma unroll
@@ -1340,15 +1410,10 @@ lstm_bwd_mma_kernel(float* __restrict__ gates, const float* __restrict__ c_stash
           }
         };
         auto step = [&](const FragA& fa, int ks) {
-          uint32_t r[24], b6h[2] = {0u, 0u}, b6l[2] = {0u, 0u};
-          asm volatile("tcgen05.ld.sync.aligned.32x32b.x16.b32 {%0, %1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15}, [%16];"
-                       : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]), "=r"(r[7]), "=r"(r[8]), "=r"(r[9]),
-                         "=r"(r[10]), "=r"(r[11]), "=r"(r[12]), "=r"(r[13]), "=r"(r[14]), "=r"(r[15])
-                       : "r"(tm_w + (uint32_t)(ks * 24)));
-          asm volatile("tcgen05.ld.sync.aligned.32x32b.x8.b32 {%0, %1, %2, %3, %4, %5, %6, %7}, [%8];"
-                       : "=r"(r[16]), "=r"(r[17]), "=r"(r[18]), "=r"(r[19]), "=r"(r[20]), "=r"(r[21]), "=r"(r[22]), "=r"(r[23])
-                       : "r"(tm_w + (uint32_t)(ks * 24 + 16)));
-          if (seven) {
+          constexpr int NTM = G3::NTM;
+          uint32_t r[4 * NTM], b6h[2] = {0u, 0u}, b6l[2] = {0u, 0u};
+          tm_ld<4 * NTM>(r, tm_w + (uint32_t)(ks * 4 * NTM));
+          if (G3::NSM > 0 && active(NTM)) {
             const uint32_t bc = (((uint32_t)(2 * ks) + b_kh) ^ b_x) << 4;
             ldsm_x2(w_local + b_row6 + bc, b6h[0], b6h[1]);
             if (!SINGLE) ldsm_x2(w_local + G3::W7_PLANE + b_row6 + bc, b6l[0], b6l[1]);
@@ -1358,21 +1423,24 @@ lstm_bwd_mma_kernel(float* __restrict__ gates, const float* __restrict__ c_stash
 #pragma unroll
             for (int mt = 0; mt < 2; ++mt) {
 #pragma unroll
-              for (int nt = 0; nt < 6; ++nt) mma16816<false>(acc[mt][nt], fa.al[mt], r[4 * nt], r[4 * nt + 1]);
-              if (seven) mma16816<false>(acc[mt][6], fa.al[mt], b6h[0], b6h[1]);
+              for (int nt = 0; nt < NTM; ++nt)
+                if (active(nt)) mma16816<false>(acc[mt][nt], fa.al[mt], r[4 * nt], r[4 * nt + 1]);
+              if (G3::NSM > 0 && active(NTM)) mma16816<false>(acc[mt][NTWB - 1], fa.al[mt], b6h[0], b6h[1]);
             }
 #pragma unroll
             for (int mt = 0; mt < 2; ++mt) {
 #pragma unroll
-              for (int nt = 0; nt < 6; ++nt) mma16816<false>(acc[mt][nt], fa.ah[mt], r[4 * nt + 2], r[4 * nt + 3]);
-              if (seven) mma16816<false>(acc[mt][6], fa.ah[mt], b6l[0], b6l[1]);
+              for (int nt = 0; nt < NTM; ++nt)
+                if (active(nt)) mma16816<false>(acc[mt][nt], fa.ah[mt], r[4 * nt + 2], r[4 * nt + 3]);
+              if (G3::NSM > 0 && active(NTM)) mma16816<false>(acc[mt][NTWB - 1], fa.ah[mt], b6l[0], b6l[1]);
             }
           }
 #pragma unroll
           for (int mt = 0; mt < 2; ++mt) {
 #pragma unroll
-            for (int nt = 0; nt < 6; ++nt) mma16816<false>(acc[mt][nt], fa.ah[mt], r[4 * nt], r[4 * nt + 1]);
-            if (seven) mma16816<false>(acc[mt][6], fa.ah[mt], b6h[0], b6h[1]);
+            for (int nt = 0; nt < NTM; ++nt)
+              if (active(nt)) mma16816<false>(acc[mt][nt], fa.ah[mt], r[4 * nt], r[4 * nt + 1]);
+            if (G3::NSM > 0 && active(NTM)) mma16816<false>(acc[mt][NTWB - 1], fa.ah[mt], b6h[0], b6h[1]);
           }
         };
         FragA a0, a1;
@@ -1392,8 +1460,8 @@ lstm_bwd_mma_kernel(float* __restrict__ gates, const float* __restrict__ c_stash
       ph_free ^= 1u;
       PROF_MARK(6)
 #pragma unroll
-      for (int nt = 0; nt < 7; ++nt) {
-        if (nt < 6 || seven) {
+      for (int nt = 0; nt < NTWB; ++nt) {
+        if (active(nt)) {
           const int k = 8 * (nt0 + nt) + 2 * q;          // output hidden unit of acc[..][nt][0]
           const int owner = k / UPC, kl = k - owner * UPC;
           unsigned char* dst = Ssm + (size_t)owner * G::B_RBLK;
@@ -1428,9 +1496,9 @@ lstm_bwd_mma_kernel(float* __restrict__ gates, const float* __restrict__ c_stash
   cluster_wait();
 }
 
-template <class K>
-int launch_cluster5(K kernel, size_t smem, int ntiles, cudaStream_t st, void** args, const char* name, int (*cache_tab)[16],
-                    bool (*attr_tab)[16], int variant, int nthreads = G::NT, bool bwd = false) {
+template <int CL, class K>
+int launch_cluster(K kernel, size_t smem, int ntiles, cudaStream_t st, void** args, const char* name, int (*cache_tab)[16],
+                   bool (*attr_tab)[16], int variant, int nthreads = G<CL>::NT, bool bwd = false) {
   int dev = 0;
   NNR_CUDA(cudaGetDevice(&dev));
   dev &= 15;                                  // the attribute and the occupancy are per device (and per instantiation)
@@ -1446,11 +1514,11 @@ int launch_cluster5(K kernel, size_t smem, int ntiles, cudaStream_t st, void** a
   cudaLaunchConfig_t cfg = {};
   cudaLaunchAttribute attr[1];
   attr[0].id = cudaLaunchAttributeClusterDimension;
-  attr[0].val.clusterDim.x = G::CL; attr[0].val.clusterDim.y = 1; attr[0].val.clusterDim.z = 1;
+  attr[0].val.clusterDim.x = CL; attr[0].val.clusterDim.y = 1; attr[0].val.clusterDim.z = 1;
   cfg.attrs = attr; cfg.numAttrs = 1;
   cfg.blockDim = dim3(nthreads); cfg.dynamicSmemBytes = smem; cfg.stream = st;
   if (*cache == 0) {
-    cfg.gridDim = dim3(G::CL * 2);
+    cfg.gridDim = dim3(CL * 2);
     int nc = 0;
     cudaError_t e = cudaOccupancyMaxActiveClusters(&nc, (const void*)kernel, &cfg);
     if (e != cudaSuccess || nc < 2) { (void)cudaGetLastError(); nc = 24; }
@@ -1459,8 +1527,9 @@ int launch_cluster5(K kernel, size_t smem, int ntiles, cudaStream_t st, void** a
     // twice (it answers 1 CTA / SM = 26 clusters on B200, with or without the shared-memory carve-out hint), the hardware
     // does co-schedule them.  Measured on B200, N = 3520, L = 128 forward: 26 clusters 4.67 ms, 40: 4.09, 52: 3.50, 56: 3.43,
     // 58: 3.32, 64: 3.45, 72: 3.40 -> 2 nc + 6.  Clusters beyond what fits start late, find the tile counter exhausted and exit.
-    if (nthreads == G2::NT) *cache = (2 * nc + 6) & ~1;
-    if (const char* ev = getenv(bwd ? "NNR_LSTM_BWD_CLUSTERS" : "NNR_LSTM_FWD_CLUSTERS")) { int v = atoi(ev); if (v >= 2 && nthreads == G2::NT) *cache = v & ~1; }
+    // The rule was measured at CL = 5 (hidden_dim 200); the smaller clusters of other hidden sizes use it unchanged.
+    if (nthreads == G2<CL>::NT) *cache = (2 * nc + 6) & ~1;
+    if (const char* ev = getenv(bwd ? "NNR_LSTM_BWD_CLUSTERS" : "NNR_LSTM_FWD_CLUSTERS")) { int v = atoi(ev); if (v >= 2 && nthreads == G2<CL>::NT) *cache = v & ~1; }
     if (getenv("NNR_LSTM_DEBUG")) {
       int bps = -1;
       cudaOccupancyMaxActiveBlocksPerMultiprocessor(&bps, (const void*)kernel, nthreads, smem);
@@ -1471,7 +1540,7 @@ int launch_cluster5(K kernel, size_t smem, int ntiles, cudaStream_t st, void** a
   int want = 2 * ntiles;                      // (tile, direction) pairs
   int nclusters = want < *cache ? want : *cache;
   if (nclusters < 2) nclusters = 2;
-  cfg.gridDim = dim3(nclusters * G::CL);
+  cfg.gridDim = dim3(nclusters * CL);
   cudaError_t e = cudaLaunchKernelExC(&cfg, (const void*)kernel, args);
   nnr_count_launch(1);
   if (e != cudaSuccess) { nnr_set_error("%s: launch failed: %s", name, cudaGetErrorString(e)); return (int)e; }
@@ -1519,26 +1588,56 @@ static int lstm_fwd_use_tm() {
   return use_tm;
 }
 int nnr_lstm_fwd_planes_ok(void) { return lstm_fwd_use_tm(); }
+static int lstm_bwd_use_tm() {
+  static int use_tm = -1;          // W slice in tensor memory, two CTAs per SM (default); NNR_LSTM_BWD_TM=0: W planes in shared memory
+  if (use_tm < 0) { const char* e = getenv("NNR_LSTM_BWD_TM"); use_tm = e ? atoi(e) : 1; }
+  return use_tm;
+}
+int nnr_lstm_bwd_tm_ok(void) { return lstm_bwd_use_tm(); }
 
-int nnr_lstm_fwd_mma(float* gx, const float* w_hh, const int32_t* len, const int32_t* off, const int32_t* order, int N,
+// CTAs per cluster for hidden size H (0 < H <= 200): 40 units per CTA, at least two CTAs
+static int lstm_cluster_size(int H) { return H <= 80 ? 2 : (H + 39) / 40; }
+
+// per-instantiation slots of the occupancy / attribute caches: [CL - 2] for a run-time H, [4] for hidden_dim 200
+static int lstm_kernel_slot(int H) { return H == 200 ? 4 : lstm_cluster_size(H) - 2; }
+
+template <int CL, int HC>
+static int lstm_fwd_tm_launch(void** args, int ntiles, cudaStream_t st, int single, int (*cache)[16], bool (*attr_set)[16]) {
+  return single ? launch_cluster<CL>(lstm_fwd_tm_kernel<true, CL, HC>, G2<CL>::FWD_SMEM, ntiles, st, args, "lstm_fwd_tm_kernel<single>", cache, attr_set, 3,
+                                     G2<CL>::NT)
+                : launch_cluster<CL>(lstm_fwd_tm_kernel<false, CL, HC>, G2<CL>::FWD_SMEM, ntiles, st, args, "lstm_fwd_tm_kernel", cache, attr_set, 2,
+                                     G2<CL>::NT);
+}
+
+// 0 < H <= 200 and H % 4 == 0 with the tensor-memory variant; the shared-memory variant and h_planes need H = 200 (lstm.cu checks)
+int nnr_lstm_fwd_mma(float* gx, const float* w_hh, const int32_t* len, const int32_t* off, const int32_t* order, int N, int H,
                      float* h_out, float* c_stash, float* c_n, int32_t* tile_counters, cudaStream_t st, void* h_planes,
                      size_t plane_stride, int two_planes, int cap) {
-  static int cache[4][16] = {};
-  static bool attr_set[4][16] = {};
-  int ntiles = (N + G::MT - 1) / G::MT;
+  static int cache[5][4][16] = {};     // [lstm_kernel_slot][variant][device]
+  static bool attr_set[5][4][16] = {};
+  const int CL = lstm_cluster_size(H), slot = lstm_kernel_slot(H);
+  int ntiles = (N + G<5>::MT - 1) / G<5>::MT;
   NNR_CUDA(cudaMemsetAsync(tile_counters, 0, 2 * sizeof(int32_t), st));
   const int single = nnr_lstm_single_product();
   const int use_tm = lstm_fwd_use_tm();
   if (use_tm) {
     __nv_bfloat16* hp = (__nv_bfloat16*)h_planes;
-    void* args[] = {&gx, &w_hh, &len, &off, &order, &N, &ntiles, &h_out, &c_stash, &c_n, &tile_counters, &hp, &plane_stride, &two_planes};
-    int rc2 = single ? launch_cluster5(lstm_fwd_tm_kernel<true>, G2::FWD_SMEM, ntiles, st, args, "lstm_fwd_tm_kernel<single>", cache, attr_set, 3, G2::NT)
-                     : launch_cluster5(lstm_fwd_tm_kernel<false>, G2::FWD_SMEM, ntiles, st, args, "lstm_fwd_tm_kernel", cache, attr_set, 2, G2::NT);
+    void* args[] = {&gx, &w_hh, &len, &off, &order, &N, &H, &ntiles, &h_out, &c_stash, &c_n, &tile_counters, &hp, &plane_stride, &two_planes};
+    int rc2;
+    switch (CL) {
+      case 2: rc2 = lstm_fwd_tm_launch<2, 0>(args, ntiles, st, single, cache[slot], attr_set[slot]); break;
+      case 3: rc2 = lstm_fwd_tm_launch<3, 0>(args, ntiles, st, single, cache[slot], attr_set[slot]); break;
+      case 4: rc2 = lstm_fwd_tm_launch<4, 0>(args, ntiles, st, single, cache[slot], attr_set[slot]); break;
+      default:
+        rc2 = H == 200 ? lstm_fwd_tm_launch<5, 200>(args, ntiles, st, single, cache[slot], attr_set[slot])
+                       : lstm_fwd_tm_launch<5, 0>(args, ntiles, st, single, cache[slot], attr_set[slot]);
+        break;
+    }
     int dev2 = 0;
     cudaGetDevice(&dev2);
-    nnr_lstm_mma_max_clusters = cache[2 + single][dev2 & 15];
+    nnr_lstm_mma_max_clusters = cache[slot][2 + single][dev2 & 15];
     if (rc2 || !hp) return rc2;
-    planes_zero_tail_kernel<<<32, 256, 0, st>>>(hp, plane_stride, two_planes ? 2 : 1, 2 * G::HID, cap, off + N);
+    planes_zero_tail_kernel<<<32, 256, 0, st>>>(hp, plane_stride, two_planes ? 2 : 1, 2 * H, cap, off + N);
     nnr_count_launch(1);
     cudaError_t e = cudaGetLastError();
     if (e != cudaSuccess) { nnr_set_error("planes_zero_tail_kernel: launch failed: %s", cudaGetErrorString(e)); return (int)e; }
@@ -1546,11 +1645,11 @@ int nnr_lstm_fwd_mma(float* gx, const float* w_hh, const int32_t* len, const int
   }
   if (h_planes) { nnr_set_error("nnr_lstm_fwd_planes: needs the tensor-memory forward kernel (NNR_LSTM_FWD_TM=1)"); return NNR_ERR_UNSUPPORTED; }
   void* args[] = {&gx, &w_hh, &len, &off, &order, &N, &ntiles, &h_out, &c_stash, &c_n, &tile_counters};
-  int rc = single ? launch_cluster5(lstm_fwd_mma_kernel<true>, G::FWD_SMEM, ntiles, st, args, "lstm_fwd_mma_kernel<single>", cache, attr_set, 1)
-                  : launch_cluster5(lstm_fwd_mma_kernel<false>, G::FWD_SMEM, ntiles, st, args, "lstm_fwd_mma_kernel", cache, attr_set, 0);
+  int rc = single ? launch_cluster<5>(lstm_fwd_mma_kernel<true>, G<5>::FWD_SMEM, ntiles, st, args, "lstm_fwd_mma_kernel<single>", cache[4], attr_set[4], 1)
+                  : launch_cluster<5>(lstm_fwd_mma_kernel<false>, G<5>::FWD_SMEM, ntiles, st, args, "lstm_fwd_mma_kernel", cache[4], attr_set[4], 0);
   int dev = 0;
   cudaGetDevice(&dev);
-  nnr_lstm_mma_max_clusters = cache[single][dev & 15];
+  nnr_lstm_mma_max_clusters = cache[4][single][dev & 15];
   return rc;
 }
 
@@ -1577,29 +1676,44 @@ __global__ void lstm_dz_finish_kernel(const float* __restrict__ db_partial, int 
   }
 }
 
+template <int CL, int HC>
+static int lstm_bwd_tm_launch(void** args, int ntiles, cudaStream_t st, int single, int (*cache)[16], bool (*attr_set)[16]) {
+  return single ? launch_cluster<CL>(lstm_bwd_mma_kernel<true, true, CL, HC>, G3<CL>::BWD_SMEM, ntiles, st, args, "lstm_bwd_tm_kernel<single>", cache, attr_set, 3,
+                                     G3<CL>::NT, true)
+                : launch_cluster<CL>(lstm_bwd_mma_kernel<false, true, CL, HC>, G3<CL>::BWD_SMEM, ntiles, st, args, "lstm_bwd_tm_kernel", cache, attr_set, 2,
+                                     G3<CL>::NT, true);
+}
+
+// 0 < H <= 200 and H % 4 == 0 with the tensor-memory variant; the shared-memory variant and dz_planes need H = 200 (lstm.cu checks)
 int nnr_lstm_bwd_mma(float* gates, const float* c_stash, const float* w_hh, const int32_t* len, const int32_t* off,
-                     const int32_t* order, int N, const float* dh, const float* dcn, int32_t* tile_counters, cudaStream_t st,
+                     const int32_t* order, int N, int H, const float* dh, const float* dcn, int32_t* tile_counters, cudaStream_t st,
                      void* dz_planes, size_t plane_stride, int two_planes, float* db_partial, float* db, int cap) {
-  static int cache[4][16] = {};
-  static bool attr_set[4][16] = {};
-  int ntiles = (N + G::MT - 1) / G::MT;
+  static int cache[5][4][16] = {};     // [lstm_kernel_slot][variant][device]
+  static bool attr_set[5][4][16] = {};
+  const int CL = lstm_cluster_size(H), slot = lstm_kernel_slot(H);
+  int ntiles = (N + G<5>::MT - 1) / G<5>::MT;
   NNR_CUDA(cudaMemsetAsync(tile_counters, 0, 2 * sizeof(int32_t), st));
   __nv_bfloat16* dzp = (__nv_bfloat16*)dz_planes;
-  void* args[] = {&gates, &c_stash, &w_hh, &len, &off, &order, &N, &ntiles, &dh, &dcn, &tile_counters,
+  void* args[] = {&gates, &c_stash, &w_hh, &len, &off, &order, &N, &H, &ntiles, &dh, &dcn, &tile_counters,
                   &dzp, &plane_stride, &two_planes, &db_partial};
-  static int use_tm = -1;          // W slice in tensor memory, two CTAs per SM (default); NNR_LSTM_BWD_TM=0: W planes in shared memory
-  if (use_tm < 0) { const char* e = getenv("NNR_LSTM_BWD_TM"); use_tm = e ? atoi(e) : 1; }
+  const int single = nnr_lstm_single_product();
   int rc;
-  if (use_tm)
-    rc = nnr_lstm_single_product()
-             ? launch_cluster5(lstm_bwd_mma_kernel<true, true>, G3::BWD_SMEM, ntiles, st, args, "lstm_bwd_tm_kernel<single>", cache, attr_set, 3, G3::NT, true)
-             : launch_cluster5(lstm_bwd_mma_kernel<false, true>, G3::BWD_SMEM, ntiles, st, args, "lstm_bwd_tm_kernel", cache, attr_set, 2, G3::NT, true);
-  else
-    rc = nnr_lstm_single_product()
-             ? launch_cluster5(lstm_bwd_mma_kernel<true, false>, G::BWD_SMEM, ntiles, st, args, "lstm_bwd_mma_kernel<single>", cache, attr_set, 1)
-             : launch_cluster5(lstm_bwd_mma_kernel<false, false>, G::BWD_SMEM, ntiles, st, args, "lstm_bwd_mma_kernel", cache, attr_set, 0);
+  if (lstm_bwd_use_tm()) {
+    switch (CL) {
+      case 2: rc = lstm_bwd_tm_launch<2, 0>(args, ntiles, st, single, cache[slot], attr_set[slot]); break;
+      case 3: rc = lstm_bwd_tm_launch<3, 0>(args, ntiles, st, single, cache[slot], attr_set[slot]); break;
+      case 4: rc = lstm_bwd_tm_launch<4, 0>(args, ntiles, st, single, cache[slot], attr_set[slot]); break;
+      default:
+        rc = H == 200 ? lstm_bwd_tm_launch<5, 200>(args, ntiles, st, single, cache[slot], attr_set[slot])
+                      : lstm_bwd_tm_launch<5, 0>(args, ntiles, st, single, cache[slot], attr_set[slot]);
+        break;
+    }
+  } else {
+    rc = single ? launch_cluster<5>(lstm_bwd_mma_kernel<true, false, 5, 200>, G<5>::BWD_SMEM, ntiles, st, args, "lstm_bwd_mma_kernel<single>", cache[4], attr_set[4], 1)
+                : launch_cluster<5>(lstm_bwd_mma_kernel<false, false, 5, 200>, G<5>::BWD_SMEM, ntiles, st, args, "lstm_bwd_mma_kernel", cache[4], attr_set[4], 0);
+  }
   if (rc || !dz_planes) return rc;
-  const int cols = 8 * G::HID;
+  const int cols = 8 * H;
   lstm_dz_finish_kernel<<<(cols + 255) / 256 * 4, 256, 0, st>>>(db_partial, ntiles, cols, db, dzp, plane_stride, two_planes ? 2 : 1, cap, off + N);
   nnr_count_launch(1);
   cudaError_t e = cudaGetLastError();

@@ -661,7 +661,8 @@ class CNEFunction(torch.autograd.Function):
 
         def weight_grads(x, m, dz, dz_pl, db, hp=None):
             pre = x + '_lstm.'
-            hprev, hprev_pl = hp if hp is not None else shifted_h(m, dz_pl is not None)
+            # as 16-bit planes the reverse half of h_{t-1} starts at column Hd, 16 B aligned only when Hd % 8 == 0: otherwise fp32
+            hprev, hprev_pl = hp if hp is not None else shifted_h(m, dz_pl is not None and Hd % 8 == 0)
             for d, sfx in enumerate(('', '_reverse')):
                 G[pre + 'weight_hh_l0' + sfx] = wgrad(dz[:, d * 4 * Hd:(d + 1) * 4 * Hd] if dz is not None else None,
                                                      hprev[:, d * Hd:(d + 1) * Hd] if hprev is not None else None,
