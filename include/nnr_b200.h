@@ -33,7 +33,7 @@
 extern "C" {
 #endif
 
-#define NNR_ABI_VERSION 5
+#define NNR_ABI_VERSION 6
 #define NNR_SEED_INDIRECT (1ULL << 62)
 
 const char* nnr_last_error(void);
@@ -329,6 +329,25 @@ int nnr_rowdot_fwd(const float* a, const float* b, int R, int D, float* out, voi
 /* da = dout[r]*b (+= if accumulate_a), db likewise */
 int nnr_rowdot_bwd(const float* dout, const float* a, const float* b, int R, int D, float* da,
                    int accumulate_a, float* db, int accumulate_b, void* stream);
+
+/* ---- streaming top-k over a candidate pool (news recommendation; scoring.CorpusScorer.recommend) ----------------
+ * Merges one score tile scores[B, T] (row stride lds) into a running per-row best list best_score[B, k] (fp32) /
+ * best_pos[B, k] (int64 pool positions), in place.  Tile entry j of row b has pool position pos0 + j.
+ * Order: score descending; equal scores by ascending position (= a stable descending sort of the whole row); a NaN
+ * ranks below every number, -inf included.  Entries whose news id tile_ids[j] is among exclude[b, 0:exclude_len[b]]
+ * (exclude [B, ldx] int64, lengths clamped to [0, ldx]) are skipped; exclude = NULL skips nothing (tile_ids may then be
+ * NULL).  The list is left sorted best first; slots no candidate has reached hold the fill entry (-inf, -1), which
+ * every real entry, -inf or NaN, ranks before.  init != 0 ignores the list's previous content (the first tile of a
+ * pool); otherwise the list must be as a previous call left it.
+ * Entries that do not beat the current k-th best are dropped before anything is sorted.  Deterministic, no host
+ * synchronisation, no allocation (graph-capturable).  Limits: 1 <= k <= NNR_TOPK_MAX_K, 1 <= T <= NNR_TOPK_MAX_TILE,
+ * ldx <= NNR_TOPK_MAX_EXCLUDE, 0 <= pos0 and pos0 + T < 2^31 - 1; NNR_ERR_ARG before any CUDA call otherwise.       */
+#define NNR_TOPK_MAX_K 1024
+#define NNR_TOPK_MAX_TILE 4096
+#define NNR_TOPK_MAX_EXCLUDE 1024
+int nnr_topk_merge(const float* scores, int64_t lds, int B, int T, int64_t pos0, const int64_t* tile_ids,
+                   const int64_t* exclude, const int32_t* exclude_len, int ldx, int k, int init,
+                   float* best_score, int64_t* best_pos, void* stream);
 
 /* elementwise dropout with the library's counter RNG (proxy nodes / cluster features /
  * GCN inter-layer dropout): y = x * keep(seed, i)/(1-p); the same call applies the backward.   */

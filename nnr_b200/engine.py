@@ -750,6 +750,13 @@ def sue_wo_hca_param_names(L, layer_norm=False):
             + ['attention.affine1.weight', 'attention.affine1.bias', 'attention.affine2.weight'])
 
 
+def sue_names(meta):
+    """parameter order of SUEFunction for the user encoder described by ``meta`` (SUE, SUE_wo_HCA, SUE_wo_GCN)"""
+    gcn, ln = meta.get('gcn', True), meta.get('layer_norm', False)
+    L = meta['gcn_layers'] if gcn else 0
+    return (sue_param_names(L, ln) if meta['hca'] else sue_wo_hca_param_names(L, ln)) if gcn else sue_wo_gcn_param_names()
+
+
 class SUEFunction(torch.autograd.Function):
     """user[B,n,D] = SUE(history_embedding[B,H,D], candidate[B,n,D], graph, cluster mask / indices)."""
 
@@ -758,8 +765,7 @@ class SUEFunction(torch.autograd.Function):
         hca = meta['hca']
         gcn = meta.get('gcn', True)
         L = meta['gcn_layers'] if gcn else 0
-        ln = meta.get('layer_norm', False)
-        names = (sue_param_names(L, ln) if hca else sue_wo_hca_param_names(L, ln)) if gcn else sue_wo_gcn_param_names()
+        names = sue_names(meta)
         P = dict(zip(names, params))
         B, H, D = hist.shape
         n = cand.shape[1]
@@ -768,7 +774,6 @@ class SUEFunction(torch.autograd.Function):
         dev = hist.device
         training, p = meta['training'], meta['p_drop']
         pe = p if training else 0.0
-        residual = meta['residual']
         seeds = [fresh_seed() for _ in range(L + 2)] if pe > 0 else [0] * (L + 2)
         hist = hist.contiguous()
         cand = cand.contiguous()
@@ -781,6 +786,26 @@ class SUEFunction(torch.autograd.Function):
         if hca:
             lanes.fork()
             pre = lanes.on_side(SUEFunction._cand_side, P, cand, B, n, D)
+        gfeat, graph, xs, rs, aggs, lns = SUEFunction._gcn(meta, P, hist, graph, seeds, L, pe)
+        ctx.meta, ctx.P, ctx.names = meta, P, names
+        ctx.dims = (B, H, D, n, C, Gn, C1)
+        ctx.seeds, ctx.graph = seeds, graph
+        ctx.xs, ctx.rs, ctx.aggs, ctx.lns = xs, rs, aggs, lns
+        ctx.gfeat, ctx.cand = gfeat, cand
+        if not hca:                                                                           # SUE_wo_HCA
+            pooled, ctx.u, ctx.alpha = SUEFunction._history_pool(P, gfeat)
+            return pooled.unsqueeze(1).repeat(1, n, 1)
+        lanes.join()
+        return SUEFunction._clusters_tail(ctx, P, gfeat, cand, cmask, cidx, seeds, (B, H, D, n, C, Gn, C1), L, pe, pre)
+
+    @staticmethod
+    def _gcn(meta, P, hist, graph, seeds, L, pe):
+        """X0 = [history | proxy nodes] through the GCN layers; returns gfeat [B, H, D] = (X_L + X0)[:, :H], the contiguous
+        graph and the stash of the backward pass (xs, rs, aggs, lns)"""
+        B, H, D = hist.shape
+        Gn = H + P['proxy_node_embedding'].shape[0]
+        dev = hist.device
+        residual, ln = meta['residual'], meta.get('layer_norm', False)
         # X0 = [history | dropout_(proxy nodes)]   (userEncoders.py:80)
         x0 = _empty((B, Gn, D), dev)
         x0[:, :H] = hist
@@ -820,22 +845,20 @@ class SUEFunction(torch.autograd.Function):
             x = xn.view(B, Gn, D)
             xs.append(x)
         gfeat = (x + x0)[:, :H, :].contiguous()                                              # userEncoders.py:81-82
-        ctx.meta, ctx.P, ctx.names = meta, P, names
-        ctx.dims = (B, H, D, n, C, Gn, C1)
-        ctx.seeds, ctx.graph = seeds, graph
-        ctx.xs, ctx.rs, ctx.aggs, ctx.lns = xs, rs, aggs, lns
-        ctx.gfeat, ctx.cand = gfeat, cand
-        if not hca:                                                                           # SUE_wo_HCA
-            A = P['attention.affine1.weight'].shape[0]
-            u = linear(gfeat.view(B * H, D), P['attention.affine1.weight'], B * H, None, P['attention.affine1.bias'], EPI_BIAS_TANH)
-            pooled = _empty((B, D), dev)
-            alpha = _empty((B * H,), dev)
-            ops.attn_pool_fwd(X=gfeat, ldx=D, D=D, S=B, max_len=H, mode=0, fixed_len=H, U=u, ldu=A, A=A,
-                              w2=P['attention.affine2.weight'], pooled=pooled, ldp=D, alpha=alpha)
-            ctx.u, ctx.alpha = u, alpha
-            return pooled.unsqueeze(1).repeat(1, n, 1)
-        lanes.join()
-        return SUEFunction._clusters_tail(ctx, P, gfeat, cand, cmask, cidx, seeds, (B, H, D, n, C, Gn, C1), L, pe, pre)
+        return gfeat, graph, xs, rs, aggs, lns
+
+    @staticmethod
+    def _history_pool(P, gfeat):
+        """SUE_wo_HCA: additive attention over the history rows (variantEncoders.py:416-419); returns (pooled [B, D], the
+        attention projection u, the weights alpha)"""
+        B, H, D = gfeat.shape
+        A = P['attention.affine1.weight'].shape[0]
+        u = linear(gfeat.view(B * H, D), P['attention.affine1.weight'], B * H, None, P['attention.affine1.bias'], EPI_BIAS_TANH)
+        pooled = _empty((B, D), gfeat.device)
+        alpha = _empty((B * H,), gfeat.device)
+        ops.attn_pool_fwd(X=gfeat, ldx=D, D=D, S=B, max_len=H, mode=0, fixed_len=H, U=u, ldu=A, A=A,
+                          w2=P['attention.affine2.weight'], pooled=pooled, ldp=D, alpha=alpha)
+        return pooled, u, alpha
 
     @staticmethod
     def _cand_side(P, cand, B, n, D):
@@ -860,8 +883,18 @@ class SUEFunction(torch.autograd.Function):
         return SUEFunction._clusters_tail(ctx, P, hist, cand, cmask, cidx, seeds, dims, L, pe)
 
     @staticmethod
-    def _clusters_tail(ctx, P, gfeat, cand, cmask, cidx, seeds, dims, L, pe, pre=None):
-        """intra-cluster attention, cluster affine, inter-cluster attention (userEncoders.py:83-97)"""
+    def _user_keys(P, gfeat):
+        """what the cluster attentions need from the history alone: gfeat's operand planes and the keys of the intra-cluster
+        attention (userEncoders.py:85)"""
+        B, H, D = gfeat.shape
+        gfeat_pl = _shared_split(gfeat.view(B * H, D), B * H, D)   # gfeat, cand, q2: split once for the forward GEMMs and the
+        Kp = linear(gfeat.view(B * H, D), P['intraCluster_K.weight'], B * H, x_planes=gfeat_pl)   # weight-gradient GEMMs of the backward
+        return gfeat_pl, Kp
+
+    @staticmethod
+    def _clusters_tail(ctx, P, gfeat, cand, cmask, cidx, seeds, dims, L, pe, pre=None, keys=None):
+        """intra-cluster attention, cluster affine, inter-cluster attention (userEncoders.py:83-97); ``keys``: the result of
+        _user_keys when the history side is already computed"""
         B, H, D, n, C, Gn, C1 = dims
         dev = gfeat.device
         Au = P['intraCluster_K.weight'].shape[0]
@@ -869,8 +902,7 @@ class SUEFunction(torch.autograd.Function):
         # (an intraCluster_K.bias -- SUE_wo_GCN only -- shifts every score of a (user, candidate) pair equally and
         #  cancels in the per-cluster softmax: it is not applied, and its gradient is exactly zero)
         cand_pl, Qp, q2, q2_pl, qk2 = pre if pre is not None else SUEFunction._cand_side(P, cand, B, n, D)
-        gfeat_pl = _shared_split(gfeat.view(B * H, D), B * H, D)   # gfeat, cand, q2: split once for the forward GEMMs and the
-        Kp = linear(gfeat.view(B * H, D), P['intraCluster_K.weight'], B * H, x_planes=gfeat_pl)   # weight-gradient GEMMs of the backward
+        gfeat_pl, Kp = keys if keys is not None else SUEFunction._user_keys(P, gfeat)
         alpha = _empty((B * n, H), dev)
         intra = _empty((B * n * C1, D), dev)
         cidx = cidx.contiguous()
@@ -1062,3 +1094,45 @@ class RowDot(torch.autograd.Function):
         du, dn = torch.empty_like(user), torch.empty_like(news)
         ops.rowdot_bwd(dout.contiguous(), user, news, B * n, D, du, False, dn, False)
         return du, dn
+
+
+# ------------------------------------------------------------------------------------------------
+# SUE inference in two halves: the user side once per batch of users, the candidate tail per tile of candidates
+# ------------------------------------------------------------------------------------------------
+# Scoring a pool of candidates against the same users (news recommendation) repeats only the candidate tail of
+# SUEFunction.forward: the GCN and the intra-cluster keys depend on the history alone.  Both halves call the forward's own
+# pieces on the same shapes, so a tile's scores equal SUEFunction.forward + RowDot on [B, T] candidates bit for bit.
+# Inference only: eval mode (no dropout), no autograd.
+@torch.no_grad()
+def sue_user_side(meta, hist, graph, cmask, cidx, *params):
+    """the history half of SUEFunction.forward for the users of hist [B, H, D]: returns the tuple of tensors
+    ``sue_tile_scores`` takes -- (gfeat, Kp, cmask, cidx) with the hierarchical cluster attention, (pooled user vector,)
+    for SUE_wo_HCA"""
+    assert not meta['training'], 'the split SUE forward is for inference (eval mode)'
+    P = dict(zip(sue_names(meta), params))
+    gcn = meta.get('gcn', True)
+    L = meta['gcn_layers'] if gcn else 0
+    hist = hist.contiguous()
+    gfeat = SUEFunction._gcn(meta, P, hist, graph, [0] * (L + 2), L, 0.0)[0] if gcn else hist
+    if not meta['hca']:
+        return (SUEFunction._history_pool(P, gfeat)[0],)
+    return gfeat, SUEFunction._user_keys(P, gfeat)[1], cmask, cidx.contiguous()
+
+
+@torch.no_grad()
+def sue_tile_scores(meta, side, cand, *params):
+    """click scores [B, T] of the candidates cand [B, T, D] for the users of ``side`` (from ``sue_user_side``): the
+    candidate tail of SUEFunction.forward and the dot product (model.py:127)"""
+    P = dict(zip(sue_names(meta), params))
+    B, T, D = cand.shape
+    cand = cand.contiguous()
+    if not meta['hca']:
+        return RowDot.apply(side[0].unsqueeze(1).repeat(1, T, 1), cand)
+    gfeat, Kp, cmask, cidx = side
+    gcn = meta.get('gcn', True)
+    L = meta['gcn_layers'] if gcn else 0
+    C = P['proxy_node_embedding'].shape[0] if gcn else meta['category_num']
+    H = gfeat.shape[1]
+    user = SUEFunction._clusters_tail(_Mod(), P, gfeat, cand, cmask, cidx, [0] * (L + 2), (B, H, D, T, C, H + C, C + 1), L, 0.0,
+                                      keys=(None, Kp))
+    return RowDot.apply(user, cand)

@@ -443,6 +443,19 @@ def rowdot_bwd(dout, a, b, R, D, da, accumulate_a, db, accumulate_b):
                              _p(db, _F32), int(accumulate_b), _stream()), 'nnr_rowdot_bwd')
 
 
+TOPK_MAX_K, TOPK_MAX_TILE, TOPK_MAX_EXCLUDE = 1024, 4096, 1024      # include/nnr_b200.h: NNR_TOPK_MAX_*
+
+
+def topk_merge(scores, pos0, tile_ids, exclude, exclude_len, init, best_score, best_pos):
+    """merge the score tile scores [B, T] (pool positions pos0 + j) into the running best list best_score / best_pos
+    [B, k], skipping entries whose id tile_ids[j] is among the row's exclude[b, :exclude_len[b]] (nnr_topk_merge)"""
+    B, T = scores.shape
+    ldx = exclude.shape[1] if exclude is not None else 0
+    check(lib.nnr_topk_merge(_p(scores, _F32), scores.stride(0), B, T, int(pos0), _p(tile_ids, _I64), _p(exclude, _I64),
+                             _p(exclude_len, _I32), ldx, best_score.shape[1], int(init), _p(best_score, _F32),
+                             _p(best_pos, _I64), _stream()), 'nnr_topk_merge')
+
+
 def dropout(x, p_drop, seed, y):
     check(lib.nnr_dropout(_p(x, _F32), x.numel(), float(p_drop), int(seed), _p(y, _F32), _stream()), 'nnr_dropout')
 
@@ -510,6 +523,8 @@ _SCHEMAS = {
     'ln_relu_res_bwd': ('(Tensor dout, Tensor y, Tensor gamma, Tensor relu_out, Tensor mean, Tensor rstd, int R, int D, float p_drop, int seed, '
                         'Tensor(a!)? dout_dropped, Tensor(b!) dy, Tensor(c!) dgamma, Tensor(d!) dbeta) -> ()', ln_relu_res_bwd),
     'dropout': ('(Tensor x, float p_drop, int seed, Tensor(a!) y) -> ()', dropout),
+    'topk_merge': ('(Tensor scores, int pos0, Tensor? tile_ids, Tensor? exclude, Tensor? exclude_len, bool init, '
+                   'Tensor(a!) best_score, Tensor(b!) best_pos) -> ()', topk_merge),
     'flat_clip_adam': ('(Tensor(a!) param, Tensor grad, Tensor(b!) exp_avg, Tensor(c!) exp_avg_sq, float lr, float beta1, '
                        'float beta2, float eps, float max_norm, float grad_scale, int step, Tensor(d!) norm_out) -> ()',
                        flat_clip_adam),

@@ -38,11 +38,19 @@ def _checksum(t):
 class CorpusScorer:
     """``process_group=None`` scores on this process's device alone.  With an NCCL group, ``encode_corpus`` and
     ``evaluate`` are collectives: every rank of the group calls them with the same arguments (and the same weights, as
-    ``TrainStep`` keeps them) and gets the whole result.  ``score`` is always rank-local."""
+    ``TrainStep`` keeps them) and gets the whole result.  ``score`` and ``recommend`` are always rank-local.
+    ``graph_flags`` = ``ops.graph_flags(...)`` of the options the model was trained with (no_self_connection,
+    no_adjacent_normalization, gcn_normalization_type); 0 is the reference's default symmetric graph."""
+
+    # recommend(): candidates per pool tile by default = this many rows of the cluster tail, B * T * (C + 1).  Each row holds
+    # four D-wide fp32-sized buffers (intra-cluster features, their GEMM operand planes, the relu stash, the cluster
+    # features): about 7.5 GB at D = 900, plus ~11 KB per (user, candidate) pair on the candidate side.
+    TAIL_ROWS = 1 << 19
 
     def __init__(self, model, news_title_text, news_title_mask, news_content_text, news_content_mask, news_category,
-                 news_subCategory, chunk=4096, process_group=None):
+                 news_subCategory, chunk=4096, process_group=None, graph_flags=0):
         self.model = model
+        self.graph_flags = graph_flags                          # ops.graph_flags(...) of the model's training configuration
         self.dev = next(model.parameters()).device
         to = lambda t: torch.as_tensor(t).to(self.dev)
         self.tt, self.tm, self.ct, self.cm = to(news_title_text), to(news_title_mask).clone(), to(news_content_text), to(news_content_mask).clone()
@@ -172,19 +180,102 @@ class CorpusScorer:
             return self._graphed(key, self._score_impl, (hid, hl, cid)).clone()
         return self._score_impl(hid, hl, cid)
 
-    def _score_impl(self, hid, hl, cid):
+    def _category_num(self):
         ue = self.model.user_encoder
+        return ue.proxy_node_embedding.shape[0] if hasattr(ue, 'proxy_node_embedding') else ue.category_num - 1   # SUE_wo_GCN
+
+    def _history_graph(self, hid, hl):
+        """graph, cluster mask and cluster indices of the histories hid [B, H], built on the device from the cached
+        category ids"""
         B, H = hid.shape
-        C = ue.proxy_node_embedding.shape[0]
+        C = self._category_num()
         cats = self.cat[hid].contiguous()
         graph = torch.empty(B, H + C, H + C, device=self.dev)
         cmask = torch.empty(B, C + 1, dtype=torch.bool, device=self.dev)
         cidx = torch.empty(B, H, dtype=torch.int64, device=self.dev)
-        ops.sue_graph_build(cats, hl, C, graph, cmask, cidx)
+        ops.sue_graph_build(cats, hl, C, graph, cmask, cidx, flags=self.graph_flags)
+        return graph, cmask, cidx
+
+    def _score_impl(self, hid, hl, cid):
+        graph, cmask, cidx = self._history_graph(hid, hl)
         hist = self.cache[hid]                                  # [B, H, D]
         cand = self.cache[cid]                                  # [B, n, D]
-        user = ue.encode_user(hist, graph, cmask, cidx, cand)
+        user = self.model.user_encoder.encode_user(hist, graph, cmask, cidx, cand)
         return engine.RowDot.apply(user, cand)
+
+    def default_pool_tile(self, B):
+        """recommend()'s candidates per tile for B users: B * T * (C + 1) <= TAIL_ROWS, 1 <= T <= ops.TOPK_MAX_TILE"""
+        return max(1, min(ops.TOPK_MAX_TILE, self.TAIL_ROWS // (max(B, 1) * (self._category_num() + 1))))
+
+    @torch.no_grad()
+    def recommend(self, history_ids, history_len, pool_ids, k, exclude_history=True, pool_tile=None, cuda_graph=True):
+        """The k best news of a candidate pool for each user: history_ids [B, H] (0-padded at the end) and history_len [B]
+        as in ``score``, pool_ids [P] corpus row ids shared by the B users.  Returns (ids [B, k] int64, scores [B, k] fp32),
+        best first.
+
+        Order: score descending; equal scores in ascending pool position (a stable descending sort of the user's whole
+        [P] score row, the convention of ``metrics.rank_impressions``); a NaN score ranks below every number.  With
+        ``exclude_history`` a pool entry whose id is among the user's first history_len[b] history ids is never returned.
+        When fewer than k entries are eligible, the tail is filled with id -1 and score -inf (a real candidate scoring
+        -inf still ranks before the fill).  Duplicate pool ids are separate entries.
+
+        The scores are those of ``score(history_ids, history_len, tile.expand(B, T))`` for each tile of the pool, bit for
+        bit: the user side (graph, GCN, intra-cluster keys) is computed once, then the pool is scored in tiles of
+        ``pool_tile`` candidates, each folded into a running top-k list by nnr_topk_merge.  Memory does not grow with P.
+        The default tile holds B * T * (C + 1) <= TAIL_ROWS = 2^19 rows of the cluster tail (about 7.5 GB at D = 900,
+        C = 18; T = 107 for B = 256) and at most 4096 candidates.  Full tiles replay one captured CUDA graph per
+        (B, H, T); a last partial tile runs eagerly.  Rank-local: never a collective, also with a process group.
+        Limits: 1 <= k <= ops.TOPK_MAX_K (1024), 1 <= pool_tile <= ops.TOPK_MAX_TILE (4096), H <= ops.TOPK_MAX_EXCLUDE
+        with ``exclude_history``."""
+        if self.cache is None:
+            raise RuntimeError('CorpusScorer.recommend: call encode_corpus() first')
+        k = int(k)
+        if not 1 <= k <= ops.TOPK_MAX_K:
+            raise ValueError('CorpusScorer.recommend: k must be in [1, %d], got %d' % (ops.TOPK_MAX_K, k))
+        pool = torch.as_tensor(pool_ids)
+        if pool.dim() != 1 or pool.dtype.is_floating_point or pool.dtype == torch.bool:
+            raise ValueError('CorpusScorer.recommend: pool_ids must be a 1-D integer tensor, got %s of shape %s'
+                             % (pool.dtype, tuple(pool.shape)))
+        news_num = self.cache.shape[0]
+        if pool.numel() and (int(pool.min()) < 0 or int(pool.max()) >= news_num):
+            raise ValueError('CorpusScorer.recommend: pool_ids must be in [0, %d), got [%d, %d]'
+                             % (news_num, int(pool.min()), int(pool.max())))
+        hid = torch.as_tensor(history_ids).to(self.dev).long().contiguous()
+        hl = torch.as_tensor(history_len).to(self.dev).to(torch.int32)
+        B, H = hid.shape
+        T = int(self.default_pool_tile(B) if pool_tile is None else pool_tile)
+        if not 1 <= T <= ops.TOPK_MAX_TILE:
+            raise ValueError('CorpusScorer.recommend: pool_tile must be in [1, %d], got %d' % (ops.TOPK_MAX_TILE, T))
+        if exclude_history and H > ops.TOPK_MAX_EXCLUDE:
+            raise ValueError('CorpusScorer.recommend: exclude_history takes at most %d history ids, got %d' % (ops.TOPK_MAX_EXCLUDE, H))
+        pool = pool.to(self.dev).long()
+        P = pool.numel()
+        if P == 0 or B == 0:
+            return (torch.full((B, k), -1, dtype=torch.int64, device=self.dev),
+                    torch.full((B, k), float('-inf'), device=self.dev))
+        ue = self.model.user_encoder
+        side = ue.user_side(self.cache[hid], *self._history_graph(hid, hl))
+
+        def tile_scores(*args):
+            *user, ids = args
+            return ue.tile_scores(tuple(user), self.cache[ids].unsqueeze(0).expand(B, -1, -1))
+
+        best_score = torch.empty(B, k, device=self.dev)
+        best_pos = torch.empty(B, k, dtype=torch.int64, device=self.dev)
+        key = ('recommend', B, H, T, self.cache.data_ptr())
+        for a in range(0, P, T):
+            ids = pool[a:a + T]
+            if cuda_graph and ids.numel() == T:
+                scores = self._graphed(key, tile_scores, (*side, ids))
+                # from now on hand the graph its own static copy of the user side: copy_ onto itself is a no-op, so only
+                # the tile's ids are copied per replay
+                side = self._graphs[key][0][:-1]
+            else:
+                scores = tile_scores(*side, ids)
+            ops.topk_merge(scores, a, ids, hid if exclude_history else None, hl if exclude_history else None, a == 0,
+                           best_score, best_pos)
+        ids = torch.where(best_pos >= 0, pool[best_pos.clamp(min=0)], torch.full_like(best_pos, -1))
+        return ids, best_score
 
     @torch.no_grad()
     def _impression_scores(self, history_ids, history_len, candidate_ids, batch, candidate_count=None, labels=None):

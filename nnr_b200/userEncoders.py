@@ -81,8 +81,22 @@ class SUE(UserEncoder):
         """userEncoders.py:73-97 given the already encoded history (Model.forward encodes candidates and history
         with one CNE schedule, see CNE.encode_calls)."""
         user_history_category_mask[:, -1] = 1                                    # userEncoders.py:73 (in place, like the reference)
-        meta = dict(hca=self.hca, gcn=self.use_gcn, gcn_layers=self.gcn_layer_num, residual=self.gcn_residual,
+        return engine.SUEFunction.apply(self._meta(), history_embedding, candidate_news_representation, user_history_graph,
+                                        user_history_category_mask, user_history_category_indices.long(), *self._params())
+
+    def _meta(self):
+        return dict(hca=self.hca, gcn=self.use_gcn, gcn_layers=self.gcn_layer_num, residual=self.gcn_residual,
                     layer_norm=getattr(self, 'gcn_layer_norm', False),
                     training=self.training, p_drop=float(self.dropout_rate), category_num=self.category_num - 1 if self.hca else 0)
-        return engine.SUEFunction.apply(meta, history_embedding, candidate_news_representation, user_history_graph,
-                                        user_history_category_mask, user_history_category_indices.long(), *self._params())
+
+    def user_side(self, history_embedding, user_history_graph, user_history_category_mask, user_history_category_indices):
+        """inference (eval mode): the part of encode_user that depends on the history alone, computed once for every tile of
+        candidates scored against these users with ``tile_scores`` (engine.sue_user_side)"""
+        user_history_category_mask[:, -1] = 1
+        return engine.sue_user_side(self._meta(), history_embedding, user_history_graph, user_history_category_mask,
+                                    user_history_category_indices.long(), *self._params())
+
+    def tile_scores(self, user_side, candidate_news_representation):
+        """click scores [B, T] of candidates [B, T, D] for the users of ``user_side``: equal, bit for bit, to
+        RowDot(encode_user(...), candidates) on the same inputs (engine.sue_tile_scores)"""
+        return engine.sue_tile_scores(self._meta(), user_side, candidate_news_representation, *self._params())

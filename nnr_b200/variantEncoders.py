@@ -39,6 +39,7 @@ class SUE_wo_GCN(UserEncoder):
     _params = SUE._params
     forward = SUE.forward
     encode_user = SUE.encode_user
+    _meta, user_side, tile_scores = SUE._meta, SUE.user_side, SUE.tile_scores
 
     def __init__(self, news_encoder, config):
         super().__init__(news_encoder, config)
@@ -73,6 +74,7 @@ class SUE_wo_HCA(UserEncoder):
     _params = SUE._params
     forward = SUE.forward
     encode_user = SUE.encode_user
+    _meta, user_side, tile_scores = SUE._meta, SUE.user_side, SUE.tile_scores
 
     def __init__(self, news_encoder, config):
         super().__init__(news_encoder, config)
