@@ -33,7 +33,7 @@
 extern "C" {
 #endif
 
-#define NNR_ABI_VERSION 6
+#define NNR_ABI_VERSION 7
 #define NNR_SEED_INDIRECT (1ULL << 62)
 
 const char* nnr_last_error(void);
@@ -348,6 +348,18 @@ int nnr_rowdot_bwd(const float* dout, const float* a, const float* b, int R, int
 int nnr_topk_merge(const float* scores, int64_t lds, int B, int T, int64_t pos0, const int64_t* tile_ids,
                    const int64_t* exclude, const int32_t* exclude_len, int ldx, int k, int init,
                    float* best_score, int64_t* best_pos, void* stream);
+/* The same merge with at most `cap` entries per group (a news category): tile entry j belongs to group
+ * id_group[tile_ids[j]] (id_group: int32 per news id, values in [0, num_groups); an entry of another group is never kept),
+ * and best_group[B, k] (int32) holds each list entry's group next to best_score / best_pos (-1 for the fill).  The list is
+ * the first k entries of the eligible entries seen so far, taken in the order above, each taken unless `cap` entries of its
+ * group were already taken; the fill entry counts toward nothing.  With cap >= k the result equals nnr_topk_merge's.
+ * Rejects, besides what nnr_topk_merge rejects: cap < 1, num_groups outside [1, NNR_TOPK_MAX_GROUPS], NULL id_group,
+ * best_group or tile_ids.                                                                                             */
+#define NNR_TOPK_MAX_GROUPS 1024
+int nnr_topk_merge_capped(const float* scores, int64_t lds, int B, int T, int64_t pos0, const int64_t* tile_ids,
+                          const int64_t* exclude, const int32_t* exclude_len, int ldx, int k, int init,
+                          const int32_t* id_group, int num_groups, int cap, float* best_score, int64_t* best_pos,
+                          int32_t* best_group, void* stream);
 
 /* elementwise dropout with the library's counter RNG (proxy nodes / cluster features /
  * GCN inter-layer dropout): y = x * keep(seed, i)/(1-p); the same call applies the backward.   */

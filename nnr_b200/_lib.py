@@ -115,6 +115,8 @@ SIGNATURES = {
     'nnr_rowdot_fwd': (C.c_int, [vp, vp, C.c_int, C.c_int, vp, vp]),
     'nnr_rowdot_bwd': (C.c_int, [vp, vp, vp, C.c_int, C.c_int, vp, C.c_int, vp, C.c_int, vp]),
     'nnr_topk_merge': (C.c_int, [vp, i64, C.c_int, C.c_int, i64, vp, vp, vp, C.c_int, C.c_int, C.c_int, vp, vp, vp]),
+    'nnr_topk_merge_capped': (C.c_int, [vp, i64, C.c_int, C.c_int, i64, vp, vp, vp, C.c_int, C.c_int, C.c_int, vp, C.c_int,
+                                        C.c_int, vp, vp, vp, vp]),
     'nnr_dropout': (C.c_int, [vp, i64, f32, u64, vp, vp]),
     'nnr_flat_clip_adam_workspace_bytes': (sz, [i64]),
     'nnr_flat_clip_adam': (C.c_int, [vp, vp, vp, vp, i64, f32, f32, f32, f32, f32, f32, i32, vp, vp, sz, vp]),

@@ -443,7 +443,7 @@ def rowdot_bwd(dout, a, b, R, D, da, accumulate_a, db, accumulate_b):
                              _p(db, _F32), int(accumulate_b), _stream()), 'nnr_rowdot_bwd')
 
 
-TOPK_MAX_K, TOPK_MAX_TILE, TOPK_MAX_EXCLUDE = 1024, 4096, 1024      # include/nnr_b200.h: NNR_TOPK_MAX_*
+TOPK_MAX_K, TOPK_MAX_TILE, TOPK_MAX_EXCLUDE, TOPK_MAX_GROUPS = 1024, 4096, 1024, 1024     # include/nnr_b200.h: NNR_TOPK_MAX_*
 
 
 def topk_merge(scores, pos0, tile_ids, exclude, exclude_len, init, best_score, best_pos):
@@ -454,6 +454,18 @@ def topk_merge(scores, pos0, tile_ids, exclude, exclude_len, init, best_score, b
     check(lib.nnr_topk_merge(_p(scores, _F32), scores.stride(0), B, T, int(pos0), _p(tile_ids, _I64), _p(exclude, _I64),
                              _p(exclude_len, _I32), ldx, best_score.shape[1], int(init), _p(best_score, _F32),
                              _p(best_pos, _I64), _stream()), 'nnr_topk_merge')
+
+
+def topk_merge_capped(scores, pos0, tile_ids, exclude, exclude_len, id_group, num_groups, cap, init, best_score, best_pos,
+                      best_group):
+    """topk_merge keeping at most ``cap`` entries per group: entry j's group is id_group[tile_ids[j]] (int32, in
+    [0, num_groups)), best_group [B, k] int32 holds each list entry's group (nnr_topk_merge_capped)"""
+    B, T = scores.shape
+    ldx = exclude.shape[1] if exclude is not None else 0
+    check(lib.nnr_topk_merge_capped(_p(scores, _F32), scores.stride(0), B, T, int(pos0), _p(tile_ids, _I64),
+                                    _p(exclude, _I64), _p(exclude_len, _I32), ldx, best_score.shape[1], int(init),
+                                    _p(id_group, _I32), int(num_groups), int(cap), _p(best_score, _F32), _p(best_pos, _I64),
+                                    _p(best_group, _I32), _stream()), 'nnr_topk_merge_capped')
 
 
 def dropout(x, p_drop, seed, y):
@@ -525,6 +537,9 @@ _SCHEMAS = {
     'dropout': ('(Tensor x, float p_drop, int seed, Tensor(a!) y) -> ()', dropout),
     'topk_merge': ('(Tensor scores, int pos0, Tensor? tile_ids, Tensor? exclude, Tensor? exclude_len, bool init, '
                    'Tensor(a!) best_score, Tensor(b!) best_pos) -> ()', topk_merge),
+    'topk_merge_capped': ('(Tensor scores, int pos0, Tensor tile_ids, Tensor? exclude, Tensor? exclude_len, Tensor id_group, '
+                          'int num_groups, int cap, bool init, Tensor(a!) best_score, Tensor(b!) best_pos, '
+                          'Tensor(c!) best_group) -> ()', topk_merge_capped),
     'flat_clip_adam': ('(Tensor(a!) param, Tensor grad, Tensor(b!) exp_avg, Tensor(c!) exp_avg_sq, float lr, float beta1, '
                        'float beta2, float eps, float max_norm, float grad_scale, int step, Tensor(d!) norm_out) -> ()',
                        flat_clip_adam),

@@ -15,6 +15,8 @@ runs the single-GPU computation on a contiguous share of the same corpus chunks 
 (``contiguous_blocks``) and one NCCL all-gather assembles the whole result on every rank, so the cache, the ranks and
 the metrics are bit-identical to one GPU.  The all-gathers run on the current stream, outside any captured graph.
 """
+import numbers
+
 import torch
 
 from . import engine, metrics, ops
@@ -58,6 +60,7 @@ class CorpusScorer:
         self.chunk = chunk
         self.cache = None
         self._graphs = {}
+        self._num_groups = None                                 # recommend(max_per_category=): 1 + largest category id
         self.group = process_group
         if process_group is not None:
             import torch.distributed as dist
@@ -207,8 +210,20 @@ class CorpusScorer:
         """recommend()'s candidates per tile for B users: B * T * (C + 1) <= TAIL_ROWS, 1 <= T <= ops.TOPK_MAX_TILE"""
         return max(1, min(ops.TOPK_MAX_TILE, self.TAIL_ROWS // (max(B, 1) * (self._category_num() + 1))))
 
+    def _category_groups(self):
+        """number of groups of the capped merge (1 + the largest corpus category id), after checking once that every
+        category id is in [0, ops.TOPK_MAX_GROUPS)"""
+        if self._num_groups is None:
+            lo, hi = (int(self.cat.min()), int(self.cat.max())) if self.cat.numel() else (0, 0)
+            if lo < 0 or hi >= ops.TOPK_MAX_GROUPS:
+                raise ValueError('CorpusScorer.recommend: max_per_category needs corpus category ids in [0, %d), got [%d, %d]'
+                                 % (ops.TOPK_MAX_GROUPS, lo, hi))
+            self._num_groups = hi + 1
+        return self._num_groups
+
     @torch.no_grad()
-    def recommend(self, history_ids, history_len, pool_ids, k, exclude_history=True, pool_tile=None, cuda_graph=True):
+    def recommend(self, history_ids, history_len, pool_ids, k, exclude_history=True, pool_tile=None, cuda_graph=True,
+                  max_per_category=None):
         """The k best news of a candidate pool for each user: history_ids [B, H] (0-padded at the end) and history_len [B]
         as in ``score``, pool_ids [P] corpus row ids shared by the B users.  Returns (ids [B, k] int64, scores [B, k] fp32),
         best first.
@@ -226,12 +241,24 @@ class CorpusScorer:
         C = 18; T = 107 for B = 256) and at most 4096 candidates.  Full tiles replay one captured CUDA graph per
         (B, H, T); a last partial tile runs eagerly.  Rank-local: never a collective, also with a process group.
         Limits: 1 <= k <= ops.TOPK_MAX_K (1024), 1 <= pool_tile <= ops.TOPK_MAX_TILE (4096), H <= ops.TOPK_MAX_EXCLUDE
-        with ``exclude_history``."""
+        with ``exclude_history``.
+
+        ``max_per_category = m`` caps how many of a user's k news may share a ``news_category`` (the corpus category ids
+        the history is clustered by): the user's eligible pool entries are taken in the order above, each unless m
+        entries of its category were already taken, until k are taken; the rest is filled as above.  Excluded history
+        entries count toward no cap, duplicate pool ids count once per entry.  None, or any m >= k, returns exactly the
+        uncapped result.  m < k runs nnr_topk_merge_capped, which keeps the same k entries of state per user, so memory
+        still does not grow with P.  Corpus category ids must be in [0, ops.TOPK_MAX_GROUPS) (1024)."""
         if self.cache is None:
             raise RuntimeError('CorpusScorer.recommend: call encode_corpus() first')
         k = int(k)
         if not 1 <= k <= ops.TOPK_MAX_K:
             raise ValueError('CorpusScorer.recommend: k must be in [1, %d], got %d' % (ops.TOPK_MAX_K, k))
+        m = max_per_category
+        if m is not None and (isinstance(m, bool) or not isinstance(m, numbers.Integral) or m < 1):
+            raise ValueError('CorpusScorer.recommend: max_per_category must be None or an int >= 1, got %r' % (m,))
+        capped = m is not None and m < k
+        groups = self._category_groups() if capped else None
         pool = torch.as_tensor(pool_ids)
         if pool.dim() != 1 or pool.dtype.is_floating_point or pool.dtype == torch.bool:
             raise ValueError('CorpusScorer.recommend: pool_ids must be a 1-D integer tensor, got %s of shape %s'
@@ -262,6 +289,7 @@ class CorpusScorer:
 
         best_score = torch.empty(B, k, device=self.dev)
         best_pos = torch.empty(B, k, dtype=torch.int64, device=self.dev)
+        best_group = torch.empty(B, k, dtype=torch.int32, device=self.dev) if capped else None
         key = ('recommend', B, H, T, self.cache.data_ptr())
         for a in range(0, P, T):
             ids = pool[a:a + T]
@@ -272,8 +300,12 @@ class CorpusScorer:
                 side = self._graphs[key][0][:-1]
             else:
                 scores = tile_scores(*side, ids)
-            ops.topk_merge(scores, a, ids, hid if exclude_history else None, hl if exclude_history else None, a == 0,
-                           best_score, best_pos)
+            if capped:
+                ops.topk_merge_capped(scores, a, ids, hid if exclude_history else None, hl if exclude_history else None,
+                                      self.cat.contiguous(), groups, int(m), a == 0, best_score, best_pos, best_group)
+            else:
+                ops.topk_merge(scores, a, ids, hid if exclude_history else None, hl if exclude_history else None, a == 0,
+                               best_score, best_pos)
         ids = torch.where(best_pos >= 0, pool[best_pos.clamp(min=0)], torch.full_like(best_pos, -1))
         return ids, best_score
 
