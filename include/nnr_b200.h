@@ -33,7 +33,7 @@
 extern "C" {
 #endif
 
-#define NNR_ABI_VERSION 7
+#define NNR_ABI_VERSION 8
 #define NNR_SEED_INDIRECT (1ULL << 62)
 
 const char* nnr_last_error(void);
@@ -360,6 +360,19 @@ int nnr_topk_merge_capped(const float* scores, int64_t lds, int B, int T, int64_
                           const int64_t* exclude, const int32_t* exclude_len, int ldx, int k, int init,
                           const int32_t* id_group, int num_groups, int cap, float* best_score, int64_t* best_pos,
                           int32_t* best_group, void* stream);
+/* The same merges of entries that carry their own pool positions: entry j of row b has score scores[b*lds + j] and
+ * position pos[b*ldp + j] (int64), and in the capped variant group grp[b*ldg + j] (int32), instead of pos0 + j and
+ * id_group[tile_ids[j]].  A negative position is an empty slot (the fill entry of a best list) and is dropped before
+ * anything else; a real entry scoring -inf is kept.  No exclusion list.  Used to fold the per-rank best lists of a
+ * data-parallel CorpusScorer.recommend() into one: positions of different calls' entries must be distinct (keys are
+ * unique), and must be < 2^31 - 1.  Order, state, determinism and limits are those of nnr_topk_merge[_capped]; a best
+ * list of k entries fits T = k.  Rejects, besides what nnr_topk_merge[_capped] rejects: NULL pos, ldp < T, and in the
+ * capped variant NULL grp or best_group and ldg < T.                                                                 */
+int nnr_topk_merge_lists(const float* scores, int64_t lds, int B, int T, const int64_t* pos, int64_t ldp,
+                         int k, int init, float* best_score, int64_t* best_pos, void* stream);
+int nnr_topk_merge_lists_capped(const float* scores, int64_t lds, int B, int T, const int64_t* pos, int64_t ldp,
+                                const int32_t* grp, int64_t ldg, int num_groups, int cap, int k, int init,
+                                float* best_score, int64_t* best_pos, int32_t* best_group, void* stream);
 
 /* elementwise dropout with the library's counter RNG (proxy nodes / cluster features /
  * GCN inter-layer dropout): y = x * keep(seed, i)/(1-p); the same call applies the backward.   */

@@ -13,6 +13,10 @@
 // The capped variant (nnr_topk_merge_capped) keeps at most `group_cap` entries per group (news category): every key
 // carries its group through the sort, and one warp then walks the sorted keys in order, keeping an entry while fewer than
 // group_cap entries of its group were kept before it, until k are kept.  Why the k-entry state stays exact: DESIGN.md §4.
+//
+// The list variants (nnr_topk_merge_lists[_capped], LISTS) merge a [B, T] block of entries that carry their own pool
+// position pos[b, j] (and group grp[b, j]) instead of pos0 + j and id_group[tile_ids[j]]: the per-rank best lists of a
+// data-parallel recommend() call, folded into one.  A negative position is an empty (fill) slot and is dropped first.
 #include "common.cuh"
 #include "../../include/nnr_b200.h"
 
@@ -45,13 +49,15 @@ __device__ __forceinline__ void topk_unkey(uint64_t key, float* s, int64_t* pos)
 }
 
 // shared memory: key[cap] (cap = next power of two >= k + T), then the row's exclusion ids [ldx]; CAPPED adds each key's
-// group grp[cap] and the per-group counters cnt[num_groups]
-template <bool CAPPED>
+// group grp[cap] and the per-group counters cnt[num_groups].  LISTS reads positions from list_pos [B, ldp] and groups from
+// list_grp [B, ldg]; it has no exclusion list.
+template <bool CAPPED, bool LISTS>
 __global__ void __launch_bounds__(TOPK_THREADS) topk_merge_kernel(
     const float* __restrict__ scores, int64_t lds, int T, int64_t pos0, const int64_t* __restrict__ tile_ids,
     const int64_t* __restrict__ excl, const int32_t* __restrict__ excl_len, int ldx, int k, int cap, int init,
     float* __restrict__ best_score, int64_t* __restrict__ best_pos, const int32_t* __restrict__ id_group, int num_groups,
-    int group_cap, int32_t* __restrict__ best_group) {
+    int group_cap, int32_t* __restrict__ best_group, const int64_t* __restrict__ list_pos, int64_t ldp,
+    const int32_t* __restrict__ list_grp, int64_t ldg) {
   extern __shared__ uint64_t topk_smem[];
   uint64_t* key = topk_smem;
   int64_t* s_excl = reinterpret_cast<int64_t*>(topk_smem + cap);
@@ -81,9 +87,14 @@ __global__ void __launch_bounds__(TOPK_THREADS) topk_merge_kernel(
   const uint64_t thr = s_thr;                                  // the k-th best so far: only keys above it can enter
   const float* row = scores + (size_t)b * lds;
   for (int j = tid; j < T; j += blockDim.x) {
-    const uint64_t kk = topk_key(row[j], pos0 + j);
+    int64_t p = pos0 + j;
+    if constexpr (LISTS) {
+      p = list_pos[(size_t)b * ldp + j];
+      if (p < 0) continue;                                      // an empty slot of the list, not a -inf entry
+    }
+    const uint64_t kk = topk_key(row[j], p);
     if (kk <= thr) continue;
-    if (nx > 0) {
+    if (!LISTS && nx > 0) {
       const int64_t id = tile_ids[j];
       bool hit = false;
       for (int h = 0; h < nx && !hit; ++h) hit = s_excl[h] == id;
@@ -91,7 +102,10 @@ __global__ void __launch_bounds__(TOPK_THREADS) topk_merge_kernel(
     }
     const int slot = k + atomicAdd(&s_m, 1);
     key[slot] = kk;
-    if constexpr (CAPPED) grp[slot] = id_group[tile_ids[j]];
+    if constexpr (CAPPED) {
+      if constexpr (LISTS) grp[slot] = list_grp[(size_t)b * ldg + j];
+      else grp[slot] = id_group[tile_ids[j]];
+    }
   }
   __syncthreads();
   const int m = s_m;
@@ -187,11 +201,11 @@ static int topk_check(const char* who, const float* scores, int64_t lds, int B, 
   return 0;
 }
 
-template <bool CAPPED>
+template <bool CAPPED, bool LISTS>
 static int topk_launch(const float* scores, int64_t lds, int B, int T, int64_t pos0, const int64_t* tile_ids,
                        const int64_t* exclude, const int32_t* exclude_len, int ldx, int k, int init, float* best_score,
                        int64_t* best_pos, const int32_t* id_group, int num_groups, int group_cap, int32_t* best_group,
-                       void* stream) {
+                       const int64_t* list_pos, int64_t ldp, const int32_t* list_grp, int64_t ldg, void* stream) {
   if (B == 0) return 0;
   int cap = 1;
   while (cap < k + T) cap <<= 1;
@@ -205,14 +219,16 @@ static int topk_launch(const float* scores, int64_t lds, int B, int T, int64_t p
     if (dev >= 64 || !attr_set[dev]) {
       // cap <= 8192 for k + T <= 5120
       const int most = (8192 + NNR_TOPK_MAX_EXCLUDE) * 8 + (CAPPED ? (8192 + NNR_TOPK_MAX_GROUPS) * 4 : 0);
-      NNR_CUDA(cudaFuncSetAttribute((const void*)topk_merge_kernel<CAPPED>, cudaFuncAttributeMaxDynamicSharedMemorySize, most));
+      NNR_CUDA(cudaFuncSetAttribute((const void*)topk_merge_kernel<CAPPED, LISTS>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                    most));
       if (dev < 64) attr_set[dev] = true;
     }
   }
-  topk_merge_kernel<CAPPED><<<B, TOPK_THREADS, smem, (cudaStream_t)stream>>>(
+  topk_merge_kernel<CAPPED, LISTS><<<B, TOPK_THREADS, smem, (cudaStream_t)stream>>>(
       scores, lds, T, pos0, tile_ids, exclude, exclude_len, nx, k, cap, init, best_score, best_pos, id_group, num_groups,
-      group_cap, best_group);
-  NNR_LAUNCH_CHECK(CAPPED ? "topk_merge_kernel<capped>" : "topk_merge_kernel");
+      group_cap, best_group, list_pos, ldp, list_grp, ldg);
+  NNR_LAUNCH_CHECK(LISTS ? (CAPPED ? "topk_merge_kernel<capped, lists>" : "topk_merge_kernel<lists>")
+                         : (CAPPED ? "topk_merge_kernel<capped>" : "topk_merge_kernel"));
   return 0;
 }
 
@@ -222,8 +238,8 @@ extern "C" int nnr_topk_merge(const float* scores, int64_t lds, int B, int T, in
   const int rc = topk_check("nnr_topk_merge", scores, lds, B, T, pos0, tile_ids, exclude, exclude_len, ldx, k, best_score,
                             best_pos);
   if (rc) return rc;
-  return topk_launch<false>(scores, lds, B, T, pos0, tile_ids, exclude, exclude_len, ldx, k, init, best_score, best_pos,
-                            nullptr, 0, 0, nullptr, stream);
+  return topk_launch<false, false>(scores, lds, B, T, pos0, tile_ids, exclude, exclude_len, ldx, k, init, best_score,
+                                   best_pos, nullptr, 0, 0, nullptr, nullptr, 0, nullptr, 0, stream);
 }
 
 extern "C" int nnr_topk_merge_capped(const float* scores, int64_t lds, int B, int T, int64_t pos0, const int64_t* tile_ids,
@@ -237,6 +253,40 @@ extern "C" int nnr_topk_merge_capped(const float* scores, int64_t lds, int B, in
   NNR_REQUIRE(num_groups >= 1 && num_groups <= NNR_TOPK_MAX_GROUPS, NNR_ERR_ARG, "%s: num_groups must be in [1, %d], got %d",
               who, NNR_TOPK_MAX_GROUPS, num_groups);
   NNR_REQUIRE(id_group && best_group && tile_ids, NNR_ERR_ARG, "%s: id_group, best_group and tile_ids must not be NULL", who);
-  return topk_launch<true>(scores, lds, B, T, pos0, tile_ids, exclude, exclude_len, ldx, k, init, best_score, best_pos,
-                           id_group, num_groups, cap, best_group, stream);
+  return topk_launch<true, false>(scores, lds, B, T, pos0, tile_ids, exclude, exclude_len, ldx, k, init, best_score,
+                                  best_pos, id_group, num_groups, cap, best_group, nullptr, 0, nullptr, 0, stream);
+}
+
+// the checks nnr_topk_merge_lists and nnr_topk_merge_lists_capped share (those of topk_check for a tile at position 0
+// without exclusion list, plus pos and ldp)
+static int topk_lists_check(const char* who, const float* scores, int64_t lds, int B, int T, const int64_t* pos, int64_t ldp,
+                            int k, const float* best_score, const int64_t* best_pos) {
+  const int rc = topk_check(who, scores, lds, B, T, 0, nullptr, nullptr, nullptr, 0, k, best_score, best_pos);
+  if (rc) return rc;
+  NNR_REQUIRE(pos, NNR_ERR_ARG, "%s: pos must not be NULL", who);
+  NNR_REQUIRE(ldp >= T, NNR_ERR_ARG, "%s: ldp (%lld) < T (%d)", who, (long long)ldp, T);
+  return 0;
+}
+
+extern "C" int nnr_topk_merge_lists(const float* scores, int64_t lds, int B, int T, const int64_t* pos, int64_t ldp, int k,
+                                    int init, float* best_score, int64_t* best_pos, void* stream) {
+  const int rc = topk_lists_check("nnr_topk_merge_lists", scores, lds, B, T, pos, ldp, k, best_score, best_pos);
+  if (rc) return rc;
+  return topk_launch<false, true>(scores, lds, B, T, 0, nullptr, nullptr, nullptr, 0, k, init, best_score, best_pos, nullptr,
+                                  0, 0, nullptr, pos, ldp, nullptr, 0, stream);
+}
+
+extern "C" int nnr_topk_merge_lists_capped(const float* scores, int64_t lds, int B, int T, const int64_t* pos, int64_t ldp,
+                                           const int32_t* grp, int64_t ldg, int num_groups, int cap, int k, int init,
+                                           float* best_score, int64_t* best_pos, int32_t* best_group, void* stream) {
+  const char* who = "nnr_topk_merge_lists_capped";
+  const int rc = topk_lists_check(who, scores, lds, B, T, pos, ldp, k, best_score, best_pos);
+  if (rc) return rc;
+  NNR_REQUIRE(grp && best_group, NNR_ERR_ARG, "%s: grp and best_group must not be NULL", who);
+  NNR_REQUIRE(ldg >= T, NNR_ERR_ARG, "%s: ldg (%lld) < T (%d)", who, (long long)ldg, T);
+  NNR_REQUIRE(cap >= 1, NNR_ERR_ARG, "%s: cap must be >= 1, got %d", who, cap);
+  NNR_REQUIRE(num_groups >= 1 && num_groups <= NNR_TOPK_MAX_GROUPS, NNR_ERR_ARG, "%s: num_groups must be in [1, %d], got %d",
+              who, NNR_TOPK_MAX_GROUPS, num_groups);
+  return topk_launch<true, true>(scores, lds, B, T, 0, nullptr, nullptr, nullptr, 0, k, init, best_score, best_pos, nullptr,
+                                 num_groups, cap, best_group, pos, ldp, grp, ldg, stream);
 }

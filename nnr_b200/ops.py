@@ -468,6 +468,25 @@ def topk_merge_capped(scores, pos0, tile_ids, exclude, exclude_len, id_group, nu
                                     _p(best_group, _I32), _stream()), 'nnr_topk_merge_capped')
 
 
+def topk_merge_lists(scores, pos, init, best_score, best_pos):
+    """merge entries scores [B, T] whose pool positions are pos [B, T] (int64; < 0: an empty slot, skipped) into the running
+    best list best_score / best_pos [B, k]: folds best lists of disjoint position sets into one (nnr_topk_merge_lists)"""
+    B, T = scores.shape
+    check(lib.nnr_topk_merge_lists(_p(scores, _F32), scores.stride(0), B, T, _p(pos, _I64), pos.stride(0),
+                                   best_score.shape[1], int(init), _p(best_score, _F32), _p(best_pos, _I64), _stream()),
+          'nnr_topk_merge_lists')
+
+
+def topk_merge_lists_capped(scores, pos, grp, num_groups, cap, init, best_score, best_pos, best_group):
+    """topk_merge_lists keeping at most ``cap`` entries per group: entry (b, j)'s group is grp[b, j] (int32, in
+    [0, num_groups)), best_group [B, k] int32 holds each list entry's group (nnr_topk_merge_lists_capped)"""
+    B, T = scores.shape
+    check(lib.nnr_topk_merge_lists_capped(_p(scores, _F32), scores.stride(0), B, T, _p(pos, _I64), pos.stride(0),
+                                          _p(grp, _I32), grp.stride(0), int(num_groups), int(cap), best_score.shape[1],
+                                          int(init), _p(best_score, _F32), _p(best_pos, _I64), _p(best_group, _I32),
+                                          _stream()), 'nnr_topk_merge_lists_capped')
+
+
 def dropout(x, p_drop, seed, y):
     check(lib.nnr_dropout(_p(x, _F32), x.numel(), float(p_drop), int(seed), _p(y, _F32), _stream()), 'nnr_dropout')
 
@@ -540,6 +559,11 @@ _SCHEMAS = {
     'topk_merge_capped': ('(Tensor scores, int pos0, Tensor tile_ids, Tensor? exclude, Tensor? exclude_len, Tensor id_group, '
                           'int num_groups, int cap, bool init, Tensor(a!) best_score, Tensor(b!) best_pos, '
                           'Tensor(c!) best_group) -> ()', topk_merge_capped),
+    'topk_merge_lists': ('(Tensor scores, Tensor pos, bool init, Tensor(a!) best_score, Tensor(b!) best_pos) -> ()',
+                         topk_merge_lists),
+    'topk_merge_lists_capped': ('(Tensor scores, Tensor pos, Tensor grp, int num_groups, int cap, bool init, '
+                                'Tensor(a!) best_score, Tensor(b!) best_pos, Tensor(c!) best_group) -> ()',
+                                topk_merge_lists_capped),
     'flat_clip_adam': ('(Tensor(a!) param, Tensor grad, Tensor(b!) exp_avg, Tensor(c!) exp_avg_sq, float lr, float beta1, '
                        'float beta2, float eps, float max_norm, float grad_scale, int step, Tensor(d!) norm_out) -> ()',
                        flat_clip_adam),

@@ -14,6 +14,8 @@ Data parallel (SURVEY 8e): with a ``process_group``, ``encode_corpus`` and ``eva
 runs the single-GPU computation on a contiguous share of the same corpus chunks / impression batches
 (``contiguous_blocks``) and one NCCL all-gather assembles the whole result on every rank, so the cache, the ranks and
 the metrics are bit-identical to one GPU.  The all-gathers run on the current stream, outside any captured graph.
+``recommend(collective=True)`` shares the pool tiles the same way: each rank folds its tiles into a k-entry best list, and
+the all-gathered rank lists are merged into one on every rank (``nnr_topk_merge_lists``).
 """
 import numbers
 
@@ -40,7 +42,8 @@ def _checksum(t):
 class CorpusScorer:
     """``process_group=None`` scores on this process's device alone.  With an NCCL group, ``encode_corpus`` and
     ``evaluate`` are collectives: every rank of the group calls them with the same arguments (and the same weights, as
-    ``TrainStep`` keeps them) and gets the whole result.  ``score`` and ``recommend`` are always rank-local.
+    ``TrainStep`` keeps them) and gets the whole result.  ``score`` is always rank-local; ``recommend`` is rank-local unless
+    called with ``collective=True``.
     ``graph_flags`` = ``ops.graph_flags(...)`` of the options the model was trained with (no_self_connection,
     no_adjacent_normalization, gcn_normalization_type); 0 is the reference's default symmetric graph."""
 
@@ -103,7 +106,8 @@ class CorpusScorer:
 
     # fields of the descriptor every rank contributes before the first collective of a call
     _FIELDS = ('call', 'news_num', 'chunk', 'D', 'I', 'n_max', 'H', 'batch', 'corpus ids checksum', 'history_ids checksum',
-               'history_len checksum', 'candidate_ids checksum', 'candidate_count checksum', 'labels checksum')
+               'history_len checksum', 'candidate_ids checksum', 'candidate_count checksum', 'labels checksum', 'B', 'P', 'k',
+               'T', 'm', 'exclude_history', 'pool_ids checksum', 'argument error')
 
     def _agree(self, call, **fields):
         """all-gather a small int64 descriptor of this call's inputs and raise on every rank if any field differs between
@@ -120,7 +124,7 @@ class CorpusScorer:
         if bad:
             what = '; '.join('%s: %s' % (self._FIELDS[i], table[:, i].tolist()) for i in bad)
             raise RuntimeError('CorpusScorer.%s: the ranks of the process group were called with different arguments (%s). '
-                               'Every rank must pass the same inputs.' % (('encode_corpus', 'evaluate')[call - 1], what))
+                               'Every rank must pass the same inputs.' % (('encode_corpus', 'evaluate', 'recommend')[call - 1], what))
 
     def _corpus_fields(self):
         return dict(news_num=self.tt.shape[0], chunk=self.chunk, D=self.model.news_encoder.news_embedding_dim)
@@ -223,7 +227,7 @@ class CorpusScorer:
 
     @torch.no_grad()
     def recommend(self, history_ids, history_len, pool_ids, k, exclude_history=True, pool_tile=None, cuda_graph=True,
-                  max_per_category=None):
+                  max_per_category=None, collective=False):
         """The k best news of a candidate pool for each user: history_ids [B, H] (0-padded at the end) and history_len [B]
         as in ``score``, pool_ids [P] corpus row ids shared by the B users.  Returns (ids [B, k] int64, scores [B, k] fp32),
         best first.
@@ -239,7 +243,7 @@ class CorpusScorer:
         ``pool_tile`` candidates, each folded into a running top-k list by nnr_topk_merge.  Memory does not grow with P.
         The default tile holds B * T * (C + 1) <= TAIL_ROWS = 2^19 rows of the cluster tail (about 7.5 GB at D = 900,
         C = 18; T = 107 for B = 256) and at most 4096 candidates.  Full tiles replay one captured CUDA graph per
-        (B, H, T); a last partial tile runs eagerly.  Rank-local: never a collective, also with a process group.
+        (B, H, T); a last partial tile runs eagerly.
         Limits: 1 <= k <= ops.TOPK_MAX_K (1024), 1 <= pool_tile <= ops.TOPK_MAX_TILE (4096), H <= ops.TOPK_MAX_EXCLUDE
         with ``exclude_history``.
 
@@ -248,7 +252,33 @@ class CorpusScorer:
         entries of its category were already taken, until k are taken; the rest is filled as above.  Excluded history
         entries count toward no cap, duplicate pool ids count once per entry.  None, or any m >= k, returns exactly the
         uncapped result.  m < k runs nnr_topk_merge_capped, which keeps the same k entries of state per user, so memory
-        still does not grow with P.  Corpus category ids must be in [0, ops.TOPK_MAX_GROUPS) (1024)."""
+        still does not grow with P.  Corpus category ids must be in [0, ops.TOPK_MAX_GROUPS) (1024).
+
+        ``collective=False`` is rank-local: never a collective, also with a process group.  ``collective=True`` needs a
+        scorer with a process group and is a collective: every rank calls it with the same arguments, after
+        ``encode_corpus()``.  Rank r scores the pool tiles [a, a + T) of its contiguous share (``contiguous_blocks`` of the
+        ceil(P / T) tiles) into its own k-entry list, one all-gather brings every rank's list to every rank, and
+        nnr_topk_merge_lists[_capped] folds them in rank order.  Every rank returns the whole result, bit-identical to a
+        plain call with the same arguments (the same ``pool_tile``) on one GPU.  The ranks first all-gather a descriptor
+        of their arguments: if it differs between ranks, or the arguments fail a check on some ranks only, every rank
+        raises RuntimeError naming the fields; a check that fails on every rank raises its ValueError there.  Either way
+        no rank is left in a collective, and the group can be used for the next call."""
+        if collective:
+            return self._recommend_collective(history_ids, history_len, pool_ids, k, exclude_history, pool_tile, cuda_graph,
+                                              max_per_category)
+        hid, hl, pool, k, T, m, groups = self._recommend_inputs(history_ids, history_len, pool_ids, k, exclude_history,
+                                                                pool_tile, max_per_category)
+        B, P = hid.shape[0], pool.numel()
+        if P == 0 or B == 0:
+            best_score, best_pos, _ = self._fill(B, k)
+            return best_pos, best_score                         # ids -1, scores -inf
+        best_score, best_pos, _ = self._recommend_tiles(hid, hl, pool, k, T, 0, -(-P // T), exclude_history, m, groups,
+                                                        cuda_graph)
+        return self._pool_ids(pool, best_pos), best_score
+
+    def _recommend_inputs(self, history_ids, history_len, pool_ids, k, exclude_history, pool_tile, max_per_category):
+        """recommend()'s argument checks, before any kernel launch.  Returns (hid [B, H] int64, hl [B] int32, pool [P] int64
+        on the device, k, T, m (None when uncapped), the number of category groups (None when uncapped))."""
         if self.cache is None:
             raise RuntimeError('CorpusScorer.recommend: call encode_corpus() first')
         k = int(k)
@@ -275,11 +305,24 @@ class CorpusScorer:
             raise ValueError('CorpusScorer.recommend: pool_tile must be in [1, %d], got %d' % (ops.TOPK_MAX_TILE, T))
         if exclude_history and H > ops.TOPK_MAX_EXCLUDE:
             raise ValueError('CorpusScorer.recommend: exclude_history takes at most %d history ids, got %d' % (ops.TOPK_MAX_EXCLUDE, H))
-        pool = pool.to(self.dev).long()
+        return hid, hl, pool.to(self.dev).long(), k, T, (int(m) if capped else None), groups
+
+    def _fill(self, B, k, capped=False):
+        """an empty best list: (score -inf, position -1, group -1 or None)"""
+        return (torch.full((B, k), float('-inf'), device=self.dev), torch.full((B, k), -1, dtype=torch.int64, device=self.dev),
+                torch.full((B, k), -1, dtype=torch.int32, device=self.dev) if capped else None)
+
+    @staticmethod
+    def _pool_ids(pool, best_pos):
+        return torch.where(best_pos >= 0, pool[best_pos.clamp(min=0)], torch.full_like(best_pos, -1))
+
+    def _recommend_tiles(self, hid, hl, pool, k, T, first, end, exclude_history, m, groups, cuda_graph):
+        """the best list of pool tiles [first, end) (tile t: pool positions [t * T, min((t + 1) * T, P))): returns
+        (best_score [B, k], best_pos [B, k] pool positions, best_group [B, k] or None when m is None).  No tiles: the fill."""
+        B, H = hid.shape
         P = pool.numel()
-        if P == 0 or B == 0:
-            return (torch.full((B, k), -1, dtype=torch.int64, device=self.dev),
-                    torch.full((B, k), float('-inf'), device=self.dev))
+        if first >= end:
+            return self._fill(B, k, m is not None)
         ue = self.model.user_encoder
         side = ue.user_side(self.cache[hid], *self._history_graph(hid, hl))
 
@@ -289,9 +332,9 @@ class CorpusScorer:
 
         best_score = torch.empty(B, k, device=self.dev)
         best_pos = torch.empty(B, k, dtype=torch.int64, device=self.dev)
-        best_group = torch.empty(B, k, dtype=torch.int32, device=self.dev) if capped else None
+        best_group = torch.empty(B, k, dtype=torch.int32, device=self.dev) if m is not None else None
         key = ('recommend', B, H, T, self.cache.data_ptr())
-        for a in range(0, P, T):
+        for a in range(first * T, min(end * T, P), T):
             ids = pool[a:a + T]
             if cuda_graph and ids.numel() == T:
                 scores = self._graphed(key, tile_scores, (*side, ids))
@@ -300,14 +343,76 @@ class CorpusScorer:
                 side = self._graphs[key][0][:-1]
             else:
                 scores = tile_scores(*side, ids)
-            if capped:
+            init = a == first * T
+            if m is not None:
                 ops.topk_merge_capped(scores, a, ids, hid if exclude_history else None, hl if exclude_history else None,
-                                      self.cat.contiguous(), groups, int(m), a == 0, best_score, best_pos, best_group)
+                                      self.cat.contiguous(), groups, m, init, best_score, best_pos, best_group)
             else:
-                ops.topk_merge(scores, a, ids, hid if exclude_history else None, hl if exclude_history else None, a == 0,
+                ops.topk_merge(scores, a, ids, hid if exclude_history else None, hl if exclude_history else None, init,
                                best_score, best_pos)
-        ids = torch.where(best_pos >= 0, pool[best_pos.clamp(min=0)], torch.full_like(best_pos, -1))
-        return ids, best_score
+        return best_score, best_pos, best_group
+
+    def _merge_rank_lists(self, scores, pos, grp, m, groups):
+        """fold W best lists scores / pos (/ grp) [W, B, k] of disjoint pool positions into one, in rank order
+        (nnr_topk_merge_lists[_capped], one launch per list).  Returns (best_score [B, k], best_pos [B, k])."""
+        W, B, k = scores.shape
+        best_score = torch.empty(B, k, device=self.dev)
+        best_pos = torch.empty(B, k, dtype=torch.int64, device=self.dev)
+        best_group = torch.empty(B, k, dtype=torch.int32, device=self.dev) if m is not None else None
+        for r in range(W):
+            if m is not None:
+                ops.topk_merge_lists_capped(scores[r], pos[r], grp[r], groups, m, r == 0, best_score, best_pos, best_group)
+            else:
+                ops.topk_merge_lists(scores[r], pos[r], r == 0, best_score, best_pos)
+        return best_score, best_pos
+
+    def _recommend_collective(self, history_ids, history_len, pool_ids, k, exclude_history, pool_tile, cuda_graph,
+                              max_per_category):
+        """recommend(collective=True): agree on the arguments, score this rank's share of the tiles, all-gather the rank
+        lists and merge them"""
+        if self.group is None:
+            raise ValueError('CorpusScorer.recommend: collective=True needs a scorer built with a process_group')
+        err = None
+        try:
+            hid, hl, pool, k, T, m, groups = self._recommend_inputs(history_ids, history_len, pool_ids, k, exclude_history,
+                                                                    pool_tile, max_per_category)
+        except (ValueError, RuntimeError) as e:        # raised after the agreement, so that no rank waits in a collective
+            err = e
+        fields = {'argument error': int(err is not None)}
+        if err is None:
+            fields.update({'B': hid.shape[0], 'H': hid.shape[1], 'P': pool.numel(), 'k': k, 'T': T,
+                           'm': 0 if max_per_category is None else int(max_per_category),
+                           'exclude_history': int(bool(exclude_history)), 'pool_ids checksum': _checksum(pool),
+                           'history_ids checksum': _checksum(hid), 'history_len checksum': _checksum(hl)})
+        try:
+            self._agree(3, **self._corpus_fields(), **{'corpus ids checksum': self._corpus_sum or 0}, **fields)
+        except RuntimeError as e:
+            if err is not None:
+                raise RuntimeError('%s On this rank: %s' % (e, err)) from err
+            raise
+        if err is not None:
+            raise err
+        B, P = hid.shape[0], pool.numel()
+        if P == 0 or B == 0:
+            best_score, best_pos, _ = self._fill(B, k)
+            return best_pos, best_score                         # ids -1, scores -inf
+        _, parts = contiguous_blocks(-(-P // T), self.world)
+        first, end = parts[self.rank]
+        mine = self._recommend_tiles(hid, hl, pool, k, T, first, end, exclude_history, m, groups, cuda_graph)
+        best_score, best_pos = self._gather_and_merge(mine, m, groups)
+        return self._pool_ids(pool, best_pos), best_score
+
+    def _gather_and_merge(self, mine, m, groups):
+        """all-gather every rank's best list ``mine`` = (score, pos, group or None) [B, k] and fold them into one"""
+        import torch.distributed as dist
+        B, k = mine[0].shape
+        gathered = []
+        for t in mine:
+            if t is not None:
+                out = torch.empty(self.world * B, k, dtype=t.dtype, device=self.dev)
+                dist.all_gather_into_tensor(out, t, group=self.group)
+                gathered.append(out.view(self.world, B, k))
+        return self._merge_rank_lists(gathered[0], gathered[1], gathered[2] if m is not None else None, m, groups)
 
     @torch.no_grad()
     def _impression_scores(self, history_ids, history_len, candidate_ids, batch, candidate_count=None, labels=None):
