@@ -8,7 +8,6 @@
 //   mode 0: score = w2 . U[p]                 (U = tanh(W1 x + b1) produced by nnr_gemm's epilogue)
 //   mode 1: score = scale * X[p] . qvec[s]    (K folded onto the query: (K x).(q) == x.(K^T q))
 #include "common.cuh"
-#include <stdlib.h>
 #include "../../include/nnr_b200.h"
 
 #define POOL_THREADS 128       // backward kernels
@@ -337,14 +336,12 @@ extern "C" int nnr_attn_pool_fwd(const nnr_pool_args* a, void* stream) {
 extern "C" int nnr_attn_pool_bwd(const nnr_pool_args* a, void* stream) {
   int rc = pool_validate(a, true);
   if (rc) return rc;
-  static int rows_mode = -1;
-  if (rows_mode < 0) { const char* e = getenv("NNR_POOL_BWD_ROWS"); rows_mode = (e && e[0] == '0') ? 0 : 1; }
   const bool al = nnr_aligned16(a->X) && nnr_aligned16(a->dX) && nnr_aligned16(a->dpooled) && a->ldx % 4 == 0 && a->lddx % 4 == 0 &&
                   a->lddp % 4 == 0 && a->D % 4 == 0 && a->D <= 128 * POOL_K4;
   const bool al0 = a->mode != 0 || (nnr_aligned16(a->U) && nnr_aligned16(a->dU) && nnr_aligned16(a->w2) && nnr_aligned16(a->dw2_partial) &&
                                     a->ldu % 4 == 0 && a->lddu % 4 == 0 && a->A % 4 == 0 && a->A <= 128 * POOL_K4);
   const bool al1 = a->mode != 1 || (nnr_aligned16(a->qvec) && a->ldq % 4 == 0 && (!a->dqvec || (nnr_aligned16(a->dqvec) && a->lddq % 4 == 0)));
-  if (rows_mode && al && al0 && al1) {
+  if (al && al0 && al1) {
     const int ml4 = (a->max_len + 3) / 4 * 4;
     const int R = a->mode == 1 ? a->D : a->A;
     const size_t smem = ((size_t)2 * ml4 + a->D + (a->mode == 1 ? a->D : 0) + (size_t)(POOL_THREADS / 32) * R) * sizeof(float);

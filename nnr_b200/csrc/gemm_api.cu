@@ -15,8 +15,7 @@ static int default_algo() {
   static int algo = -1;
   if (algo < 0) {
     const char* e = getenv("NNR_GEMM_ALGO");
-    const char* off = getenv("NNR_DISABLE_TC");        // debugging switch: no tensor-core kernels -> no operand planes either
-    if ((off && off[0] == '1') || (e && !strcmp(e, "simt"))) algo = NNR_GEMM_SIMT_FP32;
+    if (e && !strcmp(e, "simt")) algo = NNR_GEMM_SIMT_FP32;
     else if (e && !strcmp(e, "tf32x3")) algo = NNR_GEMM_TC_TF32X3;
     else if (e && !strcmp(e, "bf16")) algo = NNR_GEMM_TC_BF16;
     else if (e && !strcmp(e, "bf16x3")) algo = NNR_GEMM_TC_BF16X3;

@@ -34,7 +34,6 @@
 #include "gemm_epilogue.cuh"
 #include <cuda.h>
 #include <cuda_bf16.h>
-#include <stdlib.h>
 
 extern "C" int nnr_gemm_default_algo(void);
 
@@ -1007,16 +1006,6 @@ struct TcPlan {
   size_t a_plane, b_plane, a_off, b_off, partial_off, total, smem;
 };
 
-static double stage_penalty() {
-  static double v = -1.0;
-  if (v < 0) { const char* e = getenv("NNR_TC_STAGE_PENALTY"); v = e ? atof(e) : 1.3; }   // measured: a two-stage ring loses more than the larger tile gains
-  return v;
-}
-static double stage_penalty3() {
-  static double v = -1.0;
-  if (v < 0) { const char* e = getenv("NNR_TC_STAGE_PENALTY3"); v = e ? atof(e) : 1.0; }
-  return v;
-}
 static int pick_block_n(int N, int step, int nplanes) {
   int best = step;
   double best_cost = 1e30;
@@ -1024,9 +1013,9 @@ static int pick_block_n(int N, int step, int nplanes) {
     double padded = (double)((N + bn - 1) / bn) * bn;
     double cost = padded * (1.0 + 40.0 / bn);
     // a two-stage ring cannot hide the TMA latency behind one stage of MMAs: prefer tiles that leave room for three
+    // (measured: a two-stage ring loses more than the larger tile gains)
     size_t stage = (size_t)nplanes * ((size_t)TC_BM * 128 + (size_t)bn * 128);
-    if (TC_SMEM_BUDGET / stage < 3) cost *= stage_penalty();
-    else if (TC_SMEM_BUDGET / stage < 4) cost *= stage_penalty3();
+    if (TC_SMEM_BUDGET / stage < 3) cost *= 1.3;
     if (cost < best_cost - 1e-9) { best_cost = cost; best = bn; }
   }
   return best;
@@ -1034,33 +1023,6 @@ static int pick_block_n(int N, int step, int nplanes) {
 
 // CTA-pair tiles: 256 x bn with bn <= 256, bn % 16 == 0 (K-major B) or % 128 == 0 (MN-major B: each CTA holds whole 64-wide
 // groups), three pipeline stages required.  Returns 0 when no such tile keeps the padding reasonable.
-static int chain_k_limit() {
-  static int v = -1;
-  if (v < 0) { const char* e = getenv("NNR_TC_CHAIN_K"); v = e ? atoi(e) : TC_CHAIN_K; if (v < 256) v = 256; }
-  return v;
-}
-static int fast_epilogue_enabled() {
-  static int v = -1;
-  if (v < 0) { const char* e = getenv("NNR_TC_FAST_EPILOGUE"); v = e ? atoi(e) : 1; }
-  return v;
-}
-static int pair_mode() {
-  static int v = -1;
-  if (v < 0) { const char* e = getenv("NNR_TC_PAIR"); v = e ? atoi(e) : 1; }
-  return v;
-}
-// Row count from which 256-row pair tiles are considered, and the least number of pair tiles a mid-size problem must have
-// (below it the 128-row grid fills more SMs).  Token-level GEMMs (M >= 2*128*148) always qualify.
-static int pair_min_m() {
-  static int v = -1;
-  if (v < 0) { const char* e = getenv("NNR_TC_PAIR_MIN_M"); v = e ? atoi(e) : 2 * TC_BM * 148; }
-  return v;
-}
-static int pair_min_tiles() {
-  static int v = -1;
-  if (v < 0) { const char* e = getenv("NNR_TC_PAIR_MIN_TILES"); v = e ? atoi(e) : 48; }
-  return v;
-}
 static int pick_block_n_pair(int N, int step, int nplanes) {
   int best = 0;
   double best_cost = 1e30;
@@ -1096,25 +1058,20 @@ static TcPlan make_plan(const nnr_gemm_args* a, int mode) {
   pl.block_n = pick_block_n(a->N, pl.b_mn ? pl.kelem : 16, pl.nplanes);
   // large row counts (token-level GEMMs) are bound by L2->SM operand delivery: use 256-row tiles on CTA pairs
   pl.pair = 0;
-  if (pair_mode() && a->M >= pair_min_m() && !(a->transA) && a->k_dev == nullptr) {
+  if (a->M >= 2 * TC_BM * 148 && !(a->transA) && a->k_dev == nullptr) {
     int bnp = pick_block_n_pair(a->N, pl.b_mn ? 2 * pl.kelem : 16, pl.nplanes);
-    if (bnp && a->M < 2 * TC_BM * 148) {   // mid-size problem: only when the pair grid still fills the machine
-      long ptiles = (long)((a->M + 2 * TC_BM - 1) / (2 * TC_BM)) * ((a->N + bnp - 1) / bnp);
-      if (ptiles < pair_min_tiles()) bnp = 0;
-    }
     if (bnp) { pl.pair = 1; pl.block_n = bnp; }
   }
   long tiles = (long)((a->M + TC_BM - 1) / TC_BM) * ((a->N + pl.block_n - 1) / pl.block_n);
   // split-K: (a) fill the machine when the output grid is small, (b) bound the TMEM accumulation chain
   int nkb_cap = (a->K + pl.kelem - 1) / pl.kelem;
   pl.split_k = 0;
-  const int chain_k = chain_k_limit();
-  pl.chain_kb = chain_k / pl.kelem;
+  pl.chain_kb = TC_CHAIN_K / pl.kelem;
   if (!pl.pair && tiles * 2 <= 148 && nkb_cap >= 8) {   // an output grid that already fills more than half the SMs is not split
     int target = (int)((148 + tiles - 1) / tiles);
     int chain = (nkb_cap + target - 1) / target;
     if (chain < 4) chain = 4;
-    if (chain > chain_k / pl.kelem) chain = chain_k / pl.kelem;
+    if (chain > TC_CHAIN_K / pl.kelem) chain = TC_CHAIN_K / pl.kelem;
     if (chain < nkb_cap) { pl.split_k = 1; pl.chain_kb = chain; }
   }
   pl.max_splits = pl.split_k ? (nkb_cap + pl.chain_kb - 1) / pl.chain_kb : 1;
@@ -1137,9 +1094,6 @@ static TcPlan make_plan(const nnr_gemm_args* a, int mode) {
 }
 
 int nnr_gemm_tc_supported(const nnr_gemm_args* a) {
-  static int disabled = -1;
-  if (disabled < 0) { const char* e = getenv("NNR_DISABLE_TC"); disabled = (e && e[0] == '1') ? 1 : 0; }
-  if (disabled) return 0;
   if (!get_encode()) return 0;
   // tiny problems are launch-bound either way; the FFMA kernel handles them exactly
   // (an operand that exists only as planes cannot go there, so it stays on this path whatever the size)
@@ -1252,7 +1206,7 @@ static int run_tc(const nnr_gemm_args* a, cudaStream_t st) {
   {
     auto ok = [](const void* ptr, int64_t ld) { return !ptr || (nnr_aligned16(ptr) && ld % 4 == 0); };
     p.epi_fast = (a->N % 4 == 0) && ok(a->C, a->ldc) && ok(a->aux, a->ldaux) && ok(a->aux_out, a->ldaux_out) &&
-                 ok(a->rowbias, a->ldrowbias) && ok(a->bias, 4) && fast_epilogue_enabled();
+                 ok(a->rowbias, a->ldrowbias) && ok(a->bias, 4);
     if (a->epilogue == NNR_EPI_GATE && !(a->rowbias && a->rowmap && a->aux)) p.epi_fast = 0;
     if (a->epilogue == NNR_EPI_ADD_AUX && !a->aux) p.epi_fast = 0;
     const double lim = 4294967296.0;            // 32-bit element offsets inside the kernel
@@ -1281,7 +1235,7 @@ static int run_tc(const nnr_gemm_args* a, cudaStream_t st) {
   // kernels keep the run-time-switched epilogue)
   int epk = (BF16 && p.epi_fast && !pl.split_k) ? a->epilogue : -1;
   // split-K partials: plain 16-byte stores into the [split][M][N] slices (offsets in 32 bits)
-  if (BF16 && pl.split_k && fast_epilogue_enabled() && a->N % 4 == 0 && nnr_aligned16(p.partial) &&
+  if (BF16 && pl.split_k && a->N % 4 == 0 && nnr_aligned16(p.partial) &&
       (double)pl.max_splits * (double)a->M * (double)a->N < 4294967296.0)
     epk = TC_EPK_PARTIAL;
   const void* kernel = tc_kernel_ptr<BF16>(pl.pair != 0, epk);

@@ -186,13 +186,6 @@ __device__ __forceinline__ void bar_arrive(int id, int n) { asm volatile("bar.ar
 __device__ __forceinline__ void cp_async16(uint32_t dst_smem, const void* src) {
   asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"(dst_smem), "l"(src) : "memory");
 }
-// Optional L2 prefetch of the recurrent-step operands NNR_LSTM_PFD steps ahead (compile-time, 0 = off = default).  Measured in
-// round 2 with distance 3: no gain (4.71 -> 4.82 ms forward, 6.47 -> 6.51 ms BPTT at N = 3520, L = 128) -- a step is bound by
-// its own dependency chain (exchange wait -> ldmatrix/MMA -> cell -> exchange), not by the latency of the gx / stash loads.
-#ifndef NNR_LSTM_PFD
-#define NNR_LSTM_PFD 0
-#endif
-__device__ __forceinline__ void prefetch_l2(const void* p) { asm volatile("prefetch.global.L2 [%0];" ::"l"(p)); }
 __device__ __forceinline__ void cp_async_commit() { asm volatile("cp.async.commit_group;" ::: "memory"); }
 __device__ __forceinline__ void cp_async_wait_all() { asm volatile("cp.async.wait_group 0;" ::: "memory"); }
 __device__ __forceinline__ void fence_proxy_async_smem() { asm volatile("fence.proxy.async.shared::cta;" ::: "memory"); }
@@ -294,7 +287,6 @@ lstm_fwd_mma_kernel(float* __restrict__ gx, const float* __restrict__ w_hh, cons
   const bool copy_role = w >= 4;                                 // warps 4-7 move the staging tile to / from global memory
   const int c_ch = tid & 15, c_rs = (tid - G::CT) >> 4;          // cooperative copy: chunk and row slot of a copy thread
   const uint32_t c_so = (uint32_t)(c_rs * G::SROW + c_ch * 16);  // its offset inside an array of the staging tile
-  const bool pf_lane = (c_ch == 0 || c_ch == 4 || c_ch == 8 || c_ch == 9);   // copy threads that issue the L2 prefetches
   const uint32_t b_off = (uint32_t)((w * 40 + (lane >> 4) * 8 + (lane & 7)) * PITCH + ((lane >> 3) & 1) * 16);
   const uint32_t b_off4 = (uint32_t)((w * 40 + 32 + (lane & 7)) * PITCH + ((lane >> 3) & 1) * 16);
   // where this lane's h values go inside this CTA's block of an h tile (plane 0; plane 1 is F_HPLANE further)
@@ -369,11 +361,6 @@ lstm_fwd_mma_kernel(float* __restrict__ gx, const float* __restrict__ w_hh, cons
                 const float* g1 = dir ? g0 - GS : g0 + GS;
 #pragma unroll
                 for (int a = 0; a < 4; ++a) cp_async16(stg_local + c_so + rr * 8 * G::SROW + a * G::SARR, g1 + a * HID);
-              }
-              if (NNR_LSTM_PFD > 0 && pf_lane && s + NNR_LSTM_PFD < rl) {   // 160 B segment: chunks 0, 4, 8, 9 touch every line of it
-                const float* g3 = dir ? g0 - (size_t)NNR_LSTM_PFD * GS : g0 + (size_t)NNR_LSTM_PFD * GS;
-#pragma unroll
-                for (int a = 0; a < 4; ++a) prefetch_l2(g3 + a * HID);
               }
             }
           }
@@ -650,7 +637,6 @@ lstm_fwd_tm_kernel(float* __restrict__ gx, const float* __restrict__ w_hh, const
   const int c_ch = tid & 15, c_rs = (tid - G2::CT) >> 4;          // cooperative copy: chunk and row slot of a copy thread
   const bool ch_ok = c_ch < 10 && rank * UPC + c_ch * 4 < H;     // the chunk's 4 units are all real or all ghost (H % 4 == 0)
   const uint32_t c_so = (uint32_t)(c_rs * G2::SROW + c_ch * 16);  // its offset inside an array of the staging tile
-  const bool pf_lane = (c_ch == 0 || c_ch == 4 || c_ch == 8 || c_ch == 9);   // copy threads that issue the L2 prefetches
   // where this lane's h values go inside this CTA's block of an h tile (plane 0; plane 1 is F_HPLANE further)
   const uint32_t stage_v4 = (uint32_t)(rank * G2::F_HBLK + R * G2::F_HROW + w * 16);
   const uint32_t stage_b32 = (uint32_t)(rank * G2::F_HBLK + R * G2::F_HROW + 64 + w * 4);
@@ -737,11 +723,6 @@ lstm_fwd_tm_kernel(float* __restrict__ gx, const float* __restrict__ w_hh, const
                 const float* g1 = dir ? g0 - GS : g0 + GS;
 #pragma unroll
                 for (int a = 0; a < 4; ++a) cp_async16(stg_local + c_so + rr * 4 * G2::SROW + a * G2::SARR, g1 + a * H);
-              }
-              if (NNR_LSTM_PFD > 0 && pf_lane && s + NNR_LSTM_PFD < rl) {   // 160 B segment: chunks 0, 4, 8, 9 touch every line of it
-                const float* g3 = dir ? g0 - (size_t)NNR_LSTM_PFD * GS : g0 + (size_t)NNR_LSTM_PFD * GS;
-#pragma unroll
-                for (int a = 0; a < 4; ++a) prefetch_l2(g3 + a * H);
               }
             }
           }
@@ -1085,7 +1066,6 @@ lstm_bwd_mma_kernel(float* __restrict__ gates, const float* __restrict__ c_stash
   const int c_ch = tid & 15, c_rs = (tid - G::CT) >> 4;
   const uint32_t c_so = (uint32_t)(c_rs * G::SROW + c_ch * 16);
   const bool ch_ok = c_ch < 10 && rank * UPC + c_ch * 4 < H;     // the chunk's 4 units are all real or all ghost (H % 4 == 0)
-  const bool pf_lane = (c_ch == 0 || c_ch == 4 || c_ch == 8 || c_ch == 9);   // copy threads that issue the L2 prefetches
   const bool leader = (tid == 96);                               // barrier / copy-engine duties (a warp with the fewest n-tiles)
 
   for (;;) {
@@ -1127,15 +1107,6 @@ lstm_bwd_mma_kernel(float* __restrict__ gates, const float* __restrict__ c_stash
 #pragma unroll
               for (int a = 0; a < 4; ++a) cp_async16(stg_local + c_so + rr * RSLOT * G::SROW + a * G::SARR, g1 + a * H);
               cp_async16(stg_local + c_so + rr * RSLOT * G::SROW + 4 * G::SARR, dh + p * 2 * H + (size_t)dir * H + rank * UPC + c_ch * 4);
-            }
-            const int s3 = s1 - NNR_LSTM_PFD;                  // the iteration NNR_LSTM_PFD steps ahead: pull its lines into L2
-            if (NNR_LSTM_PFD > 0 && pf_lane && s3 >= 0 && s3 < c_len[rr]) {
-              const int t3 = dir ? (c_len[rr] - 1 - s3) : s3;
-              const size_t p3 = (size_t)c_off[rr] + t3;
-              const float* g3 = gates + p3 * GS + (size_t)dir * 4 * H + rank * UPC + c_ch * 4;
-#pragma unroll
-              for (int a = 0; a < 4; ++a) prefetch_l2(g3 + a * H);
-              prefetch_l2(dh + p3 * 2 * H + (size_t)dir * H + rank * UPC + c_ch * 4);
             }
           }
         }
@@ -1498,7 +1469,7 @@ lstm_bwd_mma_kernel(float* __restrict__ gates, const float* __restrict__ c_stash
 
 template <int CL, class K>
 int launch_cluster(K kernel, size_t smem, int ntiles, cudaStream_t st, void** args, const char* name, int (*cache_tab)[16],
-                   bool (*attr_tab)[16], int variant, int nthreads = G<CL>::NT, bool bwd = false) {
+                   bool (*attr_tab)[16], int variant, int nthreads = G<CL>::NT) {
   int dev = 0;
   NNR_CUDA(cudaGetDevice(&dev));
   dev &= 15;                                  // the attribute and the occupancy are per device (and per instantiation)
@@ -1529,7 +1500,6 @@ int launch_cluster(K kernel, size_t smem, int ntiles, cudaStream_t st, void** ar
     // 58: 3.32, 64: 3.45, 72: 3.40 -> 2 nc + 6.  Clusters beyond what fits start late, find the tile counter exhausted and exit.
     // The rule was measured at CL = 5 (hidden_dim 200); the smaller clusters of other hidden sizes use it unchanged.
     if (nthreads == G2<CL>::NT) *cache = (2 * nc + 6) & ~1;
-    if (const char* ev = getenv(bwd ? "NNR_LSTM_BWD_CLUSTERS" : "NNR_LSTM_FWD_CLUSTERS")) { int v = atoi(ev); if (v >= 2 && nthreads == G2<CL>::NT) *cache = v & ~1; }
     if (getenv("NNR_LSTM_DEBUG")) {
       int bps = -1;
       cudaOccupancyMaxActiveBlocksPerMultiprocessor(&bps, (const void*)kernel, nthreads, smem);
@@ -1679,9 +1649,9 @@ __global__ void lstm_dz_finish_kernel(const float* __restrict__ db_partial, int 
 template <int CL, int HC>
 static int lstm_bwd_tm_launch(void** args, int ntiles, cudaStream_t st, int single, int (*cache)[16], bool (*attr_set)[16]) {
   return single ? launch_cluster<CL>(lstm_bwd_mma_kernel<true, true, CL, HC>, G3<CL>::BWD_SMEM, ntiles, st, args, "lstm_bwd_tm_kernel<single>", cache, attr_set, 3,
-                                     G3<CL>::NT, true)
+                                     G3<CL>::NT)
                 : launch_cluster<CL>(lstm_bwd_mma_kernel<false, true, CL, HC>, G3<CL>::BWD_SMEM, ntiles, st, args, "lstm_bwd_tm_kernel", cache, attr_set, 2,
-                                     G3<CL>::NT, true);
+                                     G3<CL>::NT);
 }
 
 // 0 < H <= 200 and H % 4 == 0 with the tensor-memory variant; the shared-memory variant and dz_planes need H = 200 (lstm.cu checks)

@@ -4,7 +4,6 @@
 // Replaces: MIND_corpus.py:162-216 (numpy preprocessing), torch.bmm(graph, feature) at layers.py:286,
 // and torch_scatter.scatter_softmax / scatter_sum at userEncoders.py:88-89.
 #include "common.cuh"
-#include <stdlib.h>
 #include "../../include/nnr_b200.h"
 
 // ------------------------------------------------------------------------------------------------
@@ -205,9 +204,7 @@ static int gcn_aggregate_launch(const int32_t* nnz, const int32_t* col, const fl
                                 const float* add, float* out, void* stream, const char* who) {
   NNR_REQUIRE(nnz && col && val && x && out && B > 0 && G > 0 && D > 0, NNR_ERR_ARG, "%s: bad arguments", who);
   const size_t smem = (sizeof(int) + sizeof(float)) * G;
-  static int vec_mode = -1;
-  if (vec_mode < 0) { const char* e = getenv("NNR_GCN_VEC"); vec_mode = (e && e[0] == '0') ? 0 : 1; }
-  if (vec_mode && D % 4 == 0 && nnr_aligned16(x) && nnr_aligned16(out) && (!add || nnr_aligned16(add))) {
+  if (D % 4 == 0 && nnr_aligned16(x) && nnr_aligned16(out) && (!add || nnr_aligned16(add))) {
     const int threads = ((D / 4 + 31) / 32 * 32) < 256 ? ((D / 4 + 31) / 32 * 32) : 256;
     gcn_aggregate_vec_kernel<<<B * G, threads, smem, (cudaStream_t)stream>>>(nnz, col, val, x, G, D, add, out);
   } else {

@@ -69,9 +69,6 @@ def _empty(shape, dev, dtype=torch.float32):
 # inside a captured step the two lanes become parallel branches of the CUDA graph.  NNR_LANES=0 (or
 # engine.concurrent = False, used by the per-op profiler) issues everything on the caller's stream in the same order.
 _LANES = os.environ.get('NNR_LANES', '1') != '0'
-_PRODUCER_PLANES = os.environ.get('NNR_PRODUCER_PLANES', '1') != '0'   # A/B switch: h / gated-state planes written by their producers
-_CONTENT_FIRST = os.environ.get('NNR_CONTENT_FIRST', '1') != '0'     # A/B switch: issue order of the two BPTT recurrences
-_FWD_CONTENT_FIRST = os.environ.get('NNR_FWD_CONTENT_FIRST', '1') != '0'   # A/B switch: issue order of the two forward recurrences
 concurrent = True
 _side_streams = {}
 
@@ -90,9 +87,7 @@ class Lanes:
             self.main = torch.cuda.current_stream(idx)
             self.sides = _side_streams.get(idx)
             if self.sides is None:
-                # NNR_SIDE_PRIORITIES (A/B switch): stream priorities of lanes 1, 2 (0 = lowest ... -5); a captured step keeps them
-                prios = [int(v) for v in os.environ.get('NNR_SIDE_PRIORITIES', '0,0').split(',')]
-                self.sides = _side_streams[idx] = [torch.cuda.Stream(device=idx, priority=prios[i]) for i in range(self.NSIDE)]
+                self.sides = _side_streams[idx] = [torch.cuda.Stream(device=idx) for _ in range(self.NSIDE)]
             if any(s == self.main for s in self.sides):      # nested use from a side lane itself: stay serial
                 self.on = False
 
@@ -178,25 +173,15 @@ def _param_grads(P, names, G):
     return tuple(G.get(k) for k in names)
 
 
-_SHARE_SPLITS = os.environ.get('NNR_SHARE_SPLITS', '1') != '0'   # A/B switch: split small operands once per tensor
-
-
 def _shared_split(x, rows, cols, colsum_out=None):
     """operand planes of a small activation that feeds two GEMMs (and, with ``colsum_out``, its column sums = a bias
-    gradient); NNR_SHARE_SPLITS=0 restores one split per GEMM call"""
-    if _SHARE_SPLITS:
-        return ops.tc_split(x, rows, cols, x.stride(0), colsum_out=colsum_out)
-    if colsum_out is not None:
-        ops.colsum(x, x.stride(0), rows, cols, colsum_out, False, None)
-    return None
-
-
-_FUSE_SUE_BWD = os.environ.get('NNR_FUSE_SUE_BWD', '1') != '0'     # A/B switch for the fused relu-backward split
+    gradient)"""
+    return ops.tc_split(x, rows, cols, x.stride(0), colsum_out=colsum_out)
 
 
 def _fused_relu_bwd(dy, cols):
     """nnr_relu_bwd_split_colsum applies: tensor-core GEMM planes in use, contiguous 16-byte aligned rows, <= 2048 columns"""
-    return (_FUSE_SUE_BWD and ops.default_algo() != ops.ALGO_SIMT and cols <= 2048 and cols % 4 == 0 and dy.is_contiguous()
+    return (ops.default_algo() != ops.ALGO_SIMT and cols <= 2048 and cols % 4 == 0 and dy.is_contiguous()
             and dy.data_ptr() % 16 == 0)
 
 
@@ -383,7 +368,7 @@ def _cne_recurrent(P, x, m, N, E, Hd, training, p_drop, seed, want_h_planes=Fals
     m.c_stash = _empty((cap, 2 * Hd), dev)
     m.c_n = _empty((N, 2 * Hd), dev)
     m.h_pl = None
-    if want_h_planes and _PRODUCER_PLANES and ops.lstm_fwd_planes_supported(Hd):
+    if want_h_planes and ops.lstm_fwd_planes_supported(Hd):
         # h feeds GEMMs (selective gate, two weight gradients): the recurrence writes its operand planes next to the fp32 states
         m.h_pl = ops.lstm_fwd_planes(m.gates, m.w_hh, m.len, m.off, m.order, N, L, Hd, m.h, m.c_stash, m.c_n, cap)
     else:
@@ -409,7 +394,7 @@ def _cne_gate_self(P, x, m, m_other_cn, partner, N, Hd, A, gate=True):
         if m.h_pl is None:
             m.h_pl = split_tokens(m.h, m.cap, D2, m.ntok)
         # the gated states feed the attention projection and its weight gradient: the epilogue also writes their planes
-        m.hg_pl = ops.planes_empty(m.cap, D2, dev) if (_PRODUCER_PLANES and D2 % 8 == 0) else None
+        m.hg_pl = ops.planes_empty(m.cap, D2, dev) if D2 % 8 == 0 else None
         m.hg = linear(m.h, P[x + '_H.weight'], m.cap, m.ntok, None, EPI_GATE, rowbias=m.mproj, ldrowbias=D2,
                       rowmap=m.tok_row, aux=m.h, ldaux=D2, aux_out=m.g, ldaux_out=D2, x_planes=m.h_pl, c_planes=m.hg_pl)
     else:
@@ -475,9 +460,8 @@ class CNEFunction(torch.autograd.Function):
         t, c = lanes.run(lambda: _cne_prepare(title_text.view(N, T), title_mask.reshape(N, T), N, T, domains),
                          lambda: _cne_prepare(content_text.view(N, Lc), content_mask.reshape(N, Lc), N, Lc, domains))
         lanes.fork()
-        if _FWD_CONTENT_FIRST:
-            # the content branch (gather, input projection, 128-step recurrence) is the critical path of the forward stage
-            _cne_recurrent(P, 'content', c, N, E, Hd, training, p, seeds[1], True)
+        # the content branch (gather, input projection, 128-step recurrence) is the critical path of the forward stage
+        _cne_recurrent(P, 'content', c, N, E, Hd, training, p, seeds[1], True)
         lanes.on_side(_cne_recurrent, P, 'title', t, N, E, Hd, training, p, seeds[0], True)
         # pairing by sort rank inside each domain (newsEncoders.py:124-129, SURVEY finding 2): title row r of a call is
         # gated with the content memory of the news at the same sorted rank.  (A handful of [N]-sized kernels: issued here
@@ -485,8 +469,6 @@ class CNEFunction(torch.autograd.Function):
         partner_t = torch.cat([cs.index_select(0, td) for cs, td in zip(c.sorted_idx, t.desorted_idx)])
         partner_c = torch.cat([ts.index_select(0, cd) for ts, cd in zip(t.sorted_idx, c.desorted_idx)])
         t.partner, c.partner = partner_t, partner_c
-        if not _FWD_CONTENT_FIRST:
-            _cne_recurrent(P, 'content', c, N, E, Hd, training, p, seeds[1], True)
         lanes.join()
         lanes.run(lambda: _cne_gate_self(P, 'title', t, c.c_n, partner_t, N, Hd, A, gate),
                   lambda: _cne_gate_self(P, 'content', c, t.c_n, partner_c, N, Hd, A, gate))
@@ -685,23 +667,17 @@ class CNEFunction(torch.autograd.Function):
         else:
             # lane 1: title recurrence, title scatter, content scatter (the chain the end of the backward pass waits for);
             # lane 2: the title branch's weight gradients; caller's stream: content recurrence, content weight gradients
-            # (the content recurrence is issued first: its longest sequences are the critical path of this stage, the title
-            # recurrence fills the SMs its short tiles leave idle)
             lanes.fork()
-            thp = None
-            if _CONTENT_FIRST:
-                # the content recurrence must get the SMs first -- its longest sequences are the critical path of this stage
-                # and the title recurrence fits into the SMs its short tiles leave idle: the title lane starts with a kernel
-                # it needs anyway (h_{t-1} planes), so its recurrence is launched a few microseconds after the content one
-                planes = t.emb is None and ops.lstm_bwd_planes_supported(Hd)
-                thp = lanes.on_side(shifted_h, t, planes)
-                dz, dz_pl, db, demb = recurrence_bwd('content', c, dcn['content'])
+            # the content recurrence must get the SMs first -- its longest sequences are the critical path of this stage
+            # and the title recurrence fits into the SMs its short tiles leave idle: the title lane starts with a kernel
+            # it needs anyway (h_{t-1} planes), so its recurrence is launched a few microseconds after the content one
+            planes = t.emb is None and ops.lstm_bwd_planes_supported(Hd)
+            thp = lanes.on_side(shifted_h, t, planes)
+            dz, dz_pl, db, demb = recurrence_bwd('content', c, dcn['content'])
             tz, tz_pl, tdb, tdemb = lanes.on_side(recurrence_bwd, 'title', t, dcn['title'])
             lanes.on_side(scatter, 'title', t, tdemb)
             lanes.fork(2, after=1)
             lanes.on_side(weight_grads, 'title', t, tz, tz_pl, tdb, thp, lane=2)
-            if not _CONTENT_FIRST:
-                dz, dz_pl, db, demb = recurrence_bwd('content', c, dcn['content'])
             lanes.keep.extend((tz, tz_pl, tdemb, dz, dz_pl, demb, thp))
             lanes.fork()                                       # lane 1, behind the title scatter
             lanes.on_side(scatter, 'content', c, demb)

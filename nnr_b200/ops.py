@@ -594,11 +594,10 @@ def _via_dispatcher(name):
 
 
 # The engine reaches these ops through PyTorch's dispatcher (torch.ops.nnr.*): module attributes are rebound to dispatcher
-# calls, the registered CUDA implementations are the ctypes wrappers above.  NNR_TORCH_OPS=0 calls the wrappers directly.
+# calls, the registered CUDA implementations are the ctypes wrappers above.
 # Ops whose arguments are argument STRUCTS of the C ABI (nnr_gemm, nnr_attn_pool_*) or that return operand-plane handles
 # (tc_split*, *_planes*) are plain functions: a dispatcher schema cannot carry them.
-import os as _os
-DISPATCHED = sorted(_SCHEMAS) if _os.environ.get('NNR_TORCH_OPS', '1') != '0' else []
+DISPATCHED = sorted(_SCHEMAS)
 for _name in DISPATCHED:
     globals()[_name] = _via_dispatcher(_name)
 

@@ -23,7 +23,7 @@ _KERNEL_TAGS = ['gemm_tc_kernel', 'tc_split_kernel', 'tc_splitk_reduce_kernel', 
 
 def _tc_class(M, N, K, transA, transB, m_dev, k_dev):
     """mirror of nnr_gemm_tc_supported (gemm_tc.cu): which nnr_gemm calls run on the tcgen05 kernel"""
-    if os.environ.get('NNR_GEMM_ALGO') == 'simt' or os.environ.get('NNR_DISABLE_TC') == '1':
+    if os.environ.get('NNR_GEMM_ALGO') == 'simt':
         return False
     if float(M) * N * K < 2.0e6 or K < 8:
         return False

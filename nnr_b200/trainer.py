@@ -9,7 +9,6 @@ one process per GPU and exactly one ``ncclAllReduce`` over the flat gradient buf
 (the reference's DDP issues bucketed all-reduces, trainer.py:219,297); the 1/world averaging is
 folded into the fused clip+Adam kernel (``nnr_flat_clip_adam``).
 """
-import os
 import torch
 import torch.distributed as dist
 
@@ -117,8 +116,7 @@ class TrainStep:
         for i in range(1, 4):
             bounds[i] = max(bounds[i], bounds[i - 1])
         self.stage_bounds = {'sue': (bounds[0], bounds[1]), 'cne': (bounds[1], bounds[2]), 'table': (bounds[2], bounds[3])}
-        import os
-        self.overlap = os.environ.get('NNR_DP_OVERLAP', '1') != '0'   # reduce each group as soon as it is final, on a side stream (world_size > 1)
+        self.overlap = True          # reduce each group as soon as it is final, on a side stream (world_size > 1)
         self._comm_stream = None
         self._reduced = set()
         self.params = params
@@ -223,10 +221,8 @@ class TrainStep:
             n0 = ops.launch_count()
             # lane 0 (the critical path: content branch, user encoder, optimizer) is captured on a stream above the side lanes'
             # priority; the kernel nodes inherit it, so the block scheduler serves lane 0 first whenever two lanes have CTAs
-            # waiting (7.44 -> 7.28 ms per step; NNR_CAPTURE_PRIORITY=0 is the A/B switch)
-            prio = int(os.environ.get('NNR_CAPTURE_PRIORITY', '-1'))
-            cap_kw = {'stream': torch.cuda.Stream(priority=prio)} if prio else {}
-            with torch.cuda.graph(graph, **cap_kw):
+            # waiting (7.44 -> 7.28 ms per step)
+            with torch.cuda.graph(graph, stream=torch.cuda.Stream(priority=-1)):
                 self.seeds.advance()
                 loss = self._eager_step(*static)
             self.launches_per_graph[layout_key] = ops.launch_count() - n0

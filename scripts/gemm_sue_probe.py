@@ -1,7 +1,7 @@
 """The per-news / SUE-sized GEMMs (a few thousand rows) in isolation: CUDA-event time per call at three contraction lengths,
 from which the fixed cost of a launch (prologue + the last tile's epilogue) and the cost per 64-deep k-block separate.
 
-    python scripts/gemm_sue_probe.py [reps]          (NNR_TC_PAIR_MIN_M=1024 puts these shapes on CTA pairs)
+    python scripts/gemm_sue_probe.py [reps]
 """
 import os
 import sys
