@@ -508,8 +508,6 @@ static int launch_cluster(K kernel, size_t smem, int ntiles, cudaStream_t st, vo
 int nnr_lstm_fwd_mma(float* gx, const float* w_hh, const int32_t* len, const int32_t* off, const int32_t* order, int N, int H,
                      float* h_out, float* c_stash, float* c_n, int32_t* tile_counters, cudaStream_t st, void* h_planes,
                      size_t plane_stride, int two_planes, int cap);
-int nnr_lstm_fwd_planes_ok(void);
-int nnr_lstm_bwd_tm_ok(void);
 int nnr_lstm_bwd_mma(float* gates, const float* c_stash, const float* w_hh, const int32_t* len, const int32_t* off,
                      const int32_t* order, int N, int H, const float* dh, const float* dcn, int32_t* tile_counters, cudaStream_t st,
                      void* dz_planes, size_t plane_stride, int two_planes, float* db_partial, float* db, int cap);
@@ -522,16 +520,14 @@ static bool lstm_use_mma() {
   return v == 1;
 }
 
-// The hidden sizes a recurrence entry point accepts, checked before any CUDA call.  The tensor-core kernels with the W slice in
-// tensor memory (the default) take 0 < H <= 200, H % 4 == 0 (clusters of 2..5 CTAs of 40 units, 16 B chunks of 4 units); the
-// exact-fp32 FFMA kernels and the shared-memory W variants are instantiated for hidden_dim 200 only.
-static int lstm_check_hidden(const char* fn, int H, bool tm) {
+// The hidden sizes a recurrence entry point accepts, checked before any CUDA call.  The tensor-core kernels (the default) take
+// 0 < H <= 200, H % 4 == 0 (clusters of 2..5 CTAs of 40 units, 16 B chunks of 4 units); the exact-fp32 FFMA kernels are
+// instantiated for hidden_dim 200 only.
+static int lstm_check_hidden(const char* fn, int H) {
   NNR_REQUIRE(H > 0 && H <= 200 && H % 4 == 0, NNR_ERR_UNSUPPORTED,
               "%s: hidden_dim %d: the tensor-core recurrence takes H %% 4 == 0 and H <= 200", fn, H);
   NNR_REQUIRE(H == 200 || lstm_use_mma(), NNR_ERR_UNSUPPORTED,
               "%s: hidden_dim %d: the exact-fp32 FFMA recurrence (NNR_LSTM_ALGO=ffma) takes hidden_dim 200 only", fn, H);
-  NNR_REQUIRE(H == 200 || tm, NNR_ERR_UNSUPPORTED, "%s: hidden_dim %d: the shared-memory W variant (%s=0) takes hidden_dim 200 only", fn, H,
-              !strcmp(fn, "nnr_lstm_fwd") ? "NNR_LSTM_FWD_TM" : "NNR_LSTM_BWD_TM");
   return 0;
 }
 
@@ -540,7 +536,7 @@ extern "C" int nnr_lstm_fwd(float* gx, const float* w_hh, const int32_t* len, co
                             void* stream) {
   NNR_REQUIRE(gx && w_hh && len && off && order && h_out && c_stash && c_n && tile_counters && N > 0 && L > 0, NNR_ERR_ARG,
               "nnr_lstm_fwd: bad arguments");
-  if (int rc = lstm_check_hidden("nnr_lstm_fwd", H, nnr_lstm_fwd_planes_ok())) return rc;
+  if (int rc = lstm_check_hidden("nnr_lstm_fwd", H)) return rc;
   NNR_REQUIRE(nnr_aligned16(gx) && nnr_aligned16(h_out) && nnr_aligned16(c_stash) && nnr_aligned16(c_n), NNR_ERR_ALIGN,
               "nnr_lstm_fwd: buffers must be 16B aligned");
   if (lstm_use_mma()) return nnr_lstm_fwd_mma(gx, w_hh, len, off, order, N, H, h_out, c_stash, c_n, tile_counters, (cudaStream_t)stream, NULL, 0, 0, 0);
@@ -556,7 +552,7 @@ extern "C" int nnr_lstm_bwd(float* gates, const float* c_stash, const float* w_h
                             int32_t* tile_counters, void* stream) {
   NNR_REQUIRE(gates && c_stash && w_hh && len && off && order && dh && dcn && tile_counters && N > 0 && L > 0, NNR_ERR_ARG,
               "nnr_lstm_bwd: bad arguments");
-  if (int rc = lstm_check_hidden("nnr_lstm_bwd", H, nnr_lstm_bwd_tm_ok())) return rc;
+  if (int rc = lstm_check_hidden("nnr_lstm_bwd", H)) return rc;
   NNR_REQUIRE(nnr_aligned16(gates) && nnr_aligned16(c_stash) && nnr_aligned16(dh) && nnr_aligned16(dcn), NNR_ERR_ALIGN,
               "nnr_lstm_bwd: buffers must be 16B aligned");
   if (lstm_use_mma())
@@ -573,7 +569,7 @@ extern "C" int nnr_lstm_bwd(float* gates, const float* c_stash, const float* w_h
 // nnr_tc_split(h, cap, 2H, ntok) would write them, rows [ntok, round_up(ntok, 64)) zeroed.
 extern "C" int nnr_lstm_fwd_planes_supported(int H, int algo) {
   if (algo == NNR_GEMM_AUTO) algo = nnr_gemm_default_algo();
-  return H == 200 && lstm_use_mma() && nnr_lstm_fwd_planes_ok() && (algo == NNR_GEMM_TC_BF16 || algo == NNR_GEMM_TC_BF16X3);
+  return H == 200 && lstm_use_mma() && (algo == NNR_GEMM_TC_BF16 || algo == NNR_GEMM_TC_BF16X3);
 }
 extern "C" int nnr_lstm_fwd_planes(float* gx, const float* w_hh, const int32_t* len, const int32_t* off, const int32_t* order,
                                    int N, int L, int H, float* h_out, float* c_stash, float* c_n, int32_t* tile_counters, int cap,
@@ -582,7 +578,7 @@ extern "C" int nnr_lstm_fwd_planes(float* gx, const float* w_hh, const int32_t* 
               NNR_ERR_ARG, "nnr_lstm_fwd_planes: bad arguments");
   if (algo == NNR_GEMM_AUTO) algo = nnr_gemm_default_algo();
   NNR_REQUIRE(nnr_lstm_fwd_planes_supported(H, algo), NNR_ERR_UNSUPPORTED,
-              "nnr_lstm_fwd_planes: needs H = 200, the tensor-memory forward kernel and a bf16 GEMM algorithm");
+              "nnr_lstm_fwd_planes: needs H = 200, the tensor-core recurrence and a bf16 GEMM algorithm");
   NNR_REQUIRE(nnr_aligned16(gx) && nnr_aligned16(h_out) && nnr_aligned16(c_stash) && nnr_aligned16(c_n) && nnr_aligned16(planes),
               NNR_ERR_ALIGN, "nnr_lstm_fwd_planes: buffers must be 16B aligned");
   const int two = algo == NNR_GEMM_TC_BF16X3;

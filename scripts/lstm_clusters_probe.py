@@ -1,4 +1,4 @@
-import sys, os
+import sys
 sys.path.insert(0, '/root/repo')
 import ctypes, torch
 from nnr_b200 import ops
@@ -12,4 +12,4 @@ w_hh = torch.randn(2, 4 * Hd, Hd, device=dev) * 0.05
 h = torch.empty(N * L, 2 * Hd, device=dev); cst = torch.empty(N * L, 2 * Hd, device=dev); cn = torch.empty(N, 2 * Hd, device=dev)
 ops.lstm_fwd(gx, w_hh, lens, off, order, N, L, Hd, h, cst, cn); torch.cuda.synchronize()
 lib.nnr_debug_lstm_clusters.restype = ctypes.c_int
-print('max active clusters:', lib.nnr_debug_lstm_clusters(), 'env TM =', os.environ.get('NNR_LSTM_FWD_TM'))
+print('max active clusters:', lib.nnr_debug_lstm_clusters())

@@ -5,7 +5,7 @@
     compute-sanitizer --tool synccheck python scripts/sanitize_targets.py gemm
     compute-sanitizer --tool memcheck  python scripts/sanitize_targets.py embed
 
-targets: lstm (lstm_fwd_mma_kernel / lstm_bwd_mma_kernel, 5-CTA clusters, bulk-copy exchange), gemm (gemm_tc_kernel<1,0> and the
+targets: lstm (lstm_fwd_tm_kernel / lstm_bwd_mma_kernel, 5-CTA clusters, bulk-copy exchange), gemm (gemm_tc_kernel<1,0> and the
 CTA-pair gemm_tc_kernel<1,1>, TMA + tcgen05 + mbarriers), embed (eb_keys / radix sort / eb_chunk / eb_fix scatter)."""
 import os
 import sys

@@ -7,8 +7,7 @@ import re
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 PACKAGE = os.path.join(ROOT, 'nnr_b200')
 
-SUPPORTED = {'NNR_GEMM_ALGO', 'NNR_LSTM_ALGO', 'NNR_LSTM_FWD_TM', 'NNR_LSTM_BWD_TM', 'NNR_LANES', 'NNR_LSTM_DEBUG',
-             'NNR_B200_LIB'}
+SUPPORTED = {'NNR_GEMM_ALGO', 'NNR_LSTM_ALGO', 'NNR_LANES', 'NNR_LSTM_DEBUG', 'NNR_B200_LIB'}
 
 # getenv("X") in C / CUDA, os.environ.get('X'), os.environ['X'] and os.getenv('X') in Python
 _READ = re.compile(r'''(?:getenv\s*\(|environ\s*\.\s*get\s*\(|environ\s*\[)\s*["']([A-Za-z0-9_]+)["']''')
@@ -24,7 +23,7 @@ def _sources():
                     yield os.path.relpath(path, ROOT), fh.read()
 
 
-def test_library_reads_only_the_supported_switches():
+def test_library_reads_exactly_the_supported_switches():
     read = {}
     for rel, text in _sources():
         for name in _READ.findall(text):
@@ -38,7 +37,7 @@ def test_no_compile_time_prefetch_switch():
         assert 'NNR_LSTM_PFD' not in text, rel
 
 
-def test_readme_lists_exactly_the_supported_switches():
+def test_readme_names_exactly_the_supported_switches():
     with open(os.path.join(ROOT, 'README.md'), encoding='utf-8') as fh:
         readme = fh.read()
     m = re.search(r'^Environment switches:.*?(?=\n\s*\n)', readme, re.S | re.M)
