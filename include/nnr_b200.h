@@ -33,7 +33,7 @@
 extern "C" {
 #endif
 
-#define NNR_ABI_VERSION 8
+#define NNR_ABI_VERSION 9
 #define NNR_SEED_INDIRECT (1ULL << 62)
 
 const char* nnr_last_error(void);
@@ -323,6 +323,22 @@ int nnr_cluster_intra_bwd(const float* dintra, const float* Kp, const float* Qp,
                           const int64_t* idx, const float* alpha, int B, int n, int H, int Au,
                           int D, int C1, float scale, float* da_ws /* [B,n,H] scratch */,
                           float* dKp, float* dQp, float* dg, int accumulate_dg, void* stream);
+/* Factored cluster tail for top-k recommendation: click scores of T pool candidates, shared by the B users, without the
+ * per-(user, candidate) cluster features.  The weights of a non-empty cluster's softmax sum to 1 and an empty cluster's
+ * feature is 0, so the cluster affine commutes with the weighted sum (W intra_c + b = sum_{h in c} alpha_h Wg_h + b):
+ *   Kp [B,H,Au] (intra-cluster keys), g [B,H,D], Wg [B,H,D] = g W^T (clusterFeatureAffine.weight, no bias), idx [B,H]
+ *   int64 (clamped to [0,C1)), cmask [B,C1] uint8, Qp [T,Au], qk2 [T,D], cand [T,D] (one row per candidate), bias [D]
+ *   alpha[b,t,h] = segment_softmax_h(scale * Kp[b,h].Qp[t] ; idx[b,h])   (every slot takes part, max-shifted)
+ *   f[b,t,c,:]   = relu(sum_{h: idx=c} alpha Wg[b,h] + bias) + sum_{h: idx=c} alpha g[b,h]   (empty cluster: relu(bias))
+ *   beta[b,t,c]  = softmax_c(cmask[b,c] ? scale * f.qk2[t] : -1e9)
+ *   scores[b*lds + t] = sum_c beta * (f . cand[t])
+ * = cluster_intra_fwd + the EPI_BIAS_RELU_RES affine + attn_pool mode 1 + rowdot in real arithmetic, not bit for bit.
+ * Deterministic (fixed summation order, no atomics), no allocation, no host synchronisation (graph-capturable).
+ * Limits: H <= 256, C1 <= 72, 1 <= T <= NNR_TOPK_MAX_TILE, lds >= T (NNR_ERR_ARG / NNR_ERR_UNSUPPORTED before any CUDA
+ * call otherwise); D % 4 == 0 and 16-byte aligned g, Wg, qk2, cand, bias (NNR_ERR_UNSUPPORTED).                       */
+int nnr_cluster_tail_scores(const float* Kp, const float* g, const float* Wg, const int64_t* idx, const uint8_t* cmask,
+                            const float* Qp, const float* qk2, const float* cand, const float* bias, int B, int H, int Au,
+                            int D, int C1, int T, float scale, float* scores, int64_t lds, void* stream);
 
 /* ---- click predictor: model.py:127 ---------------------------------------------------------- */
 int nnr_rowdot_fwd(const float* a, const float* b, int R, int D, float* out, void* stream);

@@ -1080,10 +1080,11 @@ class RowDot(torch.autograd.Function):
 # pieces on the same shapes, so a tile's scores equal SUEFunction.forward + RowDot on [B, T] candidates bit for bit.
 # Inference only: eval mode (no dropout), no autograd.
 @torch.no_grad()
-def sue_user_side(meta, hist, graph, cmask, cidx, *params):
+def sue_user_side(meta, hist, graph, cmask, cidx, *params, factored=False):
     """the history half of SUEFunction.forward for the users of hist [B, H, D]: returns the tuple of tensors
     ``sue_tile_scores`` takes -- (gfeat, Kp, cmask, cidx) with the hierarchical cluster attention, (pooled user vector,)
-    for SUE_wo_HCA"""
+    for SUE_wo_HCA.  ``factored``: the cluster attention's tuple also carries Wg = gfeat clusterFeatureAffine.weight^T
+    [B, H, D] (no bias), for ``sue_tile_scores_factored``"""
     assert not meta['training'], 'the split SUE forward is for inference (eval mode)'
     P = dict(zip(sue_names(meta), params))
     gcn = meta.get('gcn', True)
@@ -1092,7 +1093,12 @@ def sue_user_side(meta, hist, graph, cmask, cidx, *params):
     gfeat = SUEFunction._gcn(meta, P, hist, graph, [0] * (L + 2), L, 0.0)[0] if gcn else hist
     if not meta['hca']:
         return (SUEFunction._history_pool(P, gfeat)[0],)
-    return gfeat, SUEFunction._user_keys(P, gfeat)[1], cmask, cidx.contiguous()
+    gfeat_pl, Kp = SUEFunction._user_keys(P, gfeat)
+    if not factored:
+        return gfeat, Kp, cmask, cidx.contiguous()
+    B, H, D = gfeat.shape
+    Wg = linear(gfeat.view(B * H, D), P['clusterFeatureAffine.weight'], B * H, x_planes=gfeat_pl)
+    return gfeat, Kp, cmask, cidx.contiguous(), Wg.view(B, H, D)
 
 
 @torch.no_grad()
@@ -1112,3 +1118,25 @@ def sue_tile_scores(meta, side, cand, *params):
     user = SUEFunction._clusters_tail(_Mod(), P, gfeat, cand, cmask, cidx, [0] * (L + 2), (B, H, D, T, C, H + C, C + 1), L, 0.0,
                                       keys=(None, Kp))
     return RowDot.apply(user, cand)
+
+
+@torch.no_grad()
+def sue_tile_scores_factored(meta, side, cand_rows, *params):
+    """click scores [B, T] of the candidates cand_rows [T, D], shared by the users of ``side`` (from
+    ``sue_user_side(..., factored=True)``), through the factored cluster tail (nnr_cluster_tail_scores): the cluster affine
+    is applied to the users' history rows (Wg) instead of to every (user, candidate) cluster feature.  The scores are those
+    of SUEFunction.forward + RowDot in real arithmetic, not bit for bit; the candidate projections run once per row, not
+    once per (user, row).  SUE_wo_HCA, whose user vector does not depend on the candidate: ``sue_tile_scores``."""
+    T, D = cand_rows.shape
+    if not meta['hca']:
+        return sue_tile_scores(meta, side, cand_rows.unsqueeze(0).expand(side[0].shape[0], -1, -1), *params)
+    P = dict(zip(sue_names(meta), params))
+    gfeat, Kp, cmask, cidx, Wg = side
+    B, H, _ = gfeat.shape
+    C1 = cmask.shape[1]
+    Au = P['intraCluster_K.weight'].shape[0]
+    _, Qp, _, _, qk2 = SUEFunction._cand_side(P, cand_rows.contiguous(), 1, T, D)
+    scores = _empty((B, T), gfeat.device)
+    ops.cluster_tail_scores(Kp, gfeat, Wg, cidx, cmask.contiguous().view(torch.uint8), Qp, qk2, cand_rows.contiguous(),
+                            P['clusterFeatureAffine.bias'], B, H, Au, D, C1, T, 1.0 / math.sqrt(float(Au)), scores)
+    return scores

@@ -434,6 +434,14 @@ def cluster_intra_bwd(dintra, Kp, Qp, g, idx, alpha, B, n, H, Au, D, C1, scale, 
                                     _p(dQp, _F32), _p(dg, _F32), int(accumulate_dg), _stream()), 'nnr_cluster_intra_bwd')
 
 
+def cluster_tail_scores(Kp, g, Wg, idx, cmask, Qp, qk2, cand, bias, B, H, Au, D, C1, T, scale, scores):
+    """click scores [B, T] (row stride scores.stride(0)) of T candidates shared by B users through the factored cluster tail
+    (nnr_cluster_tail_scores)"""
+    check(lib.nnr_cluster_tail_scores(_p(Kp, _F32), _p(g, _F32), _p(Wg, _F32), _p(idx, _I64), _p(cmask, _U8), _p(Qp, _F32),
+                                      _p(qk2, _F32), _p(cand, _F32), _p(bias, _F32), B, H, Au, D, C1, T, float(scale),
+                                      _p(scores, _F32), scores.stride(0), _stream()), 'nnr_cluster_tail_scores')
+
+
 def rowdot_fwd(a, b, R, D, out):
     check(lib.nnr_rowdot_fwd(_p(a, _F32), _p(b, _F32), R, D, _p(out, _F32), _stream()), 'nnr_rowdot_fwd')
 
@@ -536,6 +544,9 @@ _SCHEMAS = {
     'cluster_intra_bwd': ('(Tensor dintra, Tensor Kp, Tensor Qp, Tensor g, Tensor idx, Tensor alpha, int B, int n, int H, int Au, int D, '
                           'int C1, float scale, Tensor(a!) da_ws, Tensor(b!) dKp, Tensor(c!) dQp, Tensor(d!) dg, bool accumulate_dg) -> ()',
                           cluster_intra_bwd),
+    'cluster_tail_scores': ('(Tensor Kp, Tensor g, Tensor Wg, Tensor idx, Tensor cmask, Tensor Qp, Tensor qk2, Tensor cand, '
+                            'Tensor bias, int B, int H, int Au, int D, int C1, int T, float scale, Tensor(a!) scores) -> ()',
+                            cluster_tail_scores),
     'rowdot_fwd': ('(Tensor a, Tensor b, int R, int D, Tensor(a!) out) -> ()', rowdot_fwd),
     'rowdot_bwd': ('(Tensor dout, Tensor a, Tensor b, int R, int D, Tensor(a!) da, bool accumulate_a, Tensor(b!) db, bool accumulate_b) -> ()',
                    rowdot_bwd),

@@ -107,7 +107,7 @@ class CorpusScorer:
     # fields of the descriptor every rank contributes before the first collective of a call
     _FIELDS = ('call', 'news_num', 'chunk', 'D', 'I', 'n_max', 'H', 'batch', 'corpus ids checksum', 'history_ids checksum',
                'history_len checksum', 'candidate_ids checksum', 'candidate_count checksum', 'labels checksum', 'B', 'P', 'k',
-               'T', 'm', 'exclude_history', 'pool_ids checksum', 'argument error')
+               'T', 'm', 'exclude_history', 'pool_ids checksum', 'exact', 'argument error')
 
     def _agree(self, call, **fields):
         """all-gather a small int64 descriptor of this call's inputs and raise on every rank if any field differs between
@@ -227,7 +227,7 @@ class CorpusScorer:
 
     @torch.no_grad()
     def recommend(self, history_ids, history_len, pool_ids, k, exclude_history=True, pool_tile=None, cuda_graph=True,
-                  max_per_category=None, collective=False):
+                  max_per_category=None, collective=False, exact=True):
         """The k best news of a candidate pool for each user: history_ids [B, H] (0-padded at the end) and history_len [B]
         as in ``score``, pool_ids [P] corpus row ids shared by the B users.  Returns (ids [B, k] int64, scores [B, k] fp32),
         best first.
@@ -262,21 +262,34 @@ class CorpusScorer:
         plain call with the same arguments (the same ``pool_tile``) on one GPU.  The ranks first all-gather a descriptor
         of their arguments: if it differs between ranks, or the arguments fail a check on some ranks only, every rank
         raises RuntimeError naming the fields; a check that fails on every rank raises its ValueError there.  Either way
-        no rank is left in a collective, and the group can be used for the next call."""
+        no rank is left in a collective, and the group can be used for the next call.
+
+        ``exact=False`` scores the tiles through the factored cluster tail (nnr_cluster_tail_scores): the intra-cluster
+        weights of a non-empty cluster sum to 1, so the cluster affine is applied once per history row (Wg = g W^T, with
+        the user side) instead of to C + 1 cluster features per (user, candidate) pair, and the candidate projections run
+        once per pool row instead of once per (user, row).  The scores are those of the SUE formula, within a relative
+        error of 1e-4 of ``score()`` (fp32 sums in another order), but not bit-identical to it or to ``exact=True``, so
+        ids whose scores lie that close to the k-th score may differ between the two.  Everything else is as above: the
+        checks, the order, the exclusions and the fill, ``max_per_category``, ``collective`` (bit-identical to the plain
+        ``exact=False`` call with the same ``pool_tile``), graph replay of full tiles, memory that does not grow with P.
+        The call is deterministic: the same arguments give the same bits.  The default tile is min(P, 4096) candidates
+        (the factored tail holds no per-pair buffers).  SUE_wo_HCA, whose user vector does not depend on the candidate,
+        returns the ``exact=True`` result."""
         if collective:
             return self._recommend_collective(history_ids, history_len, pool_ids, k, exclude_history, pool_tile, cuda_graph,
-                                              max_per_category)
+                                              max_per_category, exact)
         hid, hl, pool, k, T, m, groups = self._recommend_inputs(history_ids, history_len, pool_ids, k, exclude_history,
-                                                                pool_tile, max_per_category)
+                                                                pool_tile, max_per_category, exact)
         B, P = hid.shape[0], pool.numel()
         if P == 0 or B == 0:
             best_score, best_pos, _ = self._fill(B, k)
             return best_pos, best_score                         # ids -1, scores -inf
         best_score, best_pos, _ = self._recommend_tiles(hid, hl, pool, k, T, 0, -(-P // T), exclude_history, m, groups,
-                                                        cuda_graph)
+                                                        cuda_graph, exact)
         return self._pool_ids(pool, best_pos), best_score
 
-    def _recommend_inputs(self, history_ids, history_len, pool_ids, k, exclude_history, pool_tile, max_per_category):
+    def _recommend_inputs(self, history_ids, history_len, pool_ids, k, exclude_history, pool_tile, max_per_category,
+                          exact=True):
         """recommend()'s argument checks, before any kernel launch.  Returns (hid [B, H] int64, hl [B] int32, pool [P] int64
         on the device, k, T, m (None when uncapped), the number of category groups (None when uncapped))."""
         if self.cache is None:
@@ -300,7 +313,10 @@ class CorpusScorer:
         hid = torch.as_tensor(history_ids).to(self.dev).long().contiguous()
         hl = torch.as_tensor(history_len).to(self.dev).to(torch.int32)
         B, H = hid.shape
-        T = int(self.default_pool_tile(B) if pool_tile is None else pool_tile)
+        if pool_tile is not None:
+            T = int(pool_tile)
+        else:
+            T = self.default_pool_tile(B) if exact else max(1, min(pool.numel(), ops.TOPK_MAX_TILE))
         if not 1 <= T <= ops.TOPK_MAX_TILE:
             raise ValueError('CorpusScorer.recommend: pool_tile must be in [1, %d], got %d' % (ops.TOPK_MAX_TILE, T))
         if exclude_history and H > ops.TOPK_MAX_EXCLUDE:
@@ -316,24 +332,28 @@ class CorpusScorer:
     def _pool_ids(pool, best_pos):
         return torch.where(best_pos >= 0, pool[best_pos.clamp(min=0)], torch.full_like(best_pos, -1))
 
-    def _recommend_tiles(self, hid, hl, pool, k, T, first, end, exclude_history, m, groups, cuda_graph):
+    def _recommend_tiles(self, hid, hl, pool, k, T, first, end, exclude_history, m, groups, cuda_graph, exact=True):
         """the best list of pool tiles [first, end) (tile t: pool positions [t * T, min((t + 1) * T, P))): returns
-        (best_score [B, k], best_pos [B, k] pool positions, best_group [B, k] or None when m is None).  No tiles: the fill."""
+        (best_score [B, k], best_pos [B, k] pool positions, best_group [B, k] or None when m is None).  No tiles: the fill.
+        ``exact=False``: the tiles are scored through the factored cluster tail."""
         B, H = hid.shape
         P = pool.numel()
         if first >= end:
             return self._fill(B, k, m is not None)
         ue = self.model.user_encoder
-        side = ue.user_side(self.cache[hid], *self._history_graph(hid, hl))
+        graph = self._history_graph(hid, hl)
+        side = ue.user_side(self.cache[hid], *graph) if exact else ue.user_side(self.cache[hid], *graph, factored=True)
 
         def tile_scores(*args):
             *user, ids = args
+            if not exact:
+                return ue.tile_scores_factored(tuple(user), self.cache[ids])
             return ue.tile_scores(tuple(user), self.cache[ids].unsqueeze(0).expand(B, -1, -1))
 
         best_score = torch.empty(B, k, device=self.dev)
         best_pos = torch.empty(B, k, dtype=torch.int64, device=self.dev)
         best_group = torch.empty(B, k, dtype=torch.int32, device=self.dev) if m is not None else None
-        key = ('recommend', B, H, T, self.cache.data_ptr())
+        key = ('recommend' if exact else 'recommend_factored', B, H, T, self.cache.data_ptr())
         for a in range(first * T, min(end * T, P), T):
             ids = pool[a:a + T]
             if cuda_graph and ids.numel() == T:
@@ -367,7 +387,7 @@ class CorpusScorer:
         return best_score, best_pos
 
     def _recommend_collective(self, history_ids, history_len, pool_ids, k, exclude_history, pool_tile, cuda_graph,
-                              max_per_category):
+                              max_per_category, exact):
         """recommend(collective=True): agree on the arguments, score this rank's share of the tiles, all-gather the rank
         lists and merge them"""
         if self.group is None:
@@ -375,10 +395,10 @@ class CorpusScorer:
         err = None
         try:
             hid, hl, pool, k, T, m, groups = self._recommend_inputs(history_ids, history_len, pool_ids, k, exclude_history,
-                                                                    pool_tile, max_per_category)
+                                                                    pool_tile, max_per_category, exact)
         except (ValueError, RuntimeError) as e:        # raised after the agreement, so that no rank waits in a collective
             err = e
-        fields = {'argument error': int(err is not None)}
+        fields = {'argument error': int(err is not None), 'exact': int(bool(exact))}
         if err is None:
             fields.update({'B': hid.shape[0], 'H': hid.shape[1], 'P': pool.numel(), 'k': k, 'T': T,
                            'm': 0 if max_per_category is None else int(max_per_category),
@@ -398,7 +418,7 @@ class CorpusScorer:
             return best_pos, best_score                         # ids -1, scores -inf
         _, parts = contiguous_blocks(-(-P // T), self.world)
         first, end = parts[self.rank]
-        mine = self._recommend_tiles(hid, hl, pool, k, T, first, end, exclude_history, m, groups, cuda_graph)
+        mine = self._recommend_tiles(hid, hl, pool, k, T, first, end, exclude_history, m, groups, cuda_graph, exact)
         best_score, best_pos = self._gather_and_merge(mine, m, groups)
         return self._pool_ids(pool, best_pos), best_score
 

@@ -89,14 +89,22 @@ class SUE(UserEncoder):
                     layer_norm=getattr(self, 'gcn_layer_norm', False),
                     training=self.training, p_drop=float(self.dropout_rate), category_num=self.category_num - 1 if self.hca else 0)
 
-    def user_side(self, history_embedding, user_history_graph, user_history_category_mask, user_history_category_indices):
+    def user_side(self, history_embedding, user_history_graph, user_history_category_mask, user_history_category_indices,
+                  factored=False):
         """inference (eval mode): the part of encode_user that depends on the history alone, computed once for every tile of
-        candidates scored against these users with ``tile_scores`` (engine.sue_user_side)"""
+        candidates scored against these users with ``tile_scores`` (``tile_scores_factored`` with ``factored=True``;
+        engine.sue_user_side)"""
         user_history_category_mask[:, -1] = 1
         return engine.sue_user_side(self._meta(), history_embedding, user_history_graph, user_history_category_mask,
-                                    user_history_category_indices.long(), *self._params())
+                                    user_history_category_indices.long(), *self._params(), factored=factored)
 
     def tile_scores(self, user_side, candidate_news_representation):
         """click scores [B, T] of candidates [B, T, D] for the users of ``user_side``: equal, bit for bit, to
         RowDot(encode_user(...), candidates) on the same inputs (engine.sue_tile_scores)"""
         return engine.sue_tile_scores(self._meta(), user_side, candidate_news_representation, *self._params())
+
+    def tile_scores_factored(self, user_side, candidate_rows):
+        """click scores [B, T] of candidates [T, D] shared by the users of ``user_side(..., factored=True)``, through the
+        factored cluster tail: equal to tile_scores on the expanded candidates in real arithmetic, not bit for bit
+        (engine.sue_tile_scores_factored)"""
+        return engine.sue_tile_scores_factored(self._meta(), user_side, candidate_rows, *self._params())

@@ -3,7 +3,7 @@ tile, the [B, T] rows copied to the host, concatenated and ``torch.topk``-ed the
 ``extra.scoring``: the synthetic 100 k-news corpus (seed 5, chunk 4096) and the config-2 model (seeded weights).
 
   python scripts/recommend_bench.py [--users 256] [--pools 1000 10000 100000] [--ks 10 100] [--out FILE]
-                                    [--max-per-category M [M ...]]
+                                    [--max-per-category M [M ...] | --factored]
 
 prints one JSON line per (P, k) (appended to FILE too): ms per call and (user, candidate) pairs/s of both paths on the same
 users and pool (median over --reps calls, host clock around calls that end in a device synchronise, after one warm-up
@@ -12,6 +12,12 @@ in a separate pass); peak torch.cuda.max_memory_allocated of each path, over wha
 absolute, and the memory the warm-up call left allocated (the captured graphs' pools, held while the scorer lives); whether
 the two paths return the same top-k scores (recommend without exclusion; checked for P <= --check-max); the card name
 and power limit read in the same run.
+
+With --factored, one line per (P, k) instead: recommend(exact=False) (the factored cluster tail, its default tile) against
+recommend(exact=True) on the same users and pool, the two alternated call by call (--reps each, medians and every time);
+the speed ratio; the largest deviation of the returned scores from the exact scores of the same ids (score() of the
+returned ids, max |factored - exact| / max |exact| over the [B, k] entries); the mean overlap of the two id lists (|common
+ids| / k per user); the card name and power limit.
 
 With --max-per-category, one line per (P, k, m) instead: recommend(max_per_category=m) against the uncapped call on the
 same users and pool, the two alternated call by call (--reps each, medians and every time); the merge's share of each
@@ -109,6 +115,38 @@ def capped_lines(a, sc, ops, hist, hl, pool, P, T, name, watts):
                     f.write(json.dumps(line) + '\n')
 
 
+def emit(a, line):
+    print(json.dumps(line), flush=True)
+    if a.out:
+        with open(a.out, 'a') as f:
+            f.write(json.dumps(line) + '\n')
+
+
+def factored_lines(a, sc, hist, hl, pool, P, name, watts):
+    """--factored: one line per k, recommend(exact=False) against recommend(exact=True) alternated in the same run"""
+    B = hist.shape[0]
+    for k in a.ks:
+        exact = lambda: sc.recommend(hist, hl, pool, k)
+        fact = lambda: sc.recommend(hist, hl, pool, k, exact=False)
+        ex_out, fa_out = exact(), fact()                              # warm-up: graph capture, workspaces
+        t_ex, t_fa = [], []
+        for r in range(a.reps):                                       # alternate, and alternate which goes first
+            for fn, ts in ((exact, t_ex), (fact, t_fa))[::1 if r % 2 == 0 else -1]:
+                ts.append(timed(fn, 1)[0])
+        ids, scores = fa_out
+        real = ids >= 0
+        ref = sc.score(hist, hl, ids.clamp(min=0), cuda_graph=False)  # exact scores of the returned ids
+        dev = float(((scores - ref).abs() * real).max() / (ref.abs() * real).max())
+        overlap = float(np.mean([len(set(f.tolist()) & set(e.tolist()) - {-1}) / min(k, P)
+                                 for f, e in zip(ids.cpu(), ex_out[0].cpu())]))
+        e, f = statistics.median(t_ex), statistics.median(t_fa)
+        emit(a, dict(users=B, pool=P, k=k, factored_pool_tile=min(P, 4096), exact_pool_tile=sc.default_pool_tile(B),
+                     corpus_news=a.news, history=hist.shape[1], exact_ms=e, factored_ms=f, speed_ratio=e / f,
+                     exact_ms_all=t_ex, factored_ms_all=t_fa, factored_pairs_per_sec=B * P / (f * 1e-3),
+                     max_rel_score_deviation=dev, mean_id_overlap=overlap, card=name, power_limit_w=watts,
+                     time=time.strftime('%Y-%m-%dT%H:%M:%S')))
+
+
 def peak_mb(fn):
     """(peak over what was allocated before the call, absolute peak) of torch.cuda.max_memory_allocated during fn(), MiB"""
     torch.cuda.synchronize()
@@ -131,6 +169,7 @@ def main():
     ap.add_argument('--out', default=None)
     ap.add_argument('--max-per-category', type=int, nargs='+', default=None,
                     help='time recommend(max_per_category=m) against the uncapped call, for each m')
+    ap.add_argument('--factored', action='store_true', help='time recommend(exact=False) against recommend(exact=True)')
     a = ap.parse_args()
     import nnr_b200
     from nnr_b200 import ops
@@ -160,6 +199,9 @@ def main():
         pool = torch.from_numpy(np.random.default_rng(3).choice(a.news, P, replace=False)).to(dev)
         if a.max_per_category:
             capped_lines(a, sc, ops, hist, hl, pool, P, T, name, watts)
+            continue
+        if a.factored:
+            factored_lines(a, sc, hist, hl, pool, P, name, watts)
             continue
         for k in a.ks:
             rec = lambda: sc.recommend(hist, hl, pool, k)
