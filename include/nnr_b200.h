@@ -33,7 +33,7 @@
 extern "C" {
 #endif
 
-#define NNR_ABI_VERSION 9
+#define NNR_ABI_VERSION 10
 #define NNR_SEED_INDIRECT (1ULL << 62)
 
 const char* nnr_last_error(void);
@@ -339,6 +339,21 @@ int nnr_cluster_intra_bwd(const float* dintra, const float* Kp, const float* Qp,
 int nnr_cluster_tail_scores(const float* Kp, const float* g, const float* Wg, const int64_t* idx, const uint8_t* cmask,
                             const float* Qp, const float* qk2, const float* cand, const float* bias, int B, int H, int Au,
                             int D, int C1, int T, float scale, float* scores, int64_t lds, void* stream);
+/* The same factored tail for per-user candidate lists stored back to back (dev/test evaluation;
+ * scoring.CorpusScorer.evaluate(exact=False)): user b's candidates are rows [row_off[b], row_off[b+1]) of Qp [rows,Au],
+ * qk2 [rows,D] and cand [rows,D]; the score of its j-th candidate goes to scores[b*lds + j], and entries j >= its count
+ * are not written.  Kp, g, Wg, idx, cmask and bias are as above.  Given the same rows, every score equals
+ * nnr_cluster_tail_scores' bit for bit (one shared per-candidate code path).  The work follows the sum of the counts, not
+ * B * n_max: a CTA holds a slice of one user's list, and a slice past the count exits at once.
+ * row_off [B+1] int32 lives on the device and is not checked by the host: each count is clamped to [0, n_max] and each
+ * row to [0, rows), so bad offsets read and write nothing out of bounds.
+ * Deterministic (no atomics), no allocation, no host synchronisation (graph-capturable).
+ * Limits: B >= 0, 1 <= n_max <= lds, 0 <= rows < 2^31, H <= 256, C1 <= 72 (NNR_ERR_ARG / NNR_ERR_UNSUPPORTED before any
+ * CUDA call otherwise); D % 4 == 0 and 16-byte aligned g, Wg, qk2, cand, bias (NNR_ERR_UNSUPPORTED).                  */
+int nnr_cluster_tail_scores_packed(const float* Kp, const float* g, const float* Wg, const int64_t* idx,
+                                   const uint8_t* cmask, const int32_t* row_off, int64_t rows, const float* Qp,
+                                   const float* qk2, const float* cand, const float* bias, int B, int H, int Au, int D,
+                                   int C1, int n_max, float scale, float* scores, int64_t lds, void* stream);
 
 /* ---- click predictor: model.py:127 ---------------------------------------------------------- */
 int nnr_rowdot_fwd(const float* a, const float* b, int R, int D, float* out, void* stream);

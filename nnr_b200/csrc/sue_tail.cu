@@ -18,6 +18,11 @@
 //      score = sum_c beta_c (f_c . cand).
 // Every sum runs in a fixed order and every accumulator has one owner thread: the result is deterministic.  After phase 2
 // a thread reads only its own candidates' columns, so phases 3-5 need no barrier.
+//
+// nnr_cluster_tail_scores_packed (evaluate(exact=False)) runs the same phases (tail_cta) on per-user candidate lists
+// stored back to back, one CTA per (user, slice of TAIL_PC candidates).  A MIND list has ~37 candidates, too few to hide
+// the latency of phase 4's loads with one warp, so W warps split the slots, the clusters and the feature steps, and the
+// partial dots of a round of W steps are added in step order: the scores equal the pool kernel's bit for bit.
 #include "common.cuh"
 #include "../../include/nnr_b200.h"
 
@@ -25,6 +30,7 @@
 #define TAIL_MAXC 72
 #define TAIL_KC 16             // Au features per staged chunk of the logits
 #define TAIL_TT 2              // candidates per thread
+#define TAIL_PC 64             // candidates per CTA of the packed kernel: MIND lists are ~37 long
 
 __device__ __forceinline__ void tail_load(float* dst, const float* src, int n4) {
 #pragma unroll
@@ -34,18 +40,16 @@ __device__ __forceinline__ void tail_load(float* dst, const float* src, int n4) 
   }
 }
 
-// phase 4 for features [d0, d0 + DD) of the thread's candidates
-template <int NT, int DD>
-__device__ __forceinline__ void tail_step(int d0, const float* __restrict__ gb, const float* __restrict__ wb,
-                                          const float* __restrict__ qk2, const float* __restrict__ cand,
-                                          const float* __restrict__ bias, const float* s_al, float* s_acc,
-                                          const int* s_perm, const int* s_start, int C1, int D, int T, int t0, int tid,
-                                          float* eq, float* ec) {
-  constexpr int TC = NT * TAIL_TT;
-  float q[TAIL_TT][DD], x[TAIL_TT][DD], bv[DD];
+// the dots of relu(b) (every empty cluster's feature) with features [d0, d0 + DD) of the candidates' qk2 and cand rows,
+// accumulated into eq / ec; candidate j of the thread is column col + j * CS of the CTA's slice
+template <int CS, int DD>
+__device__ __forceinline__ void tail_empty_dots(int d0, const float* __restrict__ qk2, const float* __restrict__ cand,
+                                                const float* __restrict__ bias, int D, int T, int t0, int col,
+                                                float (&q)[TAIL_TT][DD], float (&x)[TAIL_TT][DD], float (&bv)[DD],
+                                                float* eq, float* ec) {
 #pragma unroll
   for (int j = 0; j < TAIL_TT; ++j) {
-    const int t = t0 + tid + j * NT;
+    const int t = t0 + col + j * CS;
     if (t < T) {
       tail_load(q[j], qk2 + (size_t)t * D + d0, DD / 4);
       tail_load(x[j], cand + (size_t)t * D + d0, DD / 4);
@@ -63,6 +67,20 @@ __device__ __forceinline__ void tail_step(int d0, const float* __restrict__ gb, 
       eq[j] = fmaf(f, q[j][k], eq[j]);
       ec[j] = fmaf(f, x[j][k], ec[j]);
     }
+}
+
+// phase 4 for features [d0, d0 + DD) of the thread's candidates.  ADD: add each non-empty cluster's two partial dots to
+// acc (the running per-(cluster, candidate) sums); otherwise store them there (one step's partials, summed in step order
+// by the caller)
+template <int CS, int DD, bool ADD>
+__device__ __forceinline__ void tail_step(int d0, const float* __restrict__ gb, const float* __restrict__ wb,
+                                          const float* __restrict__ qk2, const float* __restrict__ cand,
+                                          const float* __restrict__ bias, const float* s_al, float* acc,
+                                          const int* s_perm, const int* s_start, int C1, int D, int T, int t0, int col,
+                                          float* eq, float* ec) {
+  constexpr int TC = CS * TAIL_TT;
+  float q[TAIL_TT][DD], x[TAIL_TT][DD], bv[DD];
+  tail_empty_dots<CS, DD>(d0, qk2, cand, bias, D, T, t0, col, q, x, bv, eq, ec);
   for (int c = 0; c < C1; ++c) {
     const int lo = s_start[c], hi = s_start[c + 1];
     if (lo == hi) continue;
@@ -78,7 +96,7 @@ __device__ __forceinline__ void tail_step(int d0, const float* __restrict__ gb, 
       tail_load(wv, wb + (size_t)h * D + d0, DD / 4);
       tail_load(gv, gb + (size_t)h * D + d0, DD / 4);
 #pragma unroll
-      for (int j = 0; j < TAIL_TT; ++j) a[j] = s_al[e * TC + tid + j * NT];
+      for (int j = 0; j < TAIL_TT; ++j) a[j] = s_al[e * TC + col + j * CS];
 #pragma unroll
       for (int j = 0; j < TAIL_TT; ++j)
 #pragma unroll
@@ -96,19 +114,28 @@ __device__ __forceinline__ void tail_step(int d0, const float* __restrict__ gb, 
         pq = fmaf(f, q[j][k], pq);
         pc = fmaf(f, x[j][k], pc);
       }
-      s_acc[c * TC + tid + j * NT] += pq;
-      s_acc[(C1 + c) * TC + tid + j * NT] += pc;
+      float* aq = acc + c * TC + col + j * CS;
+      float* ac = acc + (C1 + c) * TC + col + j * CS;
+      if (ADD) { *aq += pq; *ac += pc; } else { *aq = pq; *ac = pc; }
     }
   }
 }
 
-template <int NT>
-__global__ void __launch_bounds__(NT) cluster_tail_scores_kernel(
-    const float* __restrict__ Kp, const float* __restrict__ g, const float* __restrict__ Wg, const int64_t* __restrict__ idx,
-    const uint8_t* __restrict__ cmask, const float* __restrict__ Qp, const float* __restrict__ qk2,
-    const float* __restrict__ cand, const float* __restrict__ bias, int H, int Au, int D, int C1, int T, float scale,
-    float* __restrict__ scores, int64_t lds) {
-  constexpr int TC = NT * TAIL_TT;
+// phases 1-5 of one CTA: candidates [t0, min(t0 + TC, T)) of user b, whose candidate rows start at Qp, qk2 and cand;
+// candidate t's score goes to srow[t].  Shared by the pool and the packed kernel, so that both sum in the same order.
+// NT = CS * W threads: thread tid owns the candidate columns col + j * CS (col = tid % CS, j < TAIL_TT) of the slice for
+// the slots e, the clusters c and the feature steps s with e, c, s = grp (mod W) (grp = tid / CS).  W = 1 (the pool
+// kernel): one thread does all of a candidate's work, and phases 3-5 need no barrier.  W > 1: the W groups take turns
+// over the feature steps; the W partial dots of a round are stored in s_part and added to the running sums in step
+// order, so every sum runs in the order of W = 1.
+template <int CS, int W>
+__device__ __forceinline__ void tail_cta(const float* __restrict__ Kp, const float* __restrict__ g,
+                                         const float* __restrict__ Wg, const int64_t* __restrict__ idx,
+                                         const uint8_t* __restrict__ cmask, const float* __restrict__ Qp,
+                                         const float* __restrict__ qk2, const float* __restrict__ cand,
+                                         const float* __restrict__ bias, int b, int H, int Au, int D, int C1, int T, int t0,
+                                         float scale, float* __restrict__ srow) {
+  constexpr int NT = CS * W, TC = CS * TAIL_TT;
   extern __shared__ __align__(16) float sm[];
   float* s_al = sm;                                   // [H][TC]: logits, then alpha (slots in cluster order)
   float* s_acc = sm + (size_t)H * TC;                 // [2][C1][TC]: f . qk2, f . cand of the non-empty clusters
@@ -117,7 +144,7 @@ __global__ void __launch_bounds__(NT) cluster_tail_scores_kernel(
   __shared__ int s_idx[TAIL_MAXH];
   __shared__ int s_perm[TAIL_MAXH];
   __shared__ int s_start[TAIL_MAXC + 1];
-  const int b = blockIdx.x, t0 = blockIdx.y * TC, tid = threadIdx.x;
+  const int tid = threadIdx.x, col = W == 1 ? tid : tid % CS, grp = W == 1 ? 0 : tid / CS;
 
   // 1. stable counting sort of the slots by cluster
   for (int h = tid; h < H; h += NT) { const int c = (int)idx[(size_t)b * H + h]; s_idx[h] = min(max(c, 0), C1 - 1); }
@@ -152,8 +179,8 @@ __global__ void __launch_bounds__(NT) cluster_tail_scores_kernel(
 #pragma unroll
     for (int j = 0; j < TAIL_TT; ++j)
 #pragma unroll
-      for (int a = 0; a < TAIL_KC; ++a) q[j][a] = s_q[a * (TC + 1) + tid + j * NT];
-    for (int e = 0; e < H; ++e) {
+      for (int a = 0; a < TAIL_KC; ++a) q[j][a] = s_q[a * (TC + 1) + col + j * CS];
+    for (int e = grp; e < H; e += W) {
       const float4* kr = reinterpret_cast<const float4*>(s_k + e * TAIL_KC);
       float v[TAIL_TT] = {};
 #pragma unroll
@@ -169,7 +196,7 @@ __global__ void __launch_bounds__(NT) cluster_tail_scores_kernel(
       }
 #pragma unroll
       for (int j = 0; j < TAIL_TT; ++j) {
-        float* p = s_al + e * TC + tid + j * NT;
+        float* p = s_al + e * TC + col + j * CS;
         *p = (a0 == 0) ? v[j] : *p + v[j];
       }
     }
@@ -179,34 +206,73 @@ __global__ void __launch_bounds__(NT) cluster_tail_scores_kernel(
   // 3. softmax within each cluster (max-shifted, like torch_scatter.scatter_softmax)
 #pragma unroll
   for (int j = 0; j < TAIL_TT; ++j) {
-    float* col = s_al + tid + j * NT;
-    for (int e = 0; e < H; ++e) col[e * TC] *= scale;
-    for (int c = 0; c < C1; ++c) {
+    float* col_j = s_al + col + j * CS;
+    if (W == 1)
+      for (int e = 0; e < H; ++e) col_j[e * TC] *= scale;
+    else
+      for (int c = grp; c < C1; c += W)
+        for (int e = s_start[c]; e < s_start[c + 1]; ++e) col_j[e * TC] *= scale;
+    for (int c = grp; c < C1; c += W) {
       const int lo = s_start[c], hi = s_start[c + 1];
       if (lo == hi) continue;
       float m = -INFINITY;
-      for (int e = lo; e < hi; ++e) m = fmaxf(m, col[e * TC]);
+      for (int e = lo; e < hi; ++e) m = fmaxf(m, col_j[e * TC]);
       float sum = 0.f;
-      for (int e = lo; e < hi; ++e) sum += expf(col[e * TC] - m);
-      for (int e = lo; e < hi; ++e) col[e * TC] = expf(col[e * TC] - m) / sum;
+      for (int e = lo; e < hi; ++e) sum += expf(col_j[e * TC] - m);
+      for (int e = lo; e < hi; ++e) col_j[e * TC] = expf(col_j[e * TC] - m) / sum;
     }
-    for (int c = 0; c < C1; ++c) s_acc[c * TC + tid + j * NT] = s_acc[(C1 + c) * TC + tid + j * NT] = 0.f;
+    for (int c = grp; c < C1; c += W) s_acc[c * TC + col + j * CS] = s_acc[(C1 + c) * TC + col + j * CS] = 0.f;
   }
 
   // 4. the two dots of every cluster feature, DD features at a time (D % 4 == 0)
   const float* gb = g + (size_t)b * H * D;
   const float* wb = Wg + (size_t)b * H * D;
   float eq[TAIL_TT] = {}, ec[TAIL_TT] = {};
-  int d0 = 0;
-  for (; d0 + 8 <= D; d0 += 8)
-    tail_step<NT, 8>(d0, gb, wb, qk2, cand, bias, s_al, s_acc, s_perm, s_start, C1, D, T, t0, tid, eq, ec);
-  if (d0 < D) tail_step<NT, 4>(d0, gb, wb, qk2, cand, bias, s_al, s_acc, s_perm, s_start, C1, D, T, t0, tid, eq, ec);
+  if (W == 1) {
+    int d0 = 0;
+    for (; d0 + 8 <= D; d0 += 8)
+      tail_step<CS, 8, true>(d0, gb, wb, qk2, cand, bias, s_al, s_acc, s_perm, s_start, C1, D, T, t0, col, eq, ec);
+    if (d0 < D) tail_step<CS, 4, true>(d0, gb, wb, qk2, cand, bias, s_al, s_acc, s_perm, s_start, C1, D, T, t0, col, eq, ec);
+  } else {
+    float* s_part = s_acc + (size_t)2 * C1 * TC;      // [W][2][C1][TC]: one round's partial dots (past the staging)
+    __syncthreads();                                  // alpha and the zeroed sums of the other groups
+    const int steps = (D + 7) / 8;
+    for (int r0 = 0; r0 < steps; r0 += W) {
+      const int d0 = 8 * (r0 + grp);
+      float* part = s_part + (size_t)grp * 2 * C1 * TC;
+      float dq[TAIL_TT] = {}, dc[TAIL_TT] = {};       // the empty-cluster dots are summed by group 0 alone, below
+      if (d0 + 8 <= D)
+        tail_step<CS, 8, false>(d0, gb, wb, qk2, cand, bias, s_al, part, s_perm, s_start, C1, D, T, t0, col, dq, dc);
+      else if (d0 < D)
+        tail_step<CS, 4, false>(d0, gb, wb, qk2, cand, bias, s_al, part, s_perm, s_start, C1, D, T, t0, col, dq, dc);
+      __syncthreads();
+      const int nw = min(W, steps - r0);
+      for (int c = grp; c < C1; c += W) {
+        if (s_start[c] == s_start[c + 1]) continue;
+#pragma unroll
+        for (int j = 0; j < TAIL_TT; ++j)
+          for (int w = 0; w < nw; ++w) {
+            s_acc[c * TC + col + j * CS] += s_part[((size_t)w * 2 * C1 + c) * TC + col + j * CS];
+            s_acc[(C1 + c) * TC + col + j * CS] += s_part[((size_t)w * 2 * C1 + C1 + c) * TC + col + j * CS];
+          }
+      }
+      __syncthreads();
+    }
+    if (grp != 0) return;
+    int d0 = 0;
+    float q[TAIL_TT][8], x[TAIL_TT][8], bv[8];
+    for (; d0 + 8 <= D; d0 += 8) tail_empty_dots<CS, 8>(d0, qk2, cand, bias, D, T, t0, col, q, x, bv, eq, ec);
+    if (d0 < D) {
+      float q4[TAIL_TT][4], x4[TAIL_TT][4], bv4[4];
+      tail_empty_dots<CS, 4>(d0, qk2, cand, bias, D, T, t0, col, q4, x4, bv4, eq, ec);
+    }
+  }
 
   // 5. inter-cluster attention and the click score
   const uint8_t* cm = cmask + (size_t)b * C1;
 #pragma unroll
   for (int j = 0; j < TAIL_TT; ++j) {
-    const int tl = tid + j * NT;
+    const int tl = col + j * CS;
     if (t0 + tl >= T) continue;
     float m = -INFINITY;
     for (int c = 0; c < C1; ++c) {
@@ -225,14 +291,55 @@ __global__ void __launch_bounds__(NT) cluster_tail_scores_kernel(
       const float l = cm[c] ? scale * (full ? s_acc[c * TC + tl] : eq[j]) : -1e9f;
       out = fmaf(expf(l - m) * inv, full ? s_acc[(C1 + c) * TC + tl] : ec[j], out);
     }
-    scores[(size_t)b * lds + t0 + tl] = out;
+    srow[t0 + tl] = out;
   }
 }
 
+template <int NT>
+__global__ void __launch_bounds__(NT) cluster_tail_scores_kernel(
+    const float* __restrict__ Kp, const float* __restrict__ g, const float* __restrict__ Wg, const int64_t* __restrict__ idx,
+    const uint8_t* __restrict__ cmask, const float* __restrict__ Qp, const float* __restrict__ qk2,
+    const float* __restrict__ cand, const float* __restrict__ bias, int H, int Au, int D, int C1, int T, float scale,
+    float* __restrict__ scores, int64_t lds) {
+  const int b = blockIdx.x;
+  tail_cta<NT, 1>(Kp, g, Wg, idx, cmask, Qp, qk2, cand, bias, b, H, Au, D, C1, T, blockIdx.y * NT * TAIL_TT, scale,
+               scores + (size_t)b * lds);
+}
+
+// packed candidate lists: CTA x = (user b, slice s) of ns slices of TAIL_PC candidates, W warps; user b's candidates are
+// rows [row_off[b], row_off[b + 1]) of Qp / qk2 / cand.  The offsets come from the device unchecked: the count is clamped
+// to [0, n_max] and the rows to [0, rows), and a CTA whose slice starts past the count exits before it reads anything else.
+template <int W>
+__global__ void __launch_bounds__(32 * W) cluster_tail_scores_packed_kernel(
+    const float* __restrict__ Kp, const float* __restrict__ g, const float* __restrict__ Wg, const int64_t* __restrict__ idx,
+    const uint8_t* __restrict__ cmask, const int32_t* __restrict__ row_off, int64_t rows, const float* __restrict__ Qp,
+    const float* __restrict__ qk2, const float* __restrict__ cand, const float* __restrict__ bias, int ns, int H, int Au,
+    int D, int C1, int n_max, float scale, float* __restrict__ scores, int64_t lds) {
+  const int b = blockIdx.x / ns, t0 = (blockIdx.x % ns) * TAIL_PC;
+  const int64_t lo = min(max((int64_t)row_off[b], (int64_t)0), rows);
+  const int64_t hi = min(max((int64_t)row_off[b + 1], lo), rows);
+  const int T = (int)min(hi - lo, (int64_t)n_max);
+  if (t0 >= T) return;
+  tail_cta<32, W>(Kp, g, Wg, idx, cmask, Qp + lo * Au, qk2 + lo * D, cand + lo * D, bias, b, H, Au, D, C1, T, t0, scale,
+                  scores + (size_t)b * lds);
+}
+
 // dynamic shared memory of a CTA of TC candidates: the logits / alpha and the larger of the accumulators and the staging
-static size_t tail_smem(int H, int C1, int TC) {
-  const size_t acc = (size_t)2 * C1 * TC, stage = (size_t)TAIL_KC * (TC + 1) + (size_t)H * TAIL_KC;
+// (W > 1: and W rounds of partial dots after the accumulators)
+static size_t tail_smem(int H, int C1, int TC, int W = 1) {
+  const size_t acc = (size_t)2 * C1 * TC * (W > 1 ? 1 + W : 1), stage = (size_t)TAIL_KC * (TC + 1) + (size_t)H * TAIL_KC;
   return ((size_t)H * TC + (acc > stage ? acc : stage)) * sizeof(float);
+}
+
+// raise a kernel's dynamic shared memory limit to ``most`` bytes, once per device
+static int tail_smem_attr(const void* fn, size_t most, bool* attr_set) {
+  int dev = 0;
+  NNR_CUDA(cudaGetDevice(&dev));
+  if (dev >= 64 || !attr_set[dev]) {
+    NNR_CUDA(cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)most));
+    if (dev < 64) attr_set[dev] = true;
+  }
+  return 0;
 }
 
 template <int NT>
@@ -240,13 +347,7 @@ static int tail_launch(const float* Kp, const float* g, const float* Wg, const i
                        const float* Qp, const float* qk2, const float* cand, const float* bias, int B, int H, int Au, int D,
                        int C1, int T, float scale, float* scores, int64_t lds, size_t smem, size_t most, void* stream) {
   static bool attr_set[64] = {};                                // one per instantiation and device
-  int dev = 0;
-  NNR_CUDA(cudaGetDevice(&dev));
-  if (dev >= 64 || !attr_set[dev]) {
-    NNR_CUDA(cudaFuncSetAttribute((const void*)cluster_tail_scores_kernel<NT>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                  (int)most));
-    if (dev < 64) attr_set[dev] = true;
-  }
+  if (int rc = tail_smem_attr((const void*)cluster_tail_scores_kernel<NT>, most, attr_set)) return rc;
   constexpr int TC = NT * TAIL_TT;
   cluster_tail_scores_kernel<NT><<<dim3(B, (T + TC - 1) / TC), NT, smem, (cudaStream_t)stream>>>(
       Kp, g, Wg, idx, cmask, Qp, qk2, cand, bias, H, Au, D, C1, T, scale, scores, lds);
@@ -281,4 +382,49 @@ extern "C" int nnr_cluster_tail_scores(const float* Kp, const float* g, const fl
                            stream);
   return tail_launch<64>(Kp, g, Wg, idx, cmask, Qp, qk2, cand, bias, B, H, Au, D, C1, T, scale, scores, lds,
                          tail_smem(H, C1, 64 * TAIL_TT), tail_smem(TAIL_MAXH, TAIL_MAXC, 64 * TAIL_TT), stream);
+}
+
+template <int W>
+static int tail_packed_launch(const float* Kp, const float* g, const float* Wg, const int64_t* idx, const uint8_t* cmask,
+                              const int32_t* row_off, int64_t rows, const float* Qp, const float* qk2, const float* cand,
+                              const float* bias, int B, int H, int Au, int D, int C1, int n_max, float scale, float* scores,
+                              int64_t lds, size_t smem, size_t most, void* stream) {
+  static bool attr_set[64] = {};
+  if (int rc = tail_smem_attr((const void*)cluster_tail_scores_packed_kernel<W>, most, attr_set)) return rc;
+  const int ns = (n_max + TAIL_PC - 1) / TAIL_PC;
+  cluster_tail_scores_packed_kernel<W><<<(unsigned)((int64_t)B * ns), 32 * W, smem, (cudaStream_t)stream>>>(
+      Kp, g, Wg, idx, cmask, row_off, rows, Qp, qk2, cand, bias, ns, H, Au, D, C1, n_max, scale, scores, lds);
+  NNR_LAUNCH_CHECK(W == 8 ? "cluster_tail_scores_packed_kernel<8>" : "cluster_tail_scores_packed_kernel<2>");
+  return 0;
+}
+
+extern "C" int nnr_cluster_tail_scores_packed(const float* Kp, const float* g, const float* Wg, const int64_t* idx,
+                                              const uint8_t* cmask, const int32_t* row_off, int64_t rows, const float* Qp,
+                                              const float* qk2, const float* cand, const float* bias, int B, int H, int Au,
+                                              int D, int C1, int n_max, float scale, float* scores, int64_t lds,
+                                              void* stream) {
+  const char* who = "nnr_cluster_tail_scores_packed";
+  NNR_REQUIRE(Kp && g && Wg && idx && cmask && row_off && Qp && qk2 && cand && bias && scores, NNR_ERR_ARG,
+              "%s: Kp, g, Wg, idx, cmask, row_off, Qp, qk2, cand, bias and scores must not be NULL", who);
+  NNR_REQUIRE(B >= 0 && H >= 1 && Au >= 1 && D >= 1 && C1 >= 1, NNR_ERR_ARG,
+              "%s: bad sizes B=%d H=%d Au=%d D=%d C1=%d (B >= 0, the others >= 1)", who, B, H, Au, D, C1);
+  NNR_REQUIRE(n_max >= 1 && n_max <= lds, NNR_ERR_ARG, "%s: n_max must be in [1, lds = %lld], got %d", who, (long long)lds,
+              n_max);
+  NNR_REQUIRE(rows >= 0 && rows < ((int64_t)1 << 31), NNR_ERR_ARG, "%s: rows must be in [0, 2^31), got %lld", who,
+              (long long)rows);
+  NNR_REQUIRE((int64_t)B * ((n_max + TAIL_PC - 1) / TAIL_PC) < ((int64_t)1 << 31), NNR_ERR_ARG,
+              "%s: bad sizes: B (%d) x n_max (%d) needs more than 2^31 - 1 CTAs", who, B, n_max);
+  NNR_REQUIRE(H <= TAIL_MAXH && C1 <= TAIL_MAXC, NNR_ERR_UNSUPPORTED, "%s: needs H <= %d and C1 <= %d, got H=%d C1=%d", who,
+              TAIL_MAXH, TAIL_MAXC, H, C1);
+  NNR_REQUIRE(D % 4 == 0 && nnr_aligned16(g) && nnr_aligned16(Wg) && nnr_aligned16(qk2) && nnr_aligned16(cand) &&
+                  nnr_aligned16(bias),
+              NNR_ERR_UNSUPPORTED, "%s: needs D %% 4 == 0 (got %d) and 16-byte aligned g, Wg, qk2, cand and bias", who, D);
+  if (B == 0) return 0;
+  // 8 warps when two CTAs fit on an SM (the default H = 50, C1 = 19 needs 98 KB), 2 otherwise (176 KB at H = 256, C1 = 72)
+  const size_t wide = tail_smem(H, C1, TAIL_PC, 8);
+  if (wide <= TAIL_SMEM_PAIR)
+    return tail_packed_launch<8>(Kp, g, Wg, idx, cmask, row_off, rows, Qp, qk2, cand, bias, B, H, Au, D, C1, n_max, scale,
+                                 scores, lds, wide, TAIL_SMEM_PAIR, stream);
+  return tail_packed_launch<2>(Kp, g, Wg, idx, cmask, row_off, rows, Qp, qk2, cand, bias, B, H, Au, D, C1, n_max, scale,
+                               scores, lds, tail_smem(H, C1, TAIL_PC, 2), tail_smem(TAIL_MAXH, TAIL_MAXC, TAIL_PC, 2), stream);
 }

@@ -173,10 +173,10 @@ def _param_grads(P, names, G):
     return tuple(G.get(k) for k in names)
 
 
-def _shared_split(x, rows, cols, colsum_out=None):
+def _shared_split(x, rows, cols, colsum_out=None, m_dev=None):
     """operand planes of a small activation that feeds two GEMMs (and, with ``colsum_out``, its column sums = a bias
-    gradient)"""
-    return ops.tc_split(x, rows, cols, x.stride(0), colsum_out=colsum_out)
+    gradient); ``m_dev``: an int32 device scalar, rows from it on are not read"""
+    return ops.tc_split(x, rows, cols, x.stride(0), m_dev, colsum_out=colsum_out)
 
 
 def _fused_relu_bwd(dy, cols):
@@ -837,16 +837,17 @@ class SUEFunction(torch.autograd.Function):
         return pooled, u, alpha
 
     @staticmethod
-    def _cand_side(P, cand, B, n, D):
+    def _cand_side(P, cand, B, n, D, m_dev=None):
         """what the cluster attentions need from the candidates alone (userEncoders.py:84,94: the two query projections;
-        the inter-cluster K is folded onto its query)"""
+        the inter-cluster K is folded onto its query).  ``m_dev``: an int32 device scalar; only the first *m_dev of the
+        B * n rows are computed (the rest of the outputs is left unwritten)"""
         Au = P['intraCluster_K.weight'].shape[0]
-        cand_pl = _shared_split(cand.view(B * n, D), B * n, D)     # also the weight-gradient operand of the backward
-        Qp = linear(cand.view(B * n, D), P['intraCluster_Q.weight'], B * n, None, P['intraCluster_Q.bias'], x_planes=cand_pl)
-        q2 = linear(cand.view(B * n, D), P['interClusterAttention.Q.weight'], B * n, None, P['interClusterAttention.Q.bias'],
+        cand_pl = _shared_split(cand.view(B * n, D), B * n, D, m_dev=m_dev)   # also the weight-gradient operand of the backward
+        Qp = linear(cand.view(B * n, D), P['intraCluster_Q.weight'], B * n, m_dev, P['intraCluster_Q.bias'], x_planes=cand_pl)
+        q2 = linear(cand.view(B * n, D), P['interClusterAttention.Q.weight'], B * n, m_dev, P['interClusterAttention.Q.bias'],
                     x_planes=cand_pl)
-        q2_pl = _shared_split(q2, B * n, Au)
-        qk2 = matmul_nn(q2, P['interClusterAttention.K.weight'], B * n, x_planes=q2_pl)
+        q2_pl = _shared_split(q2, B * n, Au, m_dev=m_dev)
+        qk2 = matmul_nn(q2, P['interClusterAttention.K.weight'], B * n, m_dev, x_planes=q2_pl)
         return cand_pl, Qp, q2, q2_pl, qk2
 
     @staticmethod
@@ -1140,3 +1141,35 @@ def sue_tile_scores_factored(meta, side, cand_rows, *params):
     ops.cluster_tail_scores(Kp, gfeat, Wg, cidx, cmask.contiguous().view(torch.uint8), Qp, qk2, cand_rows.contiguous(),
                             P['clusterFeatureAffine.bias'], B, H, Au, D, C1, T, 1.0 / math.sqrt(float(Au)), scores)
     return scores
+
+
+@torch.no_grad()
+def sue_packed_scores_factored(meta, side, cand_rows, row_off, out, *params):
+    """click scores of per-user candidate lists through the factored cluster tail (nnr_cluster_tail_scores_packed): user
+    b of ``side`` (from ``sue_user_side(..., factored=True)``) has the candidates cand_rows [row_off[b], row_off[b + 1])
+    (cand_rows [R, D] with R >= row_off[B], row_off [B + 1] int32 on the device); the score of its j-th candidate goes to
+    out[b, j], and entries past its count are left as they are.  The candidate projections cost row_off[B] rows, not R.
+    The scores are those of ``sue_tile_scores_factored`` on the same rows, bit for bit.  SUE_wo_HCA, whose user vector
+    does not depend on the candidate: RowDot of the pooled user vector and each row, bit for bit the exact path's."""
+    R, D = cand_rows.shape
+    B, n_max = out.shape
+    cand_rows = cand_rows.contiguous()
+    total = row_off[B:]                                                      # int32 device scalar: the valid rows
+    if not meta['hca']:
+        user_of_row = torch.searchsorted(row_off[1:], torch.arange(R, dtype=torch.int32, device=out.device), right=True)
+        dots = _empty((R,), out.device)
+        ops.rowdot_fwd(side[0][user_of_row.clamp_(max=B - 1)].contiguous(), cand_rows, R, D, dots)
+        j = torch.arange(n_max, device=out.device)
+        lo = row_off[:B].long()
+        valid = j[None, :] < (row_off[1:B + 1].long() - lo)[:, None]
+        out.copy_(torch.where(valid, dots[(lo[:, None] + j[None, :]).clamp_(0, max(R - 1, 0))], out))
+        return out
+    P = dict(zip(sue_names(meta), params))
+    gfeat, Kp, cmask, cidx, Wg = side
+    H = gfeat.shape[1]
+    C1 = cmask.shape[1]
+    Au = P['intraCluster_K.weight'].shape[0]
+    _, Qp, _, _, qk2 = SUEFunction._cand_side(P, cand_rows, 1, R, D, m_dev=total)
+    ops.cluster_tail_scores_packed(Kp, gfeat, Wg, cidx, cmask.contiguous().view(torch.uint8), row_off, Qp, qk2, cand_rows,
+                                   P['clusterFeatureAffine.bias'], B, H, Au, D, C1, n_max, 1.0 / math.sqrt(float(Au)), out)
+    return out

@@ -442,6 +442,16 @@ def cluster_tail_scores(Kp, g, Wg, idx, cmask, Qp, qk2, cand, bias, B, H, Au, D,
                                       _p(scores, _F32), scores.stride(0), _stream()), 'nnr_cluster_tail_scores')
 
 
+def cluster_tail_scores_packed(Kp, g, Wg, idx, cmask, row_off, Qp, qk2, cand, bias, B, H, Au, D, C1, n_max, scale, scores):
+    """click scores [B, n_max] (row stride scores.stride(0)) of per-user candidate lists: user b's are rows
+    [row_off[b], row_off[b + 1]) of Qp / qk2 / cand (Qp.shape[0] rows), through the factored cluster tail; entries past a
+    user's count are left as they are (nnr_cluster_tail_scores_packed)"""
+    check(lib.nnr_cluster_tail_scores_packed(_p(Kp, _F32), _p(g, _F32), _p(Wg, _F32), _p(idx, _I64), _p(cmask, _U8),
+                                             _p(row_off, _I32), Qp.shape[0], _p(Qp, _F32), _p(qk2, _F32), _p(cand, _F32),
+                                             _p(bias, _F32), B, H, Au, D, C1, n_max, float(scale), _p(scores, _F32),
+                                             scores.stride(0), _stream()), 'nnr_cluster_tail_scores_packed')
+
+
 def rowdot_fwd(a, b, R, D, out):
     check(lib.nnr_rowdot_fwd(_p(a, _F32), _p(b, _F32), R, D, _p(out, _F32), _stream()), 'nnr_rowdot_fwd')
 
@@ -547,6 +557,9 @@ _SCHEMAS = {
     'cluster_tail_scores': ('(Tensor Kp, Tensor g, Tensor Wg, Tensor idx, Tensor cmask, Tensor Qp, Tensor qk2, Tensor cand, '
                             'Tensor bias, int B, int H, int Au, int D, int C1, int T, float scale, Tensor(a!) scores) -> ()',
                             cluster_tail_scores),
+    'cluster_tail_scores_packed': ('(Tensor Kp, Tensor g, Tensor Wg, Tensor idx, Tensor cmask, Tensor row_off, Tensor Qp, '
+                                   'Tensor qk2, Tensor cand, Tensor bias, int B, int H, int Au, int D, int C1, int n_max, '
+                                   'float scale, Tensor(a!) scores) -> ()', cluster_tail_scores_packed),
     'rowdot_fwd': ('(Tensor a, Tensor b, int R, int D, Tensor(a!) out) -> ()', rowdot_fwd),
     'rowdot_bwd': ('(Tensor dout, Tensor a, Tensor b, int R, int D, Tensor(a!) da, bool accumulate_a, Tensor(b!) db, bool accumulate_b) -> ()',
                    rowdot_bwd),

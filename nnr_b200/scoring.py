@@ -175,9 +175,20 @@ class CorpusScorer:
         return gathered[:nitems]
 
     @torch.no_grad()
-    def score(self, history_ids, history_len, candidate_ids, cuda_graph=True):
+    def score(self, history_ids, history_len, candidate_ids, cuda_graph=True, exact=True):
         """history_ids [B,H] (0-padded at the end), history_len [B], candidate_ids [B,n] -> scores [B,n].  Rank-local:
-        never a collective, also with a process group."""
+        never a collective, also with a process group.  Full shapes with B >= 64 replay one captured CUDA graph per shape.
+
+        ``exact=False`` scores every entry through the factored cluster tail (nnr_cluster_tail_scores_packed, each user's
+        n candidates as one list): the cluster affine is applied once per history row instead of to C + 1 cluster
+        features per (user, candidate) pair, and the candidate projections run once per candidate.  The scores are those
+        of the SUE formula, within a relative error of 1e-4 of ``exact=True`` (fp32 sums in another order), but not
+        bit-identical to it.  The call is deterministic.  The candidate ids must lie in [0, news_num) (ValueError before
+        any launch otherwise).  SUE_wo_HCA, whose user vector does not depend on the candidate, returns the
+        ``exact=True`` result bit for bit."""
+        if not exact:
+            cid, cnt = self._packed_inputs('score', candidate_ids, None)
+            return self._score_packed(history_ids, history_len, cid, cnt, cuda_graph)
         assert self.cache is not None, 'call encode_corpus() first'
         hid = torch.as_tensor(history_ids).to(self.dev).long()
         cid = torch.as_tensor(candidate_ids).to(self.dev).long()
@@ -186,6 +197,63 @@ class CorpusScorer:
             key = ('score', tuple(hid.shape), tuple(cid.shape), self.cache.data_ptr())
             return self._graphed(key, self._score_impl, (hid, hl, cid)).clone()
         return self._score_impl(hid, hl, cid)
+
+    def _packed_inputs(self, who, candidate_ids, candidate_count):
+        """the checks of score() / evaluate() with exact=False, once per call and before any launch: candidate_ids [I, n]
+        integers, candidate_count [I] in [0, n] (None: all n), the valid candidate ids in [0, news_num).  Returns
+        (candidate ids [I, n] int64, counts [I] int32) as given, on the device they came on."""
+        if self.cache is None:
+            raise RuntimeError('CorpusScorer.%s: call encode_corpus() first' % who)
+        cid = torch.as_tensor(candidate_ids)
+        if cid.dim() != 2 or cid.dtype.is_floating_point or cid.dtype == torch.bool:
+            raise ValueError('CorpusScorer.%s: candidate_ids must be a 2-D integer tensor, got %s of shape %s'
+                             % (who, cid.dtype, tuple(cid.shape)))
+        I, n = cid.shape
+        cnt = torch.full((I,), n, dtype=torch.int64) if candidate_count is None else torch.as_tensor(candidate_count)
+        if tuple(cnt.shape) != (I,) or cnt.dtype.is_floating_point or cnt.dtype == torch.bool:
+            raise ValueError('CorpusScorer.%s: candidate_count must be an integer tensor of shape [%d], got %s of shape %s'
+                             % (who, I, cnt.dtype, tuple(cnt.shape)))
+        if I and (int(cnt.min()) < 0 or int(cnt.max()) > n):
+            raise ValueError('CorpusScorer.%s: candidate_count must be in [0, %d], got [%d, %d]'
+                             % (who, n, int(cnt.min()), int(cnt.max())))
+        valid = torch.arange(n, device=cnt.device)[None, :] < cnt[:, None]
+        if bool(valid.any()):
+            cid_v = cid.to(cnt.device)
+            lo = int(torch.where(valid, cid_v, torch.zeros_like(cid_v)).min())
+            hi = int(torch.where(valid, cid_v, torch.zeros_like(cid_v)).max())
+            news_num = self.cache.shape[0]
+            if lo < 0 or hi >= news_num:
+                raise ValueError('CorpusScorer.%s: the valid candidate ids must be in [0, %d), got [%d, %d]'
+                                 % (who, news_num, lo, hi))
+        return cid.long(), cnt.to(torch.int32)
+
+    def _score_packed(self, history_ids, history_len, cid, cnt, cuda_graph):
+        """scores [B, n] of the first cnt[b] candidates of each row of cid [B, n] through the factored cluster tail (0 past
+        the counts); B >= 64 replays one captured graph per shape"""
+        hid = torch.as_tensor(history_ids).to(self.dev).long()
+        hl = torch.as_tensor(history_len).to(self.dev).to(torch.int32)
+        cid, cnt = cid.to(self.dev), cnt.to(self.dev)
+        if cid.numel() == 0:
+            return torch.zeros(cid.shape, device=self.dev)
+        if cuda_graph and hid.shape[0] >= 64:
+            key = ('score_factored', tuple(hid.shape), tuple(cid.shape), self.cache.data_ptr())
+            return self._graphed(key, self._score_packed_impl, (hid, hl, cid, cnt)).clone()
+        return self._score_packed_impl(hid, hl, cid, cnt)
+
+    def _score_packed_impl(self, hid, hl, cid, cnt):
+        """the candidates are packed back to back on the device (prefix sum of the counts; no host synchronisation): list b
+        is rows [row_off[b], row_off[b + 1]) of a [B * n, D] buffer whose rows past row_off[B] hold news 0 and are not
+        scored.  Padding entries of cid are never read."""
+        B, n = cid.shape
+        row_off = torch.zeros(B + 1, dtype=torch.int32, device=self.dev)
+        torch.cumsum(cnt, 0, dtype=torch.int32, out=row_off[1:])
+        j = torch.arange(n, device=self.dev)
+        # packed row of every valid entry; padding goes to a dump slot past the end
+        dest = torch.where(j[None, :] < cnt[:, None], row_off[:B, None].long() + j[None, :], B * n)
+        ids = torch.zeros(B * n + 1, dtype=torch.int64, device=self.dev).scatter_(0, dest.view(-1), cid.reshape(-1))[:B * n]
+        ue = self.model.user_encoder
+        side = ue.user_side(self.cache[hid], *self._history_graph(hid, hl), factored=True)
+        return ue.packed_scores_factored(side, self.cache[ids], row_off, torch.zeros(B, n, device=self.dev))
 
     def _category_num(self):
         ue = self.model.user_encoder
@@ -435,33 +503,70 @@ class CorpusScorer:
         return self._merge_rank_lists(gathered[0], gathered[1], gathered[2] if m is not None else None, m, groups)
 
     @torch.no_grad()
-    def _impression_scores(self, history_ids, history_len, candidate_ids, batch, candidate_count=None, labels=None):
+    def _impression_scores(self, history_ids, history_len, candidate_ids, batch, candidate_count=None, labels=None,
+                           exact=True):
         """scores [I, n_max] of impressions batched as [a, a + batch) from 0.  With a process group: a collective; each rank
-        scores its contiguous share of the batches and every rank returns the whole matrix."""
+        scores its contiguous share of the batches and every rank returns the whole matrix.  ``exact=False``: only the
+        first candidate_count[i] entries of each row are scored, through the factored cluster tail (0 past them)."""
         cid = torch.as_tensor(candidate_ids)
-        if self.group is None:
-            out = []
-            for a in range(0, cid.shape[0], batch):
-                out.append(self.score(history_ids[a:a + batch], history_len[a:a + batch], cid[a:a + batch]))
-            return torch.cat(out)
+        err = None
+        if not exact:
+            try:
+                cid, cnt = self._packed_inputs('evaluate', cid, candidate_count)
+            except (ValueError, RuntimeError) as e:
+                if self.group is None:
+                    raise
+                err = e                                  # raised after the agreement, so that no rank waits in a collective
 
-        assert self.cache is not None, 'call encode_corpus() first'
-        I, n_max = cid.shape
-        ids = dict(history_ids=history_ids, history_len=history_len, candidate_ids=cid, candidate_count=candidate_count, labels=labels)
-        sums = {k + ' checksum': int(_checksum(torch.as_tensor(v).to(self.dev))) for k, v in ids.items() if v is not None}
-        self._agree(2, **self._corpus_fields(), **{'corpus ids checksum': self._corpus_sum}, I=I, n_max=n_max,
-                    H=torch.as_tensor(history_ids).shape[1], batch=batch, **sums)
-        return self._sharded(I, batch, n_max,
-                             lambda a: self.score(history_ids[a:a + batch], history_len[a:a + batch], cid[a:a + batch]))
+        def scores(a):
+            if exact:
+                return self.score(history_ids[a:a + batch], history_len[a:a + batch], cid[a:a + batch])
+            return self._score_packed(history_ids[a:a + batch], history_len[a:a + batch], cid[a:a + batch],
+                                      cnt[a:a + batch], True)
+
+        if self.group is None:
+            return torch.cat([scores(a) for a in range(0, cid.shape[0], batch)])
+
+        fields = {'exact': int(bool(exact)), 'argument error': int(err is not None)}
+        if err is None:
+            assert self.cache is not None, 'call encode_corpus() first'
+            ids = dict(history_ids=history_ids, history_len=history_len, candidate_ids=cid, candidate_count=candidate_count,
+                       labels=labels)
+            fields.update({k + ' checksum': int(_checksum(torch.as_tensor(v).to(self.dev))) for k, v in ids.items()
+                           if v is not None})
+            fields.update(I=cid.shape[0], n_max=cid.shape[1], H=torch.as_tensor(history_ids).shape[1], batch=batch)
+        try:
+            self._agree(2, **self._corpus_fields(), **{'corpus ids checksum': self._corpus_sum or 0}, **fields)
+        except RuntimeError as e:
+            if err is not None:
+                raise RuntimeError('%s On this rank: %s' % (e, err)) from err
+            raise
+        if err is not None:
+            raise err
+        return self._sharded(cid.shape[0], batch, cid.shape[1], scores)
 
     @torch.no_grad()
-    def evaluate(self, history_ids, history_len, candidate_ids, candidate_count, labels, batch=256):
+    def evaluate(self, history_ids, history_len, candidate_ids, candidate_count, labels, batch=256, exact=True):
         """Dev-set metrics with the cached corpus and on-device ranking (SURVEY 8f-2; replaces util.compute_scores +
         evaluate.scoring): impressions are padded to [I, n_max] candidate ids with ``candidate_count`` valid entries
         and 0/1 ``labels``.  Returns (auc, mrr, ndcg5, ndcg10, ranks [I, n_max]).  With a process group: a collective;
         the impression batches are shared out between the ranks, the scores all-gathered, and every rank ranks the whole
-        matrix and returns the same metrics as one GPU."""
-        scores = self._impression_scores(history_ids, history_len, candidate_ids, batch, candidate_count, labels)
+        matrix and returns the same metrics as one GPU.
+
+        ``exact=False`` scores each batch of ``batch`` impressions through the factored cluster tail
+        (nnr_cluster_tail_scores_packed): only the first candidate_count[i] candidates of each impression are scored,
+        packed back to back on the device, so the work follows the sum of the counts instead of I * n_max, and the cluster
+        affine is applied once per history row instead of once per (impression, candidate) cluster feature.  Padding
+        entries are never read: their ids may be anything, -1 for instance.  The scores are those of the SUE formula,
+        within a relative error of 1e-4 of ``exact=True`` (fp32 sums in another order), but not bit-identical to it, so
+        ranks of candidates whose scores lie that close may differ between the two, and with them the metrics.  The ranks
+        and metrics are computed from these scores as above, and the call is deterministic.  candidate_count must have
+        shape [I] with values in [0, n_max], and the valid candidate ids must lie in [0, news_num): ValueError, checked
+        once per call before any launch (with a process group, after the ranks' argument agreement, which includes
+        ``exact``; the sharded result equals the plain ``exact=False`` call bit for bit).  Full batches replay one
+        captured CUDA graph per (batch, H, n_max).  SUE_wo_HCA, whose user vector does not depend on the candidate,
+        returns the ``exact=True`` scores of the valid entries bit for bit."""
+        scores = self._impression_scores(history_ids, history_len, candidate_ids, batch, candidate_count, labels, exact)
         cnt = torch.as_tensor(candidate_count).to(self.dev)
         lab = torch.as_tensor(labels).to(self.dev)
         ranks, _ = metrics.rank_impressions(scores, cnt)

@@ -108,3 +108,10 @@ class SUE(UserEncoder):
         factored cluster tail: equal to tile_scores on the expanded candidates in real arithmetic, not bit for bit
         (engine.sue_tile_scores_factored)"""
         return engine.sue_tile_scores_factored(self._meta(), user_side, candidate_rows, *self._params())
+
+    def packed_scores_factored(self, user_side, candidate_rows, row_off, out):
+        """click scores of per-user candidate lists for the users of ``user_side(..., factored=True)``: user b's candidates
+        are candidate_rows [row_off[b], row_off[b + 1]) (row_off [B + 1] int32 on the device), the score of its j-th goes
+        to out[b, j] and the rest of out is left as it is; returns out.  The factored cluster tail, as in
+        tile_scores_factored (engine.sue_packed_scores_factored)"""
+        return engine.sue_packed_scores_factored(self._meta(), user_side, candidate_rows, row_off, out, *self._params())

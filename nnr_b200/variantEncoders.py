@@ -40,7 +40,7 @@ class SUE_wo_GCN(UserEncoder):
     forward = SUE.forward
     encode_user = SUE.encode_user
     _meta, user_side, tile_scores = SUE._meta, SUE.user_side, SUE.tile_scores
-    tile_scores_factored = SUE.tile_scores_factored
+    tile_scores_factored, packed_scores_factored = SUE.tile_scores_factored, SUE.packed_scores_factored
 
     def __init__(self, news_encoder, config):
         super().__init__(news_encoder, config)
@@ -76,7 +76,7 @@ class SUE_wo_HCA(UserEncoder):
     forward = SUE.forward
     encode_user = SUE.encode_user
     _meta, user_side, tile_scores = SUE._meta, SUE.user_side, SUE.tile_scores
-    tile_scores_factored = SUE.tile_scores_factored
+    tile_scores_factored, packed_scores_factored = SUE.tile_scores_factored, SUE.packed_scores_factored
 
     def __init__(self, news_encoder, config):
         super().__init__(news_encoder, config)
