@@ -1,4 +1,6 @@
 """GPU tests of the tcgen05 (3xTF32 / BF16) GEMM backend against fp64 torch and the exact-fp32 FFMA backend."""
+import ctypes
+
 import pytest
 import torch
 
@@ -176,6 +178,103 @@ def test_cta_pair_tiles_large_m(cuda, algo_name):
     gref = torch.sigmoid(A[:Mv].double() @ W.double().t() + rb.double()[rmap[:Mv].long()])
     assert (gate[:Mv].double() - gref).abs().max().item() < 2e-5
     assert (C[:Mv].double() - gref * A[:Mv].double()).abs().max().item() < 1e-4
+
+
+# The kernel paths that finish a default-algorithm (bf16x3) GEMM's epilogue, each with an NT shape that make_plan
+# (gemm_tc.cu) sends there.  ldc > N where the path allows it, so a column index taken from ldc instead of N shows.
+EPI_PATHS = {
+    # N % 4 == 0, 16-byte aligned operands, 34 x 7 = 238 tiles (more than 74: no split-K): the compile-time epilogue of the
+    # single-CTA kernel; block_n 144 leaves a 36-column N tail
+    'single': dict(M=4352, N=900, K=900, ldc=904),
+    # M >= 2 * 128 * 148 = 37 888, A row-major, no k_dev: 256-row tiles on CTA pairs (compile-time epilogue); the device-side
+    # row count ends inside a tile
+    'pair': dict(M=40000, N=900, K=900, ldc=904, m_dev=38211),
+    # tiles * 2 <= 148 and ceil(K / 64) = 15 >= 8: split-K partials, combined with the epilogue by tc_splitk_reduce4_kernel
+    # (N % 4 == 0)
+    'splitk4_m64': dict(M=64, N=900, K=900, ldc=904, splits=4),
+    'splitk4_m640': dict(M=640, N=900, K=900, ldc=904, splits=4),
+    # split-K with N % 4 != 0: the scalar tc_splitk_reduce_kernel
+    'splitk_scalar': dict(M=320, N=225, K=900, ldc=225, splits=4),
+    # N % 4 != 0 and 79 x 2 = 158 tiles (no split): the run-time-switched epilogue
+    'runtime_n225': dict(M=10000, N=225, K=900, ldc=225),
+    # leading dimensions of 901 floats (rows not 16-byte aligned): the run-time-switched epilogue at N % 4 == 0
+    'runtime_ld901': dict(M=4352, N=900, K=900, ldc=901, ld=901),
+}
+
+
+def _gemm_workspace_bytes(A, B, C, M, N, K, ldc):
+    from nnr_b200 import _lib, ops
+    a = _lib.GemmArgs()
+    a.A, a.lda, a.B, a.ldb, a.transB, a.C, a.ldc = A.data_ptr(), K, B.data_ptr(), K, 1, C.data_ptr(), ldc
+    a.M, a.N, a.K, a.algo = M, N, K, ops.ALGO_AUTO
+    return int(_lib.lib.nnr_gemm_workspace_bytes(ctypes.byref(a)))
+
+
+@pytest.mark.parametrize('path', list(EPI_PATHS))
+def test_default_epilogues_on_each_kernel_path(cuda, path):
+    """every epilogue of the default algorithm against fp64 on each kernel path that can finish it: values, rows >= m_dev
+    and columns [N, ldc) left untouched, and a repeated call bit-identical"""
+    from nnr_b200 import ops
+    from tests import dropout_ref
+    if ops.default_algo() != ops.ALGO_BF16X3:
+        pytest.skip('paths and tolerances of the bf16x3 default')
+    c = EPI_PATHS[path]
+    M, N, K, ldc = c['M'], c['N'], c['K'], c['ldc']
+    ld = c.get('ld', ldc)
+    Mv = c.get('m_dev', M)
+    m_dev = torch.tensor([Mv], dtype=torch.int32, device=cuda) if 'm_dev' in c else None
+    g = torch.Generator().manual_seed(M + N + ldc)
+    A = torch.randn(M, K, generator=g).to(cuda)
+    W = (torch.randn(N, K, generator=g) / 80).to(cuda)          # |A W^T| ~ 0.4: tanh / sigmoid are not saturated
+    bias = torch.randn(N, generator=g).to(cuda)
+    aux = torch.randn(M, ld, generator=g).to(cuda)
+    rowmap = torch.randint(0, 37, (M,), generator=g, dtype=torch.int32).to(cuda)
+    rowbias = torch.randn(37, ld, generator=g).to(cuda)
+    base = torch.randn(M, ldc, generator=g).to(cuda)
+    if 'splits' in c:                                          # the partial sums really are split: [splits][M][N] fp32
+        C0 = torch.empty(M, ldc, device=cuda)
+        planes = sum((rows * ((K + 7) // 8 * 8) * 4 + 1023) // 1024 * 1024 for rows in (M, N))
+        assert _gemm_workspace_bytes(A, W, C0, M, N, K, ldc) - planes == (c['splits'] * M * N * 4 + 1023) // 1024 * 1024
+    prod = A[:Mv].double() @ W.double().t()
+    z = prod + bias.double()
+    zmax = z.abs().max().item()
+    ax = aux[:Mv, :N].double()
+    s = torch.from_numpy(dropout_ref.keep_scale_grid(77, Mv, N, 0.25)).to(cuda).double()
+    rb = rowbias.double()[rowmap[:Mv].long(), :N]
+    sig = torch.sigmoid(prod + rb)
+    # (name, kwargs, fp64 reference of C, absolute tolerance of C, reference of aux_out or None)
+    cases = [('bias', dict(epilogue=ops.EPI_BIAS, bias=bias), z, 4e-5 * zmax, None),
+             ('bias_tanh', dict(epilogue=ops.EPI_BIAS_TANH, bias=bias), torch.tanh(z), 2e-5, None),
+             ('relu', dict(epilogue=ops.EPI_BIAS_RELU_RES, bias=bias), torch.relu(z), 4e-5 * zmax, None),
+             ('relu_res', dict(epilogue=ops.EPI_BIAS_RELU_RES, bias=bias, aux=aux, ldaux=ld), torch.relu(z) + ax,
+              4e-5 * zmax, torch.relu(z)),
+             ('relu_res_drop', dict(epilogue=ops.EPI_BIAS_RELU_RES, bias=bias, aux=aux, ldaux=ld, p_drop=0.25, seed=77),
+              (torch.relu(z) + ax) * s, 4e-5 * zmax * 4 / 3, torch.relu(z)),
+             ('gate', dict(epilogue=ops.EPI_GATE, rowbias=rowbias, ldrowbias=ld, rowmap=rowmap, aux=aux, ldaux=ld), sig * ax,
+              2e-5 * ax.abs().max().item(), sig),
+             ('add_aux', dict(epilogue=ops.EPI_ADD_AUX, aux=aux, ldaux=ld), prod + ax, 4e-5 * zmax, None),
+             ('accumulate', dict(epilogue=ops.EPI_NONE, accumulate=True), prod + base[:Mv, :N].double(), 4e-5 * zmax, None)]
+    for name, kw, ref, tol, ao_ref in cases:
+        outs = []
+        for _ in range(2):
+            C = base.clone() if kw.get('accumulate') else torch.full((M, ldc), float('nan'), device=cuda)
+            ao = torch.full((M, ld), float('nan'), device=cuda) if ao_ref is not None else None
+            extra = dict(aux_out=ao, ldaux_out=ld) if ao is not None else {}
+            ops.gemm(A, W, C, M, N, K, K, K, ldc, False, True, m_dev=m_dev, **kw, **extra)
+            outs.append((C, ao))
+        C, ao = outs[0]
+        err = (C[:Mv, :N].double() - ref).abs().max().item()
+        assert err < tol, (path, name, err, tol)
+        if kw.get('accumulate'):
+            assert torch.equal(C[Mv:], base[Mv:]) and torch.equal(C[:, N:], base[:, N:]), (path, name)
+        else:
+            assert torch.isnan(C[Mv:]).all() and torch.isnan(C[:, N:]).all(), (path, name)
+        assert torch.equal(outs[1][0][:Mv, :N], C[:Mv, :N]), (path, name)
+        if ao_ref is not None:
+            err = (ao[:Mv, :N].double() - ao_ref).abs().max().item()
+            assert err < (2e-5 if name == 'gate' else 4e-5 * zmax), (path, name, err)
+            assert torch.isnan(ao[Mv:]).all() and torch.isnan(ao[:, N:]).all(), (path, name)
+            assert torch.equal(outs[1][1][:Mv, :N], ao[:Mv, :N]), (path, name)
 
 
 @pytest.mark.parametrize('cols', [1600, 200, 300, 96])
