@@ -33,7 +33,7 @@
 extern "C" {
 #endif
 
-#define NNR_ABI_VERSION 10
+#define NNR_ABI_VERSION 11
 #define NNR_SEED_INDIRECT (1ULL << 62)
 
 const char* nnr_last_error(void);
@@ -354,6 +354,20 @@ int nnr_cluster_tail_scores_packed(const float* Kp, const float* g, const float*
                                    const uint8_t* cmask, const int32_t* row_off, int64_t rows, const float* Qp,
                                    const float* qk2, const float* cand, const float* bias, int B, int H, int Au, int D,
                                    int C1, int n_max, float scale, float* scores, int64_t lds, void* stream);
+/* nnr_cluster_tail_scores_packed that also explains every score it writes (scoring.CorpusScorer.explain(exact=False)):
+ * for user b's j-th candidate (t = b*lds + j, j below its count)
+ *   alpha_out[t*H + h]     = alpha[b,j,h], slot h's weight in its cluster's softmax (history order; sums to 1 over the
+ *                            slots of each non-empty cluster)
+ *   beta_out[t*C1 + c]     = beta[b,j,c] (exactly 0 for a masked cluster)
+ *   contrib_out[t*C1 + c]  = beta[b,j,c] * (f[b,j,c,:] . cand), whose sum over c is the score up to fp32 rounding
+ * The scores are those of nnr_cluster_tail_scores_packed on the same arguments, bit for bit.  Entries past a user's
+ * count are not written, in any of the four outputs.  The arguments, checks, error codes and limits are those of
+ * nnr_cluster_tail_scores_packed; alpha_out, beta_out and contrib_out must not be NULL either (NNR_ERR_ARG).         */
+int nnr_cluster_tail_explain_packed(const float* Kp, const float* g, const float* Wg, const int64_t* idx,
+                                    const uint8_t* cmask, const int32_t* row_off, int64_t rows, const float* Qp,
+                                    const float* qk2, const float* cand, const float* bias, int B, int H, int Au, int D,
+                                    int C1, int n_max, float scale, float* scores, int64_t lds, float* alpha_out,
+                                    float* beta_out, float* contrib_out, void* stream);
 
 /* ---- click predictor: model.py:127 ---------------------------------------------------------- */
 int nnr_rowdot_fwd(const float* a, const float* b, int R, int D, float* out, void* stream);

@@ -116,6 +116,8 @@ SIGNATURES = {
                                           C.c_int, f32, vp, i64, vp]),
     'nnr_cluster_tail_scores_packed': (C.c_int, [vp, vp, vp, vp, vp, vp, i64, vp, vp, vp, vp, C.c_int, C.c_int, C.c_int,
                                                  C.c_int, C.c_int, C.c_int, f32, vp, i64, vp]),
+    'nnr_cluster_tail_explain_packed': (C.c_int, [vp, vp, vp, vp, vp, vp, i64, vp, vp, vp, vp, C.c_int, C.c_int, C.c_int,
+                                                  C.c_int, C.c_int, C.c_int, f32, vp, i64, vp, vp, vp, vp]),
     'nnr_rowdot_fwd': (C.c_int, [vp, vp, C.c_int, C.c_int, vp, vp]),
     'nnr_rowdot_bwd': (C.c_int, [vp, vp, vp, C.c_int, C.c_int, vp, C.c_int, vp, C.c_int, vp]),
     'nnr_topk_merge': (C.c_int, [vp, i64, C.c_int, C.c_int, i64, vp, vp, vp, C.c_int, C.c_int, C.c_int, vp, vp, vp]),

@@ -23,6 +23,10 @@
 // stored back to back, one CTA per (user, slice of TAIL_PC candidates).  A MIND list has ~37 candidates, too few to hide
 // the latency of phase 4's loads with one warp, so W warps split the slots, the clusters and the feature steps, and the
 // partial dots of a round of W steps are added in step order: the scores equal the pool kernel's bit for bit.
+//
+// nnr_cluster_tail_explain_packed (CorpusScorer.explain(exact=False)) is the packed kernel with EX = true: phase 3 also
+// stores each slot's alpha at its history position, phase 5 each cluster's beta and beta * (f . cand).  The score is
+// summed by the same instructions, so it equals the packed kernel's bit for bit.
 #include "common.cuh"
 #include "../../include/nnr_b200.h"
 
@@ -128,13 +132,19 @@ __device__ __forceinline__ void tail_step(int d0, const float* __restrict__ gb, 
 // kernel): one thread does all of a candidate's work, and phases 3-5 need no barrier.  W > 1: the W groups take turns
 // over the feature steps; the W partial dots of a round are stored in s_part and added to the running sums in step
 // order, so every sum runs in the order of W = 1.
-template <int CS, int W>
+// EX: candidate t's alpha goes to ex.alpha[t * H + h] (h: the slot's history position), its beta and beta * (f . cand)
+// to ex.beta[t * C1 + c] and ex.contrib[t * C1 + c].
+// One struct parameter rather than three pointers: with three, even unused, ptxas allocates the EX = false kernels'
+// registers differently.
+struct TailEx { float* alpha; float* beta; float* contrib; };
+
+template <int CS, int W, bool EX = false>
 __device__ __forceinline__ void tail_cta(const float* __restrict__ Kp, const float* __restrict__ g,
                                          const float* __restrict__ Wg, const int64_t* __restrict__ idx,
                                          const uint8_t* __restrict__ cmask, const float* __restrict__ Qp,
                                          const float* __restrict__ qk2, const float* __restrict__ cand,
                                          const float* __restrict__ bias, int b, int H, int Au, int D, int C1, int T, int t0,
-                                         float scale, float* __restrict__ srow) {
+                                         float scale, float* __restrict__ srow, TailEx ex = {}) {
   constexpr int NT = CS * W, TC = CS * TAIL_TT;
   extern __shared__ __align__(16) float sm[];
   float* s_al = sm;                                   // [H][TC]: logits, then alpha (slots in cluster order)
@@ -219,7 +229,11 @@ __device__ __forceinline__ void tail_cta(const float* __restrict__ Kp, const flo
       for (int e = lo; e < hi; ++e) m = fmaxf(m, col_j[e * TC]);
       float sum = 0.f;
       for (int e = lo; e < hi; ++e) sum += expf(col_j[e * TC] - m);
-      for (int e = lo; e < hi; ++e) col_j[e * TC] = expf(col_j[e * TC] - m) / sum;
+      for (int e = lo; e < hi; ++e) {
+        col_j[e * TC] = expf(col_j[e * TC] - m) / sum;
+        if constexpr (EX)
+          if (t0 + col + j * CS < T) ex.alpha[(size_t)(t0 + col + j * CS) * H + s_perm[e]] = col_j[e * TC];
+      }
     }
     for (int c = grp; c < C1; c += W) s_acc[c * TC + col + j * CS] = s_acc[(C1 + c) * TC + col + j * CS] = 0.f;
   }
@@ -289,7 +303,12 @@ __device__ __forceinline__ void tail_cta(const float* __restrict__ Kp, const flo
     for (int c = 0; c < C1; ++c) {
       const bool full = s_start[c] < s_start[c + 1];
       const float l = cm[c] ? scale * (full ? s_acc[c * TC + tl] : eq[j]) : -1e9f;
-      out = fmaf(expf(l - m) * inv, full ? s_acc[(C1 + c) * TC + tl] : ec[j], out);
+      const float beta = expf(l - m) * inv, dot = full ? s_acc[(C1 + c) * TC + tl] : ec[j];
+      out = fmaf(beta, dot, out);
+      if constexpr (EX) {
+        ex.beta[(size_t)(t0 + tl) * C1 + c] = beta;
+        ex.contrib[(size_t)(t0 + tl) * C1 + c] = beta * dot;
+      }
     }
     srow[t0 + tl] = out;
   }
@@ -309,19 +328,27 @@ __global__ void __launch_bounds__(NT) cluster_tail_scores_kernel(
 // packed candidate lists: CTA x = (user b, slice s) of ns slices of TAIL_PC candidates, W warps; user b's candidates are
 // rows [row_off[b], row_off[b + 1]) of Qp / qk2 / cand.  The offsets come from the device unchecked: the count is clamped
 // to [0, n_max] and the rows to [0, rows), and a CTA whose slice starts past the count exits before it reads anything else.
-template <int W>
+// EX: also the explanation of every score, [B, lds, H] alpha_out and [B, lds, C1] beta_out / contrib_out (tail_cta).
+template <int W, bool EX>
 __global__ void __launch_bounds__(32 * W) cluster_tail_scores_packed_kernel(
     const float* __restrict__ Kp, const float* __restrict__ g, const float* __restrict__ Wg, const int64_t* __restrict__ idx,
     const uint8_t* __restrict__ cmask, const int32_t* __restrict__ row_off, int64_t rows, const float* __restrict__ Qp,
     const float* __restrict__ qk2, const float* __restrict__ cand, const float* __restrict__ bias, int ns, int H, int Au,
-    int D, int C1, int n_max, float scale, float* __restrict__ scores, int64_t lds) {
+    int D, int C1, int n_max, float scale, float* __restrict__ scores, int64_t lds, float* __restrict__ alpha_out,
+    float* __restrict__ beta_out, float* __restrict__ contrib_out) {
   const int b = blockIdx.x / ns, t0 = (blockIdx.x % ns) * TAIL_PC;
   const int64_t lo = min(max((int64_t)row_off[b], (int64_t)0), rows);
   const int64_t hi = min(max((int64_t)row_off[b + 1], lo), rows);
   const int T = (int)min(hi - lo, (int64_t)n_max);
   if (t0 >= T) return;
-  tail_cta<32, W>(Kp, g, Wg, idx, cmask, Qp + lo * Au, qk2 + lo * D, cand + lo * D, bias, b, H, Au, D, C1, T, t0, scale,
-                  scores + (size_t)b * lds);
+  if constexpr (EX)
+    tail_cta<32, W, true>(Kp, g, Wg, idx, cmask, Qp + lo * Au, qk2 + lo * D, cand + lo * D, bias, b, H, Au, D, C1, T, t0,
+                          scale, scores + (size_t)b * lds,
+                          TailEx{alpha_out + (size_t)b * lds * H, beta_out + (size_t)b * lds * C1,
+                                 contrib_out + (size_t)b * lds * C1});
+  else
+    tail_cta<32, W>(Kp, g, Wg, idx, cmask, Qp + lo * Au, qk2 + lo * D, cand + lo * D, bias, b, H, Au, D, C1, T, t0, scale,
+                    scores + (size_t)b * lds);
 }
 
 // dynamic shared memory of a CTA of TC candidates: the logits / alpha and the larger of the accumulators and the staging
@@ -384,28 +411,29 @@ extern "C" int nnr_cluster_tail_scores(const float* Kp, const float* g, const fl
                          tail_smem(H, C1, 64 * TAIL_TT), tail_smem(TAIL_MAXH, TAIL_MAXC, 64 * TAIL_TT), stream);
 }
 
-template <int W>
+template <int W, bool EX>
 static int tail_packed_launch(const float* Kp, const float* g, const float* Wg, const int64_t* idx, const uint8_t* cmask,
                               const int32_t* row_off, int64_t rows, const float* Qp, const float* qk2, const float* cand,
                               const float* bias, int B, int H, int Au, int D, int C1, int n_max, float scale, float* scores,
-                              int64_t lds, size_t smem, size_t most, void* stream) {
+                              int64_t lds, float* alpha_out, float* beta_out, float* contrib_out, size_t smem, size_t most,
+                              void* stream) {
   static bool attr_set[64] = {};
-  if (int rc = tail_smem_attr((const void*)cluster_tail_scores_packed_kernel<W>, most, attr_set)) return rc;
+  if (int rc = tail_smem_attr((const void*)cluster_tail_scores_packed_kernel<W, EX>, most, attr_set)) return rc;
   const int ns = (n_max + TAIL_PC - 1) / TAIL_PC;
-  cluster_tail_scores_packed_kernel<W><<<(unsigned)((int64_t)B * ns), 32 * W, smem, (cudaStream_t)stream>>>(
-      Kp, g, Wg, idx, cmask, row_off, rows, Qp, qk2, cand, bias, ns, H, Au, D, C1, n_max, scale, scores, lds);
-  NNR_LAUNCH_CHECK(W == 8 ? "cluster_tail_scores_packed_kernel<8>" : "cluster_tail_scores_packed_kernel<2>");
+  cluster_tail_scores_packed_kernel<W, EX><<<(unsigned)((int64_t)B * ns), 32 * W, smem, (cudaStream_t)stream>>>(
+      Kp, g, Wg, idx, cmask, row_off, rows, Qp, qk2, cand, bias, ns, H, Au, D, C1, n_max, scale, scores, lds, alpha_out,
+      beta_out, contrib_out);
+  NNR_LAUNCH_CHECK(EX ? (W == 8 ? "cluster_tail_scores_packed_kernel<8, explain>" : "cluster_tail_scores_packed_kernel<2, explain>")
+                      : (W == 8 ? "cluster_tail_scores_packed_kernel<8>" : "cluster_tail_scores_packed_kernel<2>"));
   return 0;
 }
 
-extern "C" int nnr_cluster_tail_scores_packed(const float* Kp, const float* g, const float* Wg, const int64_t* idx,
-                                              const uint8_t* cmask, const int32_t* row_off, int64_t rows, const float* Qp,
-                                              const float* qk2, const float* cand, const float* bias, int B, int H, int Au,
-                                              int D, int C1, int n_max, float scale, float* scores, int64_t lds,
-                                              void* stream) {
-  const char* who = "nnr_cluster_tail_scores_packed";
-  NNR_REQUIRE(Kp && g && Wg && idx && cmask && row_off && Qp && qk2 && cand && bias && scores, NNR_ERR_ARG,
-              "%s: Kp, g, Wg, idx, cmask, row_off, Qp, qk2, cand, bias and scores must not be NULL", who);
+// the checks and the launch of nnr_cluster_tail_scores_packed / nnr_cluster_tail_explain_packed (EX), past the NULL checks
+template <bool EX>
+static int tail_packed(const char* who, const float* Kp, const float* g, const float* Wg, const int64_t* idx,
+                       const uint8_t* cmask, const int32_t* row_off, int64_t rows, const float* Qp, const float* qk2,
+                       const float* cand, const float* bias, int B, int H, int Au, int D, int C1, int n_max, float scale,
+                       float* scores, int64_t lds, float* alpha_out, float* beta_out, float* contrib_out, void* stream) {
   NNR_REQUIRE(B >= 0 && H >= 1 && Au >= 1 && D >= 1 && C1 >= 1, NNR_ERR_ARG,
               "%s: bad sizes B=%d H=%d Au=%d D=%d C1=%d (B >= 0, the others >= 1)", who, B, H, Au, D, C1);
   NNR_REQUIRE(n_max >= 1 && n_max <= lds, NNR_ERR_ARG, "%s: n_max must be in [1, lds = %lld], got %d", who, (long long)lds,
@@ -423,8 +451,36 @@ extern "C" int nnr_cluster_tail_scores_packed(const float* Kp, const float* g, c
   // 8 warps when two CTAs fit on an SM (the default H = 50, C1 = 19 needs 98 KB), 2 otherwise (176 KB at H = 256, C1 = 72)
   const size_t wide = tail_smem(H, C1, TAIL_PC, 8);
   if (wide <= TAIL_SMEM_PAIR)
-    return tail_packed_launch<8>(Kp, g, Wg, idx, cmask, row_off, rows, Qp, qk2, cand, bias, B, H, Au, D, C1, n_max, scale,
-                                 scores, lds, wide, TAIL_SMEM_PAIR, stream);
-  return tail_packed_launch<2>(Kp, g, Wg, idx, cmask, row_off, rows, Qp, qk2, cand, bias, B, H, Au, D, C1, n_max, scale,
-                               scores, lds, tail_smem(H, C1, TAIL_PC, 2), tail_smem(TAIL_MAXH, TAIL_MAXC, TAIL_PC, 2), stream);
+    return tail_packed_launch<8, EX>(Kp, g, Wg, idx, cmask, row_off, rows, Qp, qk2, cand, bias, B, H, Au, D, C1, n_max,
+                                     scale, scores, lds, alpha_out, beta_out, contrib_out, wide, TAIL_SMEM_PAIR, stream);
+  return tail_packed_launch<2, EX>(Kp, g, Wg, idx, cmask, row_off, rows, Qp, qk2, cand, bias, B, H, Au, D, C1, n_max, scale,
+                                   scores, lds, alpha_out, beta_out, contrib_out, tail_smem(H, C1, TAIL_PC, 2),
+                                   tail_smem(TAIL_MAXH, TAIL_MAXC, TAIL_PC, 2), stream);
+}
+
+extern "C" int nnr_cluster_tail_scores_packed(const float* Kp, const float* g, const float* Wg, const int64_t* idx,
+                                              const uint8_t* cmask, const int32_t* row_off, int64_t rows, const float* Qp,
+                                              const float* qk2, const float* cand, const float* bias, int B, int H, int Au,
+                                              int D, int C1, int n_max, float scale, float* scores, int64_t lds,
+                                              void* stream) {
+  const char* who = "nnr_cluster_tail_scores_packed";
+  NNR_REQUIRE(Kp && g && Wg && idx && cmask && row_off && Qp && qk2 && cand && bias && scores, NNR_ERR_ARG,
+              "%s: Kp, g, Wg, idx, cmask, row_off, Qp, qk2, cand, bias and scores must not be NULL", who);
+  return tail_packed<false>(who, Kp, g, Wg, idx, cmask, row_off, rows, Qp, qk2, cand, bias, B, H, Au, D, C1, n_max, scale,
+                            scores, lds, nullptr, nullptr, nullptr, stream);
+}
+
+extern "C" int nnr_cluster_tail_explain_packed(const float* Kp, const float* g, const float* Wg, const int64_t* idx,
+                                               const uint8_t* cmask, const int32_t* row_off, int64_t rows, const float* Qp,
+                                               const float* qk2, const float* cand, const float* bias, int B, int H, int Au,
+                                               int D, int C1, int n_max, float scale, float* scores, int64_t lds,
+                                               float* alpha_out, float* beta_out, float* contrib_out, void* stream) {
+  const char* who = "nnr_cluster_tail_explain_packed";
+  NNR_REQUIRE(Kp && g && Wg && idx && cmask && row_off && Qp && qk2 && cand && bias && scores && alpha_out && beta_out &&
+                  contrib_out,
+              NNR_ERR_ARG,
+              "%s: Kp, g, Wg, idx, cmask, row_off, Qp, qk2, cand, bias, scores, alpha_out, beta_out and contrib_out must "
+              "not be NULL", who);
+  return tail_packed<true>(who, Kp, g, Wg, idx, cmask, row_off, rows, Qp, qk2, cand, bias, B, H, Au, D, C1, n_max, scale,
+                           scores, lds, alpha_out, beta_out, contrib_out, stream);
 }

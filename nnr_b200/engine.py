@@ -1083,9 +1083,9 @@ class RowDot(torch.autograd.Function):
 @torch.no_grad()
 def sue_user_side(meta, hist, graph, cmask, cidx, *params, factored=False):
     """the history half of SUEFunction.forward for the users of hist [B, H, D]: returns the tuple of tensors
-    ``sue_tile_scores`` takes -- (gfeat, Kp, cmask, cidx) with the hierarchical cluster attention, (pooled user vector,)
-    for SUE_wo_HCA.  ``factored``: the cluster attention's tuple also carries Wg = gfeat clusterFeatureAffine.weight^T
-    [B, H, D] (no bias), for ``sue_tile_scores_factored``"""
+    ``sue_tile_scores`` takes -- (gfeat, Kp, cmask, cidx) with the hierarchical cluster attention, (pooled user vector
+    [B, D], its attention weights over the history [B, H]) for SUE_wo_HCA.  ``factored``: the cluster attention's tuple
+    also carries Wg = gfeat clusterFeatureAffine.weight^T [B, H, D] (no bias), for ``sue_tile_scores_factored``"""
     assert not meta['training'], 'the split SUE forward is for inference (eval mode)'
     P = dict(zip(sue_names(meta), params))
     gcn = meta.get('gcn', True)
@@ -1093,7 +1093,8 @@ def sue_user_side(meta, hist, graph, cmask, cidx, *params, factored=False):
     hist = hist.contiguous()
     gfeat = SUEFunction._gcn(meta, P, hist, graph, [0] * (L + 2), L, 0.0)[0] if gcn else hist
     if not meta['hca']:
-        return (SUEFunction._history_pool(P, gfeat)[0],)
+        pooled, _, alpha = SUEFunction._history_pool(P, gfeat)
+        return pooled, alpha.view(gfeat.shape[0], gfeat.shape[1])
     gfeat_pl, Kp = SUEFunction._user_keys(P, gfeat)
     if not factored:
         return gfeat, Kp, cmask, cidx.contiguous()
@@ -1106,19 +1107,46 @@ def sue_user_side(meta, hist, graph, cmask, cidx, *params, factored=False):
 def sue_tile_scores(meta, side, cand, *params):
     """click scores [B, T] of the candidates cand [B, T, D] for the users of ``side`` (from ``sue_user_side``): the
     candidate tail of SUEFunction.forward and the dot product (model.py:127)"""
-    P = dict(zip(sue_names(meta), params))
-    B, T, D = cand.shape
+    T = cand.shape[1]
     cand = cand.contiguous()
     if not meta['hca']:
         return RowDot.apply(side[0].unsqueeze(1).repeat(1, T, 1), cand)
+    return RowDot.apply(_sue_tile_user(_Mod(), meta, side, cand, params), cand)
+
+
+def _sue_tile_user(ctx, meta, side, cand, params):
+    """the candidate tail of SUEFunction.forward with the cluster attention: user vectors [B, T, D] of the contiguous
+    candidates cand [B, T, D]; the forward's tensors are left in ctx.sv"""
+    P = dict(zip(sue_names(meta), params))
+    B, T, D = cand.shape
     gfeat, Kp, cmask, cidx = side
     gcn = meta.get('gcn', True)
     L = meta['gcn_layers'] if gcn else 0
     C = P['proxy_node_embedding'].shape[0] if gcn else meta['category_num']
     H = gfeat.shape[1]
-    user = SUEFunction._clusters_tail(_Mod(), P, gfeat, cand, cmask, cidx, [0] * (L + 2), (B, H, D, T, C, H + C, C + 1), L, 0.0,
+    return SUEFunction._clusters_tail(ctx, P, gfeat, cand, cmask, cidx, [0] * (L + 2), (B, H, D, T, C, H + C, C + 1), L, 0.0,
                                       keys=(None, Kp))
-    return RowDot.apply(user, cand)
+
+
+@torch.no_grad()
+def sue_tile_explain(meta, side, cand, *params):
+    """``sue_tile_scores`` and the explanation of each score: (scores [B, T], alpha [B, T, H], beta [B, T, C1],
+    beta * (f . cand) [B, T, C1]) -- the model's own intra-cluster weights (cluster_intra_fwd), inter-cluster weights
+    (attn_pool mode 1) and per-cluster score terms, whose sum over the clusters is the score up to fp32 rounding.  The
+    scores are sue_tile_scores' bit for bit (the same kernels on the same shapes).  SUE_wo_HCA: (scores, the pooled
+    attention's weights over the history expanded over the T candidates, None, None)."""
+    B, T, D = cand.shape
+    cand = cand.contiguous()
+    if not meta['hca']:
+        return sue_tile_scores(meta, side, cand, *params), side[1].unsqueeze(1).expand(-1, T, -1).contiguous(), None, None
+    ctx = _Mod()
+    user = _sue_tile_user(ctx, meta, side, cand, params)
+    scores = RowDot.apply(user, cand)
+    alpha, f, alpha2 = ctx.sv[2], ctx.sv[5], ctx.sv[9]
+    C1 = side[2].shape[1]
+    dots = _empty((B * T * C1,), cand.device)                                    # f_c . cand
+    ops.rowdot_fwd(f, cand.view(B * T, 1, D).expand(-1, C1, -1).contiguous(), B * T * C1, D, dots)
+    return scores, alpha.view(B, T, -1), alpha2.view(B, T, C1), (alpha2 * dots).view(B, T, C1)
 
 
 @torch.no_grad()
@@ -1151,6 +1179,22 @@ def sue_packed_scores_factored(meta, side, cand_rows, row_off, out, *params):
     out[b, j], and entries past its count are left as they are.  The candidate projections cost row_off[B] rows, not R.
     The scores are those of ``sue_tile_scores_factored`` on the same rows, bit for bit.  SUE_wo_HCA, whose user vector
     does not depend on the candidate: RowDot of the pooled user vector and each row, bit for bit the exact path's."""
+    return _sue_packed_factored(meta, side, cand_rows, row_off, out, None, params)[0]
+
+
+@torch.no_grad()
+def sue_packed_explain_factored(meta, side, cand_rows, row_off, out, alpha, beta, contrib, *params):
+    """``sue_packed_scores_factored`` that also explains each score it writes (nnr_cluster_tail_explain_packed): for user
+    b's j-th candidate, alpha[b, j] [H] the intra-cluster weights of the history slots, beta[b, j] [C1] the inter-cluster
+    weights and contrib[b, j] [C1] = beta * (f . cand) (alpha [B, n_max, H], beta / contrib [B, n_max, C1], contiguous,
+    out contiguous).  Entries past a user's count are left as they are.  The scores equal sue_packed_scores_factored's
+    bit for bit.  SUE_wo_HCA: alpha gets the pooled attention's weights over the history, beta and contrib are not
+    used.  Returns (out, alpha, beta, contrib)."""
+    return _sue_packed_factored(meta, side, cand_rows, row_off, out, (alpha, beta, contrib), params)
+
+
+def _sue_packed_factored(meta, side, cand_rows, row_off, out, ex, params):
+    """sue_packed_scores_factored (ex None) / sue_packed_explain_factored (ex = (alpha, beta, contrib))"""
     R, D = cand_rows.shape
     B, n_max = out.shape
     cand_rows = cand_rows.contiguous()
@@ -1163,13 +1207,19 @@ def sue_packed_scores_factored(meta, side, cand_rows, row_off, out, *params):
         lo = row_off[:B].long()
         valid = j[None, :] < (row_off[1:B + 1].long() - lo)[:, None]
         out.copy_(torch.where(valid, dots[(lo[:, None] + j[None, :]).clamp_(0, max(R - 1, 0))], out))
-        return out
+        if ex is not None:
+            ex[0].copy_(torch.where(valid[:, :, None], side[1][:, None, :], ex[0]))
+        return (out,) + (ex or ())
     P = dict(zip(sue_names(meta), params))
     gfeat, Kp, cmask, cidx, Wg = side
     H = gfeat.shape[1]
     C1 = cmask.shape[1]
     Au = P['intraCluster_K.weight'].shape[0]
     _, Qp, _, _, qk2 = SUEFunction._cand_side(P, cand_rows, 1, R, D, m_dev=total)
-    ops.cluster_tail_scores_packed(Kp, gfeat, Wg, cidx, cmask.contiguous().view(torch.uint8), row_off, Qp, qk2, cand_rows,
-                                   P['clusterFeatureAffine.bias'], B, H, Au, D, C1, n_max, 1.0 / math.sqrt(float(Au)), out)
-    return out
+    args = (Kp, gfeat, Wg, cidx, cmask.contiguous().view(torch.uint8), row_off, Qp, qk2, cand_rows,
+            P['clusterFeatureAffine.bias'], B, H, Au, D, C1, n_max, 1.0 / math.sqrt(float(Au)), out)
+    if ex is None:
+        ops.cluster_tail_scores_packed(*args)
+        return (out,)
+    ops.cluster_tail_explain_packed(*args, *ex)
+    return (out,) + ex

@@ -452,6 +452,18 @@ def cluster_tail_scores_packed(Kp, g, Wg, idx, cmask, row_off, Qp, qk2, cand, bi
                                              scores.stride(0), _stream()), 'nnr_cluster_tail_scores_packed')
 
 
+def cluster_tail_explain_packed(Kp, g, Wg, idx, cmask, row_off, Qp, qk2, cand, bias, B, H, Au, D, C1, n_max, scale, scores,
+                                alpha, beta, contrib):
+    """cluster_tail_scores_packed that also writes the explanation of each score: alpha [B, lds, H], beta and
+    beta * (f . cand) [B, lds, C1] (contiguous; lds = scores.stride(0)); entries past a user's count are left as they are
+    (nnr_cluster_tail_explain_packed)"""
+    check(lib.nnr_cluster_tail_explain_packed(_p(Kp, _F32), _p(g, _F32), _p(Wg, _F32), _p(idx, _I64), _p(cmask, _U8),
+                                              _p(row_off, _I32), Qp.shape[0], _p(Qp, _F32), _p(qk2, _F32), _p(cand, _F32),
+                                              _p(bias, _F32), B, H, Au, D, C1, n_max, float(scale), _p(scores, _F32),
+                                              scores.stride(0), _p(alpha, _F32), _p(beta, _F32), _p(contrib, _F32),
+                                              _stream()), 'nnr_cluster_tail_explain_packed')
+
+
 def rowdot_fwd(a, b, R, D, out):
     check(lib.nnr_rowdot_fwd(_p(a, _F32), _p(b, _F32), R, D, _p(out, _F32), _stream()), 'nnr_rowdot_fwd')
 
@@ -560,6 +572,10 @@ _SCHEMAS = {
     'cluster_tail_scores_packed': ('(Tensor Kp, Tensor g, Tensor Wg, Tensor idx, Tensor cmask, Tensor row_off, Tensor Qp, '
                                    'Tensor qk2, Tensor cand, Tensor bias, int B, int H, int Au, int D, int C1, int n_max, '
                                    'float scale, Tensor(a!) scores) -> ()', cluster_tail_scores_packed),
+    'cluster_tail_explain_packed': ('(Tensor Kp, Tensor g, Tensor Wg, Tensor idx, Tensor cmask, Tensor row_off, Tensor Qp, '
+                                    'Tensor qk2, Tensor cand, Tensor bias, int B, int H, int Au, int D, int C1, int n_max, '
+                                    'float scale, Tensor(a!) scores, Tensor(b!) alpha, Tensor(c!) beta, '
+                                    'Tensor(d!) contrib) -> ()', cluster_tail_explain_packed),
     'rowdot_fwd': ('(Tensor a, Tensor b, int R, int D, Tensor(a!) out) -> ()', rowdot_fwd),
     'rowdot_bwd': ('(Tensor dout, Tensor a, Tensor b, int R, int D, Tensor(a!) da, bool accumulate_a, Tensor(b!) db, bool accumulate_b) -> ()',
                    rowdot_bwd),

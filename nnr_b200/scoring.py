@@ -18,10 +18,14 @@ the metrics are bit-identical to one GPU.  The all-gathers run on the current st
 the all-gathered rank lists are merged into one on every rank (``nnr_topk_merge_lists``).
 """
 import numbers
+from collections import namedtuple
 
 import torch
 
 from . import engine, metrics, ops
+
+# CorpusScorer.explain(): a click score and its split over the user's interest clusters
+Explanation = namedtuple('Explanation', 'scores cluster_weight cluster_score history_weight history_cluster')
 
 
 def contiguous_blocks(nblocks, world):
@@ -240,10 +244,10 @@ class CorpusScorer:
             return self._graphed(key, self._score_packed_impl, (hid, hl, cid, cnt)).clone()
         return self._score_packed_impl(hid, hl, cid, cnt)
 
-    def _score_packed_impl(self, hid, hl, cid, cnt):
+    def _packed_rows(self, cid, cnt):
         """the candidates are packed back to back on the device (prefix sum of the counts; no host synchronisation): list b
         is rows [row_off[b], row_off[b + 1]) of a [B * n, D] buffer whose rows past row_off[B] hold news 0 and are not
-        scored.  Padding entries of cid are never read."""
+        scored.  Padding entries of cid are never read.  Returns (row_off [B + 1] int32, the B * n corpus ids)."""
         B, n = cid.shape
         row_off = torch.zeros(B + 1, dtype=torch.int32, device=self.dev)
         torch.cumsum(cnt, 0, dtype=torch.int32, out=row_off[1:])
@@ -251,9 +255,91 @@ class CorpusScorer:
         # packed row of every valid entry; padding goes to a dump slot past the end
         dest = torch.where(j[None, :] < cnt[:, None], row_off[:B, None].long() + j[None, :], B * n)
         ids = torch.zeros(B * n + 1, dtype=torch.int64, device=self.dev).scatter_(0, dest.view(-1), cid.reshape(-1))[:B * n]
+        return row_off, ids
+
+    def _score_packed_impl(self, hid, hl, cid, cnt):
+        B, n = cid.shape
+        row_off, ids = self._packed_rows(cid, cnt)
         ue = self.model.user_encoder
         side = ue.user_side(self.cache[hid], *self._history_graph(hid, hl), factored=True)
         return ue.packed_scores_factored(side, self.cache[ids], row_off, torch.zeros(B, n, device=self.dev))
+
+    @torch.no_grad()
+    def explain(self, history_ids, history_len, candidate_ids, candidate_count=None, cuda_graph=True, exact=False):
+        """Why each candidate scores as it does: the click score of ``score()`` split over the user's interest clusters.
+        SUE clusters a user's history by ``news_category``, and the score of a candidate is a sum over the clusters,
+        score = sum_c beta_c (f_c . cand): beta is the inter-cluster attention, f_c the cluster's feature, built from the
+        history news of cluster c weighted by the intra-cluster attention alpha.
+
+        history_ids [B, H] (0-padded at the end), history_len [B] and candidate_ids [B, n] are those of ``score()``;
+        with candidate_count [B] only the first candidate_count[b] entries of row b are explained (their ids must lie in
+        [0, news_num); the entries past the count are never read, -1 for instance).  Returns an ``Explanation``:
+
+        - scores [B, n] fp32: the click scores, bit for bit those of ``score(..., exact=exact)`` on the same inputs;
+        - cluster_weight [B, n, C + 1]: beta, exactly 0 for a masked cluster.  Cluster c < C is news_category c, cluster
+          C holds the padding slots of the history;
+        - cluster_score [B, n, C + 1]: beta_c (f_c . cand), whose sum over c is the score up to fp32 rounding;
+        - history_weight [B, n, H]: alpha, each history slot's weight within its cluster, in history order; it sums to 1
+          over the slots of each non-empty cluster;
+        - history_cluster [B, H] int64: the cluster of each history slot.
+        Entries past a row's count are 0.  SUE_wo_HCA has no clusters: cluster_weight, cluster_score and
+        history_cluster are None, and history_weight holds the weights of its additive attention over the history,
+        the same for every candidate.
+
+        ``exact=False`` (the default) explains through the factored cluster tail (nnr_cluster_tail_explain_packed): the
+        candidates are packed by count as in ``evaluate(exact=False)``, and no per-pair buffer beyond the outputs is
+        stored.  ``exact=True`` returns the model's own tensors (the intra-cluster weights of cluster_intra_fwd, the
+        inter-cluster weights of the attention pooling), at the memory cost of ``score()``; entries past a count score
+        news 0 and are then zeroed.  SUE_wo_HCA returns the ``exact=True`` result either way, as ``score()`` does.
+        Rank-local, never a collective.  Deterministic; B >= 64 replays one captured CUDA graph per shape.  The
+        arguments are checked once per call, before any launch (ValueError).
+
+        To explain a ``recommend()`` result, whose fill entries (id -1) sit at the tail of each row::
+
+            ids, _ = scorer.recommend(hist, hl, pool, k=10)
+            why = scorer.explain(hist, hl, ids, candidate_count=(ids >= 0).sum(1))
+            top = why.cluster_score[:, 0].argmax(1)       # the interest that weighs most in each user's first pick
+        """
+        cid, cnt = self._packed_inputs('explain', candidate_ids, candidate_count)
+        hid = torch.as_tensor(history_ids).to(self.dev).long()
+        hl = torch.as_tensor(history_len).to(self.dev).to(torch.int32)
+        cid, cnt = cid.to(self.dev), cnt.to(self.dev)
+        B, n = cid.shape
+        if B == 0 or n == 0:
+            hca = self.model.user_encoder.hca
+            cidx = (self._history_graph(hid, hl)[2] if B else torch.zeros(hid.shape, dtype=torch.int64, device=self.dev))
+            return Explanation(*self._explain_outputs(B, n, hid.shape[1]), cidx if hca else None)
+        impl = self._explain_exact_impl if exact else self._explain_packed_impl
+        if cuda_graph and B >= 64:
+            key = ('explain', bool(exact), tuple(hid.shape), tuple(cid.shape), self.cache.data_ptr())
+            out = self._graphed(key, impl, (hid, hl, cid, cnt))
+            return Explanation(*(None if t is None else t.clone() for t in out))
+        return Explanation(*impl(hid, hl, cid, cnt))
+
+    def _explain_outputs(self, B, n, H):
+        """zeroed (scores, cluster_weight, cluster_score, history_weight) of explain(); None for the cluster fields of
+        SUE_wo_HCA"""
+        z = lambda *shape: torch.zeros(*shape, device=self.dev)
+        C1 = self._category_num() + 1
+        hca = self.model.user_encoder.hca
+        return z(B, n), z(B, n, C1) if hca else None, z(B, n, C1) if hca else None, z(B, n, H)
+
+    def _explain_packed_impl(self, hid, hl, cid, cnt):
+        B, n = cid.shape
+        row_off, ids = self._packed_rows(cid, cnt)
+        graph, cmask, cidx = self._history_graph(hid, hl)
+        ue = self.model.user_encoder
+        side = ue.user_side(self.cache[hid], graph, cmask, cidx, factored=True)
+        scores, beta, contrib, alpha = self._explain_outputs(B, n, hid.shape[1])
+        ue.packed_explain_factored(side, self.cache[ids], row_off, scores, alpha, beta, contrib)
+        return scores, beta, contrib, alpha, cidx if ue.hca else None
+
+    def _explain_exact_impl(self, hid, hl, cid, cnt):
+        """every entry past a count is explained as news 0 (each pair's tail is row-independent), then zeroed"""
+        valid = torch.arange(cid.shape[1], device=self.dev)[None, :] < cnt[:, None]
+        scores, alpha, beta, contrib, cidx = self._score_impl(hid, hl, torch.where(valid, cid, 0), explain=True)
+        zero = lambda t: None if t is None else t.masked_fill_(~valid.view(valid.shape + (1,) * (t.dim() - 2)), 0.0)
+        return zero(scores), zero(beta), zero(contrib), zero(alpha), cidx if self.model.user_encoder.hca else None
 
     def _category_num(self):
         ue = self.model.user_encoder
@@ -271,11 +357,17 @@ class CorpusScorer:
         ops.sue_graph_build(cats, hl, C, graph, cmask, cidx, flags=self.graph_flags)
         return graph, cmask, cidx
 
-    def _score_impl(self, hid, hl, cid):
+    def _score_impl(self, hid, hl, cid, explain=False):
+        """scores [B, n]; ``explain``: (scores, alpha, beta, beta * (f . cand), cluster indices) of the same inputs through
+        the user side and the candidate tail of the forward (UserEncoder.user_side / tile_explain), whose scores equal
+        encode_user's bit for bit (the split recommend() scores through)"""
         graph, cmask, cidx = self._history_graph(hid, hl)
         hist = self.cache[hid]                                  # [B, H, D]
         cand = self.cache[cid]                                  # [B, n, D]
-        user = self.model.user_encoder.encode_user(hist, graph, cmask, cidx, cand)
+        ue = self.model.user_encoder
+        if explain:
+            return ue.tile_explain(ue.user_side(hist, graph, cmask, cidx), cand) + (cidx,)
+        user = ue.encode_user(hist, graph, cmask, cidx, cand)
         return engine.RowDot.apply(user, cand)
 
     def default_pool_tile(self, B):

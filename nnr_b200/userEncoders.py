@@ -103,6 +103,12 @@ class SUE(UserEncoder):
         RowDot(encode_user(...), candidates) on the same inputs (engine.sue_tile_scores)"""
         return engine.sue_tile_scores(self._meta(), user_side, candidate_news_representation, *self._params())
 
+    def tile_explain(self, user_side, candidate_news_representation):
+        """tile_scores and the explanation of each score: (scores [B, T], alpha [B, T, H], beta [B, T, C1],
+        beta * (f . cand) [B, T, C1]), the model's own attention weights and per-cluster score terms; SUE_wo_HCA:
+        (scores, its pooled attention's weights [B, T, H], None, None) (engine.sue_tile_explain)"""
+        return engine.sue_tile_explain(self._meta(), user_side, candidate_news_representation, *self._params())
+
     def tile_scores_factored(self, user_side, candidate_rows):
         """click scores [B, T] of candidates [T, D] shared by the users of ``user_side(..., factored=True)``, through the
         factored cluster tail: equal to tile_scores on the expanded candidates in real arithmetic, not bit for bit
@@ -115,3 +121,10 @@ class SUE(UserEncoder):
         to out[b, j] and the rest of out is left as it is; returns out.  The factored cluster tail, as in
         tile_scores_factored (engine.sue_packed_scores_factored)"""
         return engine.sue_packed_scores_factored(self._meta(), user_side, candidate_rows, row_off, out, *self._params())
+
+    def packed_explain_factored(self, user_side, candidate_rows, row_off, out, alpha, beta, contrib):
+        """packed_scores_factored that also writes the explanation of each score: alpha [B, n, H], beta and
+        beta * (f . cand) [B, n, C1], past the counts left as they are; returns (out, alpha, beta, contrib)
+        (engine.sue_packed_explain_factored)"""
+        return engine.sue_packed_explain_factored(self._meta(), user_side, candidate_rows, row_off, out, alpha, beta, contrib,
+                                                  *self._params())

@@ -41,6 +41,7 @@ class SUE_wo_GCN(UserEncoder):
     encode_user = SUE.encode_user
     _meta, user_side, tile_scores = SUE._meta, SUE.user_side, SUE.tile_scores
     tile_scores_factored, packed_scores_factored = SUE.tile_scores_factored, SUE.packed_scores_factored
+    tile_explain, packed_explain_factored = SUE.tile_explain, SUE.packed_explain_factored
 
     def __init__(self, news_encoder, config):
         super().__init__(news_encoder, config)
@@ -77,6 +78,7 @@ class SUE_wo_HCA(UserEncoder):
     encode_user = SUE.encode_user
     _meta, user_side, tile_scores = SUE._meta, SUE.user_side, SUE.tile_scores
     tile_scores_factored, packed_scores_factored = SUE.tile_scores_factored, SUE.packed_scores_factored
+    tile_explain, packed_explain_factored = SUE.tile_explain, SUE.packed_explain_factored
 
     def __init__(self, news_encoder, config):
         super().__init__(news_encoder, config)
